@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the B200 weighted Wagner–Fischer engine.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2|c2-iupac]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY 8d "C2"): 1,000,000 synthetic RNA pairs per GPU, lengths
 iid uniform in [100,300], alphabet ACGU iid uniform, costs = the shipped user_costs.json, distance
@@ -37,10 +38,24 @@ sys.path.insert(0, ROOT)
 
 SEEDS = {"c2": 20260002, "c2-iupac": 20260002}
 L2_FLUSH_BYTES = 512 << 20
+DUMP_BYTES = 60 << 20              # data written by --dump-outputs: with its .npy header, under 64 * 10^6 bytes
+DUMP_SEED = 20260099
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+def dump_outputs(directory, distances):
+    """Write what the timed path returned in its last step, the float64 distance of every pair, to
+    DIR/distances.npy, so that two builds run with the same arguments can be compared output for output.  A batch
+    larger than DUMP_BYTES is cut to a fixed, seeded sample of its pairs (kept in pair order)."""
+    n_max = DUMP_BYTES // distances.itemsize
+    if distances.shape[0] > n_max:
+        keep = np.sort(np.random.default_rng(DUMP_SEED).choice(distances.shape[0], n_max, replace=False))
+        distances = distances[keep]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "distances.npy"), np.ascontiguousarray(distances, dtype=np.float64))
 
 
 def gen_pairs(n_pairs: int, seed: int, alphabet_size: int):
@@ -209,7 +224,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C3/C4/C5 side measurements")
     ap.add_argument("--c5-records", type=int, default=10_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the distances of the last device-resident step to DIR/distances.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -487,6 +508,8 @@ def main():
         pass
     roofline["traffic"] = traffic
     roofline["traffic_source"] = "profiles/traffic.json: dram__bytes_read.sum + dram__bytes_write.sum of one ncu --set full capture of this kernel at this size" if traffic else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, check_dev)          # rank 0's batch
 
     print(file=out, flush=True, *[json.dumps({
         "metric": "GCUPS", "value": value, "unit": "GCUPS", "n_gpus": world, "steps": args.steps,
