@@ -80,6 +80,35 @@ def test_classifier_modes(built, default_costs, user_costs):
     assert ei.value.code == 5
 
 
+def test_classifier_edges(built, default_costs, user_costs):
+    """The documented edges of the narrow kernels, last shape inside and first shape outside: a bound that tightens
+    sends exact work to a slower kernel, which no parity test notices.  (mode, k): 1 int16x2, 2 int32, 3 fp64."""
+    import _edges as E
+    eng = built.Engine(0)
+    cases = [
+        (E.v_table(), 0xF, [((478, 478), (1, 0)), ((479, 479), (2, 0))]),            # v = 127 fits the byte table
+        (E.v_table(ins_del=(64, 64)), 0xF, [((10, 10), (2, 0))]),                     # v = 128 does not
+        (E.v_table(k=2), 0xF, [((478, 478), (1, 2)), ((479, 479), (2, 2))]),          # the same after a x4 scale
+        (E.v_table(k=2, ins_del=(64, 64)), 0xF, [((10, 10), (2, 2))]),
+        (default_costs, 0xF, [((32466, 32466), (1, 0)), ((32467, 32467), (2, 0))]),   # N < 65000
+        (user_costs, 0xF, [((12960, 12960), (1, 0)), ((12961, 12961), (2, 0))]),
+        # asymmetric: the first is bounded by the swapped orientation, the second by the stored one
+        (E.table(27, 100, E.SUBS_V), 0xF, [((40, 2017), (1, 0)), ((40, 2018), (2, 0))]),
+        (E.table(100, 27, E.SUBS_V), 0xF, [((200, 530), (1, 0)), ((200, 531), (2, 0))]),
+        (E.uniform(2.0 ** 20), 0xF, [((990, 990), (2, 0)), ((991, 991), (3, 0))]),    # |H'| < 2147483000
+        (E.uniform(2.0 ** 20), 0x7FFF, [((990, 990), (2, 0)), ((991, 991), (3, 0))]),
+        (E.K16_SMALL, 0xF, [((300, 300), (1, 16))]),
+        (E.K16_WIDE, 0xF, [((300, 300), (2, 16))]),
+        (E.K17, 0xF, [((300, 300), (3, 0))]),
+        (E.DEAR_IN, 0xF, [((300, 300), (2, 0))]),                                      # scaled costs < 2^30
+        (E.DEAR_OUT, 0xF, [((300, 300), (3, 0))]),
+    ]
+    for costs, symmask, shapes in cases:
+        eng.set_costs(costs)
+        for (m, n), want in shapes:
+            assert eng.classify(symmask, m, n) == want, (costs["insert"], costs["delete"], symmask, m, n)
+
+
 def test_topk_merge_host(built):
     import numpy as np
     eng = built.Engine(0)
