@@ -167,24 +167,6 @@ k_search_twin16(const uint32_t *__restrict__ db_words, const int64_t *__restrict
     }
 }
 
-// General path: distances of one query against a range of records were produced by the systolic
-// distance kernels (any mode); turn them into scores, optional all_scores row, and candidates.
-__global__ void k_score_filter(const double *__restrict__ dist, int64_t rec0, int64_t n_rec, const int64_t *__restrict__ perm,
-                               int64_t global_base, int q, TopkState tk, double *__restrict__ all_scores, int64_t all_stride) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= n_rec) return;
-    const double s = __ddiv_rn(1.0, __dadd_rn(1.0, dist[r]));
-    const long long g = perm[rec0 + r];
-    if (all_scores) all_scores[(size_t)q * all_stride + (g - global_base)] = s;
-    if (tk.k > 0) {
-        const double ts = tk.tau_s[q]; const long long ti = tk.tau_i[q];
-        if (s > ts || (s == ts && g <= ti)) {
-            const int slot = atomicAdd(&tk.cand_n[q], 1);
-            if (slot < tk.cap) { tk.cand_s[(size_t)q * tk.cap + slot] = s; tk.cand_i[(size_t)q * tk.cap + slot] = g; }
-        }
-    }
-}
-
 __global__ void k_topk_init(TopkState tk, int n_queries) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= n_queries) return;
@@ -297,7 +279,8 @@ __global__ void k_fill_pairs_view(const int64_t *__restrict__ q_start, const int
     b_start[p] = db_start[r]; b_len[p] = db_len[r];
 }
 
-// ... and their distances -> scores, optional all_scores rows, candidates (k_score_filter for n_q queries)
+// ... and their distances (produced by the systolic distance kernels, any mode) -> scores, optional all_scores rows, and
+// the candidates of each of the n_q queries
 __global__ void k_score_filter_pairs(const double *__restrict__ dist, int64_t rec0, int64_t n_rec, const int64_t *__restrict__ perm,
                                      int64_t global_base, int q_base, int n_q, TopkState tk, double *__restrict__ all_scores, int64_t all_stride) {
     const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -320,11 +303,4 @@ __global__ void k_score_filter_pairs(const double *__restrict__ dist, int64_t re
             if (slot < tk.cap) { tk.cand_s[(size_t)q * tk.cap + slot] = s; tk.cand_i[(size_t)q * tk.cap + slot] = g; }
         }
     }
-}
-
-__global__ void k_fill_query_view(const int64_t *__restrict__ q_start, const int32_t *__restrict__ q_len, int q,
-                                  int64_t n, int64_t *__restrict__ a_start, int32_t *__restrict__ a_len) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= n) return;
-    a_start[r] = q_start[q]; a_len[r] = q_len[q];
 }
