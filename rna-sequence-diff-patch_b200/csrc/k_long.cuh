@@ -1,6 +1,8 @@
-// k_long.cuh — one long pair (>= ~10 kb per side; BASELINE config 4: 50 kb x 50 kb with traceback).
+// k_long.cuh — one long pair whose keys do not fit the 32-bit keys of k_long2.cuh: the fallback for costs too large
+// for that bound (the integer key held exactly in a double) and for non-dyadic costs (fp64 cost, int steps).  One pair
+// per launch, the whole direction matrix resident.  Also the polling helpers both long-pair kernels use.
 //
-// Block-tiled diagonal wavefront: the matrix is cut into column panels of 32*C columns (C = 4); panel w is
+// Block-tiled diagonal wavefront: the matrix is cut into column panels of 32*C columns; panel w is
 // owned by warp w (one warp per CTA so panels spread over all SMs) and, inside the panel, lane s
 // owns C columns in registers — the same systolic row pipeline as the batched kernels.  Panels run
 // concurrently as a second-level pipeline: the right-most column of panel w streams through a
@@ -8,10 +10,6 @@
 // ready flag: the array is preset to a sentinel and polled).  All CTAs are co-resident (cooperative launch), so the waits cannot
 // deadlock.  Directions are 2 bit/cell, accumulated 16 rows per register and written with 128-bit
 // stores; the traceback walks them from (m,n).
-//
-// Keys are (cost, steps) folded into one integer (cost << S | steps) in the H' form of k_script.cuh,
-// held exactly in a double (int32 would overflow at 50 kb; see k_long_fwd) — or (fp64 cost, int
-// steps) when the costs are not dyadic.
 // Replaces (reference): wagnerFisher + create_paths(dp)[0] + generate_es for a pair the reference
 // cannot hold in memory (~500 B per cell, SURVEY section 5).
 #pragma once
@@ -21,14 +19,11 @@ struct LongArgs {
     const uint8_t *a; int m;           // 1 byte / symbol codes on the device
     const uint8_t *b; int n;
     int n_panels, n_pad;               // n_pad = n_panels * 32 * C
-    int bstride;                       // cells reserved per panel in `bound` (>= m)
     uint32_t *dirs;                    // [ceil(m/16)][n_pad]
     void *bound;                       // [n_panels][m] keys (int64 or double)
     int *bound_steps;                  // [n_panels][m] (fp64 mode)
-    int *progress;                     // [n_panels] rows published
     double *dist;
     int S;
-    unsigned long long *dbg;           // optional [n_panels][4]: start ns, end ns, poll clocks, publish clocks
 };
 
 // boundary cells are their own "ready" flag: the array is preset to this bit pattern (memset 0x80,
@@ -98,14 +93,11 @@ k_long_fwd(LongArgs la, const IntCosts *__restrict__ icp, const F64Costs *__rest
     const bool publish = (w + 1 < la.n_panels);
     uint32_t *dcol = la.dirs + col0;
     const int steps = m + 31 + 16;                  // + one block so the last rows get published
-    unsigned long long dbg_t0 = 0, dbg_poll = 0, dbg_pub = 0, dbg_ld = 0, dbg_loop = 0;
-    if (la.dbg) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(dbg_t0));
 
 #pragma unroll 1
     for (int t0 = 0; t0 < steps; t0 += 16) {
         // (0) rows finished by lane 31 during the previous block (t0-16-31 .. t0-1-31) go to the next panel:
         //     16 lanes, one coalesced non-blocking store each
-        long long c0 = la.dbg ? clock64() : 0;
         if (publish && lane < 16) {
             const int r = t0 - 47 + lane;
             if (r >= 0 && r < m) {
@@ -114,7 +106,6 @@ k_long_fwd(LongArgs la, const IntCosts *__restrict__ icp, const F64Costs *__rest
             }
         }
         __syncwarp();
-        if (la.dbg) { long long c1 = clock64(); dbg_pub += (unsigned long long)(c1 - c0); c0 = c1; }
         // (1) the 16 boundary cells lane 0 will consume in this block, fetched by lanes 0..15 in parallel
         //     The loop condition is a warp vote so all 32 lanes leave it together: a per-lane spin would
         //     leave the warp split in two for the rest of the block (every instruction issued twice).
@@ -130,7 +121,6 @@ k_long_fwd(LongArgs la, const IntCosts *__restrict__ icp, const F64Costs *__rest
                 if constexpr (F64) bval_s = bin_s[t0 + lane];
             }
         }
-        if (la.dbg) { __syncwarp(); long long c1 = clock64(); dbg_poll += (unsigned long long)(c1 - c0); c0 = c1; }
         // (2) this lane's 16 source symbols (rows t0-lane .. t0-lane+15), 4 bits each
         //     staged through shared memory: two coalesced byte loads per lane per block
         unsigned long long codes = 0ull;
@@ -143,7 +133,6 @@ k_long_fwd(LongArgs la, const IntCosts *__restrict__ icp, const F64Costs *__rest
             for (int k = 0; k < 16; ++k) codes |= (unsigned long long)s_a[31 - lane + k] << (4 * k);
             __syncwarp();
         }
-        if (la.dbg) { __syncwarp(); long long c1 = clock64(); dbg_ld += (unsigned long long)(c1 - c0 + (codes & 0)); c0 = c1; }
 #pragma unroll 1
         for (int k = 0; k < 16; ++k) {
             const int t = t0 + k;
@@ -205,11 +194,6 @@ k_long_fwd(LongArgs la, const IntCosts *__restrict__ icp, const F64Costs *__rest
             if (lane == 31) { s_pub[k] = last; if constexpr (F64) s_pub_s[k] = last_s; }
         }
         __syncwarp();
-        if (la.dbg) dbg_loop += (unsigned long long)(clock64() - c0);
-    }
-    if (la.dbg && lane == 0) {
-        unsigned long long t1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-        la.dbg[w * 8 + 0] = dbg_t0; la.dbg[w * 8 + 1] = t1; la.dbg[w * 8 + 2] = dbg_poll; la.dbg[w * 8 + 3] = dbg_pub; la.dbg[w * 8 + 4] = dbg_ld; la.dbg[w * 8 + 5] = dbg_loop;
     }
     // the cell (m, n) lives in panel (n-1)/(32C), lane ((n-1)/C)%32, column (n-1)%C
     if (strip_on && col0 <= n - 1 && n - 1 < col0 + C) {
@@ -222,322 +206,6 @@ k_long_fwd(LongArgs la, const IntCosts *__restrict__ icp, const F64Costs *__rest
             const long long key = (long long)res + (long long)m * (((long long)icp->del << la.S) + 1) + (long long)n * (((long long)icp->ins << la.S) + 1);
             la.dist[0] = (double)(key >> la.S) / (double)(1 << icp->scale_log2);
         }
-    }
-}
-
-// Integer keys in 32 bits, compared modulo 2^32.  The (cost << S | steps) key of a 50 kb pair needs ~36
-// bits, but a cell only ever compares candidates that lie a bounded distance apart (neighbouring cells
-// differ by at most (ins + del + max|w|) << S), so the sign of the 32-bit wrapped difference is the sign of
-// the true difference and min(a, b) = a + min(b - a, 0) is exact.  The host checks that bound.  The fp64
-// pipe's long latency sat on the per-row dependency chain of the double-carried keys; here the chain per
-// cell is VIADDMNMX + IADD.  Direction bits are the sign bits of the two differences, as in k_script_fwd.
-// The full 64-bit key of cell (m, n) — needed for the distance — is rebuilt from bounded row-to-row
-// differences of each lane's last column.  Boundary words between panels are (1 << 32 | key): the high
-// half doubles as the "published" tag against the 0x80.. sentinel.
-template <int C>
-__global__ void __launch_bounds__(32)
-k_long_fwd32(LongArgs la, const IntCosts *__restrict__ icp) {
-    __shared__ uint32_t s_w[256];
-    __shared__ uint32_t s_pub[16];
-    __shared__ uint8_t s_a[64];
-    for (int k = threadIdx.x; k < 256; k += 32)
-        s_w[k] = (uint32_t)(((long long)icp->w[k >> 4][k & 15] << la.S) - 1);        // (w << S) - 1, fits (host check)
-    __syncwarp();
-    const int lane = threadIdx.x;
-    const int w = blockIdx.x;                       // panel
-    const int m = la.m, n = la.n;
-    const int col0 = (w * 32 + lane) * C;
-    const bool strip_on = col0 < n;
-    int bc[C];
-#pragma unroll
-    for (int c = 0; c < C; ++c) bc[c] = (col0 + c < n) ? la.b[col0 + c] : 0;
-    uint32_t H[C], acc[C], bca[C];                  // bca: shared-memory byte address of the column's table entry in row 0
-    const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(s_w);
-#pragma unroll
-    for (int c = 0; c < C; ++c) { H[c] = 0u; acc[c] = 0u; bca[c] = sbase + 4u * (uint32_t)bc[c]; }
-    uint32_t last = 0u, prev_recv = 0u;
-    long long full = 0;                             // exact key of this lane's last column, current row
-    const unsigned long long *bin = w > 0 ? (const unsigned long long *)la.bound + (size_t)(w - 1) * m : nullptr;
-    unsigned long long *bout = (unsigned long long *)la.bound + (size_t)w * m;
-    const bool publish = (w + 1 < la.n_panels);
-    uint32_t *dcol = la.dirs + col0;
-    const int steps = m + 31 + 16;                  // + one block so the last rows get published
-    unsigned long long dbg_t0 = 0, dbg_poll = 0, dbg_pub = 0, dbg_ld = 0, dbg_loop = 0;
-    if (la.dbg) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(dbg_t0));
-    uint8_t pf0 = ((unsigned)(lane - 31) < (unsigned)m) ? la.a[lane - 31] : (uint8_t)0;      // rows of block 0
-    uint8_t pf1 = (lane < 15 && 1 + lane < m) ? la.a[1 + lane] : (uint8_t)0;
-
-#pragma unroll 1
-    for (int t0 = 0; t0 < steps; t0 += 16) {
-        long long c0 = la.dbg ? clock64() : 0;
-        const uint32_t last_at_block_start = last;
-        if (publish && lane < 16) {
-            const int r = t0 - 47 + lane;
-            if (r >= 0 && r < m) st_cg_u64(bout + r, (1ull << 32) | (unsigned long long)s_pub[lane]);
-        }
-        __syncwarp();
-        if (la.dbg) { long long c1 = clock64(); dbg_pub += (unsigned long long)(c1 - c0); c0 = c1; }
-        uint32_t bval = 0u;
-        if (w > 0) {
-            const bool mine = lane < 16 && t0 + lane < m;
-            unsigned long long raw = 0ull;
-            do {
-                if (mine) raw = ld_poll_u64(bin + t0 + lane);
-            } while (!__all_sync(RSD_FULL, raw != RSD_LONG_SENTINEL));      // warp-uniform exit (see k_long_fwd)
-            bval = (uint32_t)raw;
-        }
-        if (la.dbg) { __syncwarp(); long long c1 = clock64(); dbg_poll += (unsigned long long)(c1 - c0); c0 = c1; }
-        unsigned long long codes = 0ull;
-        {
-            // this block's source symbols were fetched one block ahead; fetch the next block's now so the
-            // global-load latency hides behind the 16 rows below
-            s_a[lane] = pf0;
-            if (lane < 15) s_a[32 + lane] = pf1;
-            const int r0 = t0 + 16 - 31 + lane, r1 = t0 + 16 + 1 + lane;
-            pf0 = ((unsigned)r0 < (unsigned)m) ? la.a[r0] : (uint8_t)0;
-            if (lane < 15) pf1 = ((unsigned)r1 < (unsigned)m) ? la.a[r1] : (uint8_t)0;
-            __syncwarp();
-#pragma unroll
-            for (int k = 0; k < 16; ++k) codes |= (unsigned long long)s_a[31 - lane + k] << (4 * k);
-            __syncwarp();
-        }
-        if (la.dbg) { __syncwarp(); long long c1 = clock64(); dbg_ld += (unsigned long long)(c1 - c0 + (codes & 0)); c0 = c1; }
-        // Blocks in which every lane is inside its rows (all but the first and last few) run a copy of the
-        // row loop without the per-row activity test: no branch for the scheduler to work around.
-        auto run16 = [&](auto steady_tag) {
-        constexpr bool STEADY = decltype(steady_tag)::value;
-#pragma unroll 2
-        for (int k = 0; k < 16; ++k) {
-            const int t = t0 + k;
-            const int i = t - lane;
-            const bool row_on = STEADY || (strip_on && (unsigned)i < (unsigned)m);
-            // phase A — everything that does not involve the left neighbour (the table row, diag + w, the
-            // DEL/UPD decision) is issued first and runs while the shuffle below is in flight
-            const uint32_t rowoff = ((uint32_t)(codes >> (4 * k)) & 15u) << 6;        // byte offset of the table row
-            uint32_t t2[C], wv[C]; int e1[C];
-#pragma unroll
-            for (int c = 0; c < C; ++c) asm volatile("ld.shared.u32 %0, [%1];" : "=r"(wv[c]) : "r"(bca[c] + rowoff));
-            {
-                uint32_t diag = prev_recv;
-#pragma unroll
-                for (int c = 0; c < C; ++c) {
-                    const uint32_t up = H[c];
-                    const uint32_t x = diag + wv[c];
-                    e1[c] = (int)(x - up);                                         // < 0  <=>  diagonal strictly better than up (ties keep DEL)
-                    t2[c] = up + (uint32_t)min(e1[c], 0);                          // min(up, x) modulo 2^32
-                    diag = up;
-                }
-            }
-            uint32_t recv = __shfl_up_sync(RSD_FULL, last, 1);
-            const uint32_t b0 = __shfl_sync(RSD_FULL, bval, k);
-            if (lane == 0) recv = w > 0 ? b0 : 0u;
-            if (row_on) {
-                // phase B — the dependency chain of the row: per cell VIADDMNMX + IADD
-                uint32_t left = recv;
-#pragma unroll
-                for (int c = 0; c < C; ++c) {
-                    const int e2 = (int)(t2[c] - left);                            // < 0  <=>  left loses (ties keep INS)
-                    const uint32_t hn = t2[c] + (uint32_t)__viaddmin_s32((int)left, -(int)t2[c], 0);   // min(left, t2)
-                    H[c] = hn; left = hn;
-                    acc[c] = __funnelshift_l((uint32_t)e2, acc[c], 1);             // "not INS"
-                    acc[c] = __funnelshift_l((uint32_t)e1[c], acc[c], 1);          // then "UPD rather than DEL"
-                }
-                last = left; prev_recv = recv;
-                if ((i & 15) == 15 || i == m - 1) {
-                    const int sh = 2 * (15 - (i & 15));
-                    if constexpr (C >= 4) {
-                        uint4 *dst = reinterpret_cast<uint4 *>(dcol + (size_t)(i >> 4) * la.n_pad);
-#pragma unroll
-                        for (int c = 0; c < C; c += 4)
-                            dst[c >> 2] = make_uint4(acc[c] << sh, acc[c + 1] << sh, acc[c + 2] << sh, acc[c + 3] << sh);
-                    } else {
-                        *reinterpret_cast<uint2 *>(dcol + (size_t)(i >> 4) * la.n_pad) = make_uint2(acc[0] << sh, acc[1] << sh);
-                    }
-                }
-            }
-            if (lane == 31) s_pub[k] = last;
-        }
-        };
-        if (t0 >= 31 && t0 + 15 <= m - 1) run16(std::true_type{}); else run16(std::false_type{});
-        full += (long long)(int)(last - last_at_block_start);          // <= 16 bounded row-to-row differences (host check)
-        __syncwarp();
-        if (la.dbg) dbg_loop += (unsigned long long)(clock64() - c0);
-    }
-    if (la.dbg && lane == 0) {
-        unsigned long long t1; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-        la.dbg[w * 8 + 0] = dbg_t0; la.dbg[w * 8 + 1] = t1; la.dbg[w * 8 + 2] = dbg_poll; la.dbg[w * 8 + 3] = dbg_pub; la.dbg[w * 8 + 4] = dbg_ld; la.dbg[w * 8 + 5] = dbg_loop;
-    }
-    if (strip_on && col0 <= n - 1 && n - 1 < col0 + C) {
-        const int cl = (n - 1) - col0;
-        uint32_t res = 0u;
-#pragma unroll
-        for (int c = 0; c < C; ++c) if (c == cl) res = H[c];
-        // `full` is the exact key of column C-1 at row m; column cl lies at most C-1 cells to its left
-        const long long hkey = full + (long long)(int)(res - H[C - 1]);
-        const long long key = hkey + (long long)m * (((long long)icp->del << la.S) + 1) + (long long)n * (((long long)icp->ins << la.S) + 1);
-        la.dist[0] = (double)(key >> la.S) / (double)(1 << icp->scale_log2);
-    }
-}
-
-// Same keys and protocol as k_long_fwd32, but every lane advances TWO rows per step (a 2 x C register tile):
-// one loop overhead, one pair of shuffles and one boundary exchange per two rows, and the two rows form a
-// small wavefront (cell (r+1, c) needs (r, c), (r, c-1), (r+1, c-1)) that gives the single resident warp
-// independent instructions to issue.  Lane l works on rows 2(s - l), 2(s - l) + 1 at step s; blocks are 16
-// steps = 32 rows, so the boundary exchange moves 32 rows at a time (one per lane).
-template <int C>
-__global__ void __launch_bounds__(32)
-k_long_fwd32x2(LongArgs la, const IntCosts *__restrict__ icp) {
-    __shared__ uint32_t s_w[256];
-    __shared__ uint32_t s_pub[32];
-    __shared__ __align__(4) uint8_t s_a[96];
-    for (int k = threadIdx.x; k < 256; k += 32)
-        s_w[k] = (uint32_t)(((long long)icp->w[k >> 4][k & 15] << la.S) - 1);
-    __syncwarp();
-    const int lane = threadIdx.x;
-    const int w = blockIdx.x;
-    const int m = la.m, n = la.n;
-    const int col0 = (w * 32 + lane) * C;
-    const bool strip_on = col0 < n;
-    uint32_t H[C], acc[C], bca[C];
-    const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(s_w);
-#pragma unroll
-    for (int c = 0; c < C; ++c) {
-        const int bc = (col0 + c < n) ? la.b[col0 + c] : 0;
-        H[c] = 0u; acc[c] = 0u; bca[c] = sbase + 4u * (uint32_t)bc;
-    }
-    uint32_t last0 = 0u, last1 = 0u, prev_recv1 = 0u;       // last column of the two rows of the previous step; recv1 of the previous step
-    long long full = 0;
-    const unsigned long long *bin = w > 0 ? (const unsigned long long *)la.bound + (size_t)(w - 1) * m : nullptr;
-    unsigned long long *bout = (unsigned long long *)la.bound + (size_t)w * m;
-    const bool publish = (w + 1 < la.n_panels);
-    uint32_t *dcol = la.dirs + col0;
-    const int steps = (m + 1) / 2 + 31 + 16;        // + one block so the last rows get published
-    // source symbols of a block: rows 2(t0 - 31) .. 2(t0 + 15) + 1 (94 rows), three per lane, fetched one block ahead
-    auto fetch = [&](int t0, int q) -> uint8_t { const int r = 2 * (t0 - 31) + lane + 32 * q; return ((unsigned)r < (unsigned)m) ? la.a[r] : (uint8_t)0; };
-    uint8_t pf0 = fetch(0, 0), pf1 = fetch(0, 1), pf2 = fetch(0, 2);
-
-#pragma unroll 1
-    for (int t0 = 0; t0 < steps; t0 += 16) {
-        const uint32_t last_at_block_start = last1;
-        if (publish) {
-            const int r = 2 * (t0 - 47) + lane;
-            if (r >= 0 && r < m) st_cg_u64(bout + r, (1ull << 32) | (unsigned long long)s_pub[lane]);
-        }
-        __syncwarp();
-        uint32_t bval = 0u;
-        if (w > 0) {
-            const bool mine = 2 * t0 + lane < m;
-            unsigned long long raw = 0ull;
-            do {
-                if (mine) raw = ld_poll_u64(bin + 2 * t0 + lane);
-            } while (!__all_sync(RSD_FULL, raw != RSD_LONG_SENTINEL));      // warp-uniform exit (see k_long_fwd)
-            bval = (uint32_t)raw;
-        }
-        // codes0 / codes1: 16 nibbles each = the table rows of this lane's first / second row in the 16 steps
-        unsigned long long codes0 = 0ull, codes1 = 0ull;
-        {
-            s_a[lane] = pf0; s_a[32 + lane] = pf1; s_a[64 + lane] = pf2;
-            pf0 = fetch(t0 + 16, 0); pf1 = fetch(t0 + 16, 1); pf2 = fetch(t0 + 16, 2);
-            __syncwarp();
-#pragma unroll
-            for (int k = 0; k < 16; ++k) {
-                const uint32_t two = *reinterpret_cast<const uint16_t *>(s_a + 2 * (31 - lane + k));
-                codes0 |= (unsigned long long)(two & 15u) << (4 * k);
-                codes1 |= (unsigned long long)((two >> 8) & 15u) << (4 * k);
-            }
-            __syncwarp();
-        }
-        auto run16 = [&](auto steady_tag) {
-        constexpr bool STEADY = decltype(steady_tag)::value;
-#pragma unroll 2
-        for (int k = 0; k < 16; ++k) {
-            const int i0 = 2 * (t0 + k - lane);
-            const bool on0 = STEADY || (strip_on && (unsigned)i0 < (unsigned)m);
-            const bool on1 = STEADY || (strip_on && (unsigned)(i0 + 1) < (unsigned)m);
-            const uint32_t off0 = ((uint32_t)(codes0 >> (4 * k)) & 15u) << 6, off1 = ((uint32_t)(codes1 >> (4 * k)) & 15u) << 6;
-            uint32_t w0[C], w1[C];
-#pragma unroll
-            for (int c = 0; c < C; ++c) {
-                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w0[c]) : "r"(bca[c] + off0));
-                asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w1[c]) : "r"(bca[c] + off1));
-            }
-            // first row, the part that does not involve the left neighbour
-            uint32_t t2a[C]; int e1a[C];
-            {
-                uint32_t diag = prev_recv1;
-#pragma unroll
-                for (int c = 0; c < C; ++c) {
-                    const uint32_t up = H[c];
-                    const uint32_t x = diag + w0[c];
-                    e1a[c] = (int)(x - up);
-                    t2a[c] = up + (uint32_t)min(e1a[c], 0);
-                    diag = up;
-                }
-            }
-            uint32_t recv0 = __shfl_up_sync(RSD_FULL, last0, 1);
-            uint32_t recv1 = __shfl_up_sync(RSD_FULL, last1, 1);
-            const uint32_t b0 = __shfl_sync(RSD_FULL, bval, 2 * k), b1 = __shfl_sync(RSD_FULL, bval, 2 * k + 1);
-            if (lane == 0) { recv0 = w > 0 ? b0 : 0u; recv1 = w > 0 ? b1 : 0u; }
-            if (on0) {
-                uint32_t left = recv0, h0[C];
-#pragma unroll
-                for (int c = 0; c < C; ++c) {
-                    const int e2 = (int)(t2a[c] - left);
-                    h0[c] = t2a[c] + (uint32_t)__viaddmin_s32((int)left, -(int)t2a[c], 0);
-                    left = h0[c];
-                    acc[c] = __funnelshift_l((uint32_t)e2, acc[c], 1);
-                    acc[c] = __funnelshift_l((uint32_t)e1a[c], acc[c], 1);
-                }
-                last0 = left;
-                if (on1) {
-                    uint32_t diag = recv0, left1 = recv1;
-#pragma unroll
-                    for (int c = 0; c < C; ++c) {
-                        const uint32_t up = h0[c];
-                        const uint32_t x = diag + w1[c];
-                        const int e1 = (int)(x - up);
-                        const uint32_t t2 = up + (uint32_t)min(e1, 0);
-                        const int e2 = (int)(t2 - left1);
-                        const uint32_t hn = t2 + (uint32_t)__viaddmin_s32((int)left1, -(int)t2, 0);
-                        diag = up; H[c] = hn; left1 = hn;
-                        acc[c] = __funnelshift_l((uint32_t)e2, acc[c], 1);
-                        acc[c] = __funnelshift_l((uint32_t)e1, acc[c], 1);
-                    }
-                    last1 = left1;
-                } else {
-#pragma unroll
-                    for (int c = 0; c < C; ++c) H[c] = h0[c];
-                    last1 = last0;                              // the panel's running last column (only used for the key tracking)
-                }
-                prev_recv1 = recv1;
-                const int il = on1 ? i0 + 1 : i0;               // last row done in this step
-                if ((il & 15) == 15 || il == m - 1) {
-                    const int sh = 2 * (15 - (il & 15));
-                    if constexpr (C >= 4) {
-                        uint4 *dst = reinterpret_cast<uint4 *>(dcol + (size_t)(il >> 4) * la.n_pad);
-#pragma unroll
-                        for (int c = 0; c < C; c += 4)
-                            dst[c >> 2] = make_uint4(acc[c] << sh, acc[c + 1] << sh, acc[c + 2] << sh, acc[c + 3] << sh);
-                    } else {
-                        *reinterpret_cast<uint2 *>(dcol + (size_t)(il >> 4) * la.n_pad) = make_uint2(acc[0] << sh, acc[1] << sh);
-                    }
-                }
-            }
-            if (lane == 31) { s_pub[2 * k] = last0; s_pub[2 * k + 1] = last1; }
-        }
-        };
-        if (2 * (t0 - 31) >= 0 && 2 * (t0 + 15) + 1 <= m - 1) run16(std::true_type{}); else run16(std::false_type{});
-        __syncwarp();
-        full += (long long)(int)(last1 - last_at_block_start);          // <= 32 bounded row-to-row differences (host check)
-    }
-    if (strip_on && col0 <= n - 1 && n - 1 < col0 + C) {
-        const int cl = (n - 1) - col0;
-        uint32_t res = 0u;
-#pragma unroll
-        for (int c = 0; c < C; ++c) if (c == cl) res = H[c];
-        const long long hkey = full + (long long)(int)(res - H[C - 1]);
-        const long long key = hkey + (long long)m * (((long long)icp->del << la.S) + 1) + (long long)n * (((long long)icp->ins << la.S) + 1);
-        la.dist[0] = (double)(key >> la.S) / (double)(1 << icp->scale_log2);
     }
 }
 
@@ -593,34 +261,5 @@ __global__ void __launch_bounds__(32) k_long_traceback(int m, int n, const uint3
         while (j > 0) { tmp[--pos] = 0; --j; }
         while (i > 0) { tmp[--pos] = 1; --i; }
         n_ops[0] = m + n - pos;
-    }
-}
-
-// packed script of the single pair: op + entered cell via two block scans (same as k_finalize, unpacked input)
-__global__ void __launch_bounds__(1024) k_long_emit(const uint8_t *__restrict__ tmp, int m, int n, const int32_t *__restrict__ n_ops,
-                                                    uint8_t *__restrict__ op, int32_t *__restrict__ oi, int32_t *__restrict__ oj) {
-    __shared__ int s_ai[1024], s_bj[1024];
-    __shared__ int carry_i, carry_j;
-    const int tid = threadIdx.x;
-    const int k_ops = n_ops[0];
-    const uint8_t *src = tmp + ((int64_t)m + n - k_ops);
-    if (tid == 0) { carry_i = 0; carry_j = 0; }
-    __syncthreads();
-    for (int base = 0; base < k_ops; base += 1024) {
-        const int k = base + tid;
-        const int o = k < k_ops ? src[k] : 3;
-        s_ai[tid] = (o == 1 || o == 2); s_bj[tid] = (o == 0 || o == 2);
-        __syncthreads();
-        for (int off = 1; off < 1024; off <<= 1) {
-            int xi = tid >= off ? s_ai[tid - off] : 0, xj = tid >= off ? s_bj[tid - off] : 0;
-            __syncthreads();
-            s_ai[tid] += xi; s_bj[tid] += xj;
-            __syncthreads();
-        }
-        const int vi = carry_i + s_ai[tid], vj = carry_j + s_bj[tid];
-        if (k < k_ops) { op[k] = (uint8_t)o; if (oi) oi[k] = vi; if (oj) oj[k] = vj; }
-        __syncthreads();
-        if (tid == 1023) { carry_i = vi; carry_j = vj; }
-        __syncthreads();
     }
 }

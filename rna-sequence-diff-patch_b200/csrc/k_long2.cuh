@@ -1,5 +1,11 @@
-// k_long2.cuh — long pairs, second generation: the panel pipeline of k_long.cuh (k_long_fwd32x2: 32-bit modular
-// keys, two rows per step) as a *job* kernel, so that one cooperative launch can carry
+// k_long2.cuh — long pairs (>= a few kb per side; BASELINE config 4: 50 kb x 50 kb with traceback) on 32-bit keys.
+//
+// Block-tiled diagonal wavefront: the matrix is cut into column panels of 32*C columns; panel w is owned by one warp (one
+// warp per CTA, so panels spread over all SMs) and, inside the panel, lane s owns C columns in registers and advances two
+// rows per step (a 2 x C register tile).  The right-most column of panel w streams through a global boundary array to
+// panel w+1, which follows one block behind; all CTAs are co-resident (cooperative launch), so the waits cannot deadlock.
+// Keys are the (cost << S | steps) keys of k_script.cuh, modulo 2^32 (see long2_panel).  It is a *job* kernel, so that
+// one cooperative launch can carry
 //   * several pairs at once (BASELINE config 4 is a batch of 50 kb pairs): the CTAs of a *ring* run panel w of
 //     one pair after the other, so the pipeline fill of pair k+1 overlaps the drain of pair k, and several rings
 //     side by side give every SM scheduler more than one warp;
@@ -47,16 +53,17 @@ struct LongLaunch2 {
     int ring_cta0[RSD_LONG2_MAX_RINGS + 1];        // CTAs [ring_cta0[g], ring_cta0[g+1]) form ring g
 };
 
-// One panel of one job: rows r0 .. r1-1 of the 32*C columns of panel w.  Same arithmetic as k_long_fwd32x2.
+// One panel of one job: rows r0 .. r1-1 of the 32*C columns of panel w.
 //
-// REL: keys are held *relative to a per-lane base* (a lane's keys, and those its left neighbour hands over, lie within
-// (C + 34) border steps of each other — the host checks that this stays below 2^30), so they can be compared as plain
-// signed integers instead of through wrapped differences: min(left, up, diag + w) is one VIMNMX3 (distance only) or two
-// VIMNMX with the two differences for the direction bits, and the chain from a cell to its right neighbour is one
-// instruction instead of VIADDMNMX + IADD — what a lone warp per scheduler waits on.  The base moves to the lane's
-// first column at every block start; values cross lanes with the difference of the two bases added, and everything
-// written to memory (boundary columns, checkpoint rows) is the absolute key modulo 2^32 as before.
-template <int C, bool DIRS, bool REL>
+// The (cost << S | steps) key of a 50 kb pair needs ~36 bits.  Everything written to memory (boundary columns, checkpoint
+// rows) is the key modulo 2^32.  In registers keys are held *relative to a per-lane base* (a lane's keys, and those its
+// left neighbour hands over, lie within (C + 34) border steps of each other — the host checks that this stays below
+// 2^30), so they compare as plain signed integers: min(left, up, diag + w) is one VIMNMX3 (distance only) or two VIMNMX
+// with the two differences for the direction bits (their sign bits, as in k_script_fwd), and the chain from a cell to its
+// right neighbour is one instruction — what a lone warp per scheduler waits on.  The base moves to the lane's first
+// column at every block start; values cross lanes with the difference of the two bases added.  The exact key of cell
+// (m, n), needed for the distance, is rebuilt from bounded row-to-row differences of the lane's last column (`full`).
+template <int C, bool DIRS>
 __device__ __forceinline__ void long2_panel(const LongJob2 &J, const int w, const int lane, const IntCosts *__restrict__ icp,
                                             uint32_t *s_w, uint32_t *s_pub, uint8_t *s_a) {
     __syncwarp();
@@ -77,13 +84,10 @@ __device__ __forceinline__ void long2_panel(const LongJob2 &J, const int w, cons
         H[c] = J.top ? __ldcg(J.top + col0 + c) : 0u; acc[c] = 0u; bca[c] = sbase + 4u * (uint32_t)bc;
     }
     uint32_t prev_recv1 = (J.top && col0 > 0) ? __ldcg(J.top + col0 - 1) : 0u;       // key of (row r0, the column left of this strip)
-    uint32_t base = 0u, d_nb = 0u;                     // REL: this lane's base; left neighbour's base minus this one
-    if constexpr (REL) {
-        base = H[0];
+    uint32_t base = H[0], d_nb = 0u;                   // this lane's base; left neighbour's base minus this one
 #pragma unroll
-        for (int c = 0; c < C; ++c) H[c] -= base;
-        prev_recv1 -= base;
-    }
+    for (int c = 0; c < C; ++c) H[c] -= base;
+    prev_recv1 -= base;
     uint32_t last0 = 0u, last1 = H[C - 1];
     long long full = 0;
     const unsigned long long *bin = w > 0 ? J.bound + (size_t)(w - 1) * J.bstride : nullptr;
@@ -102,7 +106,7 @@ __device__ __forceinline__ void long2_panel(const LongJob2 &J, const int w, cons
 
 #pragma unroll 1
     for (int t0 = 0; t0 < steps; t0 += 16) {
-        if constexpr (REL) {                           // rebase: every key this lane holds moves with its first column
+        {                                              // rebase: every key this lane holds moves with its first column
             const uint32_t delta = H[0];
             base += delta;
 #pragma unroll
@@ -166,96 +170,42 @@ __device__ __forceinline__ void long2_panel(const LongJob2 &J, const int w, cons
             uint32_t recv0 = __shfl_up_sync(RSD_FULL, last0, 1);
             uint32_t recv1 = __shfl_up_sync(RSD_FULL, last1, 1);
             const uint32_t b0 = __shfl_sync(RSD_FULL, bval, 2 * k), b1 = __shfl_sync(RSD_FULL, bval, 2 * k + 1);
-            if constexpr (REL) { recv0 += d_nb; recv1 += d_nb; }
-            if (lane == 0) { recv0 = (w > 0 ? b0 : 0u) - base; recv1 = (w > 0 ? b1 : 0u) - base; }       // (base == 0 unless REL)
-            if constexpr (REL) {
-                if (on0) {
-                    int left = (int)recv0, diag = (int)prev_recv1, h0[C];
-#pragma unroll
-                    for (int c = 0; c < C; ++c) {
-                        const int up = (int)H[c];
-                        const int x = diag + (int)w0[c];
-                        if constexpr (DIRS) {
-                            const int t2 = min(up, x);                        // ties keep DEL
-                            acc[c] = __funnelshift_l((uint32_t)(t2 - left), acc[c], 1);      // "not INS" (ties keep INS)
-                            acc[c] = __funnelshift_l((uint32_t)(x - up), acc[c], 1);         // then "UPD rather than DEL"
-                            h0[c] = min(left, t2);
-                        } else h0[c] = __vimin3_s32(x, up, left);
-                        diag = up; left = h0[c];
-                    }
-                    last0 = (uint32_t)left;
-                    if (on1) {
-                        int diag1 = (int)recv0, left1 = (int)recv1;
-#pragma unroll
-                        for (int c = 0; c < C; ++c) {
-                            const int up = h0[c];
-                            const int x = diag1 + (int)w1[c];
-                            int hn;
-                            if constexpr (DIRS) {
-                                const int t2 = min(up, x);
-                                acc[c] = __funnelshift_l((uint32_t)(t2 - left1), acc[c], 1);
-                                acc[c] = __funnelshift_l((uint32_t)(x - up), acc[c], 1);
-                                hn = min(left1, t2);
-                            } else hn = __vimin3_s32(x, up, left1);
-                            diag1 = up; H[c] = (uint32_t)hn; left1 = hn;
-                        }
-                        last1 = (uint32_t)left1;
-                    } else {
-#pragma unroll
-                        for (int c = 0; c < C; ++c) { H[c] = (uint32_t)h0[c]; if constexpr (DIRS) acc[c] <<= 2; }
-                        last1 = last0;
-                    }
-                    prev_recv1 = recv1;
-                } else if constexpr (DIRS && !STEADY) {
-#pragma unroll
-                    for (int c = 0; c < C; ++c) acc[c] <<= 4;
-                }
-            } else {
-            uint32_t t2a[C]; int e1a[C];
-            {
-                uint32_t diag = prev_recv1;
-#pragma unroll
-                for (int c = 0; c < C; ++c) {
-                    const uint32_t up = H[c];
-                    const uint32_t x = diag + w0[c];
-                    e1a[c] = (int)(x - up);
-                    t2a[c] = up + (uint32_t)min(e1a[c], 0);
-                    diag = up;
-                }
-            }
+            recv0 += d_nb; recv1 += d_nb;
+            if (lane == 0) { recv0 = (w > 0 ? b0 : 0u) - base; recv1 = (w > 0 ? b1 : 0u) - base; }
             if (on0) {
-                uint32_t left = recv0, h0[C];
+                int left = (int)recv0, diag = (int)prev_recv1, h0[C];
 #pragma unroll
                 for (int c = 0; c < C; ++c) {
-                    [[maybe_unused]] const int e2 = (int)(t2a[c] - left);
-                    h0[c] = t2a[c] + (uint32_t)__viaddmin_s32((int)left, -(int)t2a[c], 0);
-                    left = h0[c];
+                    const int up = (int)H[c];
+                    const int x = diag + (int)w0[c];
                     if constexpr (DIRS) {
-                        acc[c] = __funnelshift_l((uint32_t)e2, acc[c], 1);
-                        acc[c] = __funnelshift_l((uint32_t)e1a[c], acc[c], 1);
-                    }
+                        const int t2 = min(up, x);                        // ties keep DEL
+                        acc[c] = __funnelshift_l((uint32_t)(t2 - left), acc[c], 1);      // "not INS" (ties keep INS)
+                        acc[c] = __funnelshift_l((uint32_t)(x - up), acc[c], 1);         // then "UPD rather than DEL"
+                        h0[c] = min(left, t2);
+                    } else h0[c] = __vimin3_s32(x, up, left);
+                    diag = up; left = h0[c];
                 }
-                last0 = left;
+                last0 = (uint32_t)left;
                 if (on1) {
-                    uint32_t diag = recv0, left1 = recv1;
+                    int diag1 = (int)recv0, left1 = (int)recv1;
 #pragma unroll
                     for (int c = 0; c < C; ++c) {
-                        const uint32_t up = h0[c];
-                        const uint32_t x = diag + w1[c];
-                        const int e1 = (int)(x - up);
-                        const uint32_t t2 = up + (uint32_t)min(e1, 0);
-                        [[maybe_unused]] const int e2 = (int)(t2 - left1);
-                        const uint32_t hn = t2 + (uint32_t)__viaddmin_s32((int)left1, -(int)t2, 0);
-                        diag = up; H[c] = hn; left1 = hn;
+                        const int up = h0[c];
+                        const int x = diag1 + (int)w1[c];
+                        int hn;
                         if constexpr (DIRS) {
-                            acc[c] = __funnelshift_l((uint32_t)e2, acc[c], 1);
-                            acc[c] = __funnelshift_l((uint32_t)e1, acc[c], 1);
-                        }
+                            const int t2 = min(up, x);
+                            acc[c] = __funnelshift_l((uint32_t)(t2 - left1), acc[c], 1);
+                            acc[c] = __funnelshift_l((uint32_t)(x - up), acc[c], 1);
+                            hn = min(left1, t2);
+                        } else hn = __vimin3_s32(x, up, left1);
+                        diag1 = up; H[c] = (uint32_t)hn; left1 = hn;
                     }
-                    last1 = left1;
+                    last1 = (uint32_t)left1;
                 } else {
 #pragma unroll
-                    for (int c = 0; c < C; ++c) { H[c] = h0[c]; if constexpr (DIRS) acc[c] <<= 2; }      // bit positions follow the step, not the row count
+                    for (int c = 0; c < C; ++c) { H[c] = (uint32_t)h0[c]; if constexpr (DIRS) acc[c] <<= 2; }
                     last1 = last0;
                 }
                 prev_recv1 = recv1;
@@ -263,8 +213,7 @@ __device__ __forceinline__ void long2_panel(const LongJob2 &J, const int w, cons
 #pragma unroll
                 for (int c = 0; c < C; ++c) acc[c] <<= 4;
             }
-            }
-            if (lane == 31) { s_pub[2 * k] = last0 + base; s_pub[2 * k + 1] = last1 + base; }      // absolute keys (base == 0 unless REL)
+            if (lane == 31) { s_pub[2 * k] = last0 + base; s_pub[2 * k + 1] = last1 + base; }      // absolute keys
         }
         if constexpr (DIRS) {
             // the 16 rows of the last 8 steps, all lanes at once: 32 * C consecutive words of group (t0 + k8) / 8
@@ -298,7 +247,7 @@ __device__ __forceinline__ void long2_panel(const LongJob2 &J, const int w, cons
     }
 }
 
-template <int C, bool DIRS, bool REL>
+template <int C, bool DIRS>
 __global__ void __launch_bounds__(32)
 k_long2(const LongLaunch2 L, const IntCosts *__restrict__ icp) {
     __shared__ uint32_t s_w[320];
@@ -310,7 +259,7 @@ k_long2(const LongLaunch2 L, const IntCosts *__restrict__ icp) {
     const int wl = (int)blockIdx.x - L.ring_cta0[g];
     for (int j = L.ring_job0[g]; j < L.ring_job0[g + 1]; ++j) {
         const LongJob2 J = L.jobs[j];
-        if (wl < J.w_cnt) long2_panel<C, DIRS, REL>(J, J.w_lo + wl, lane, icp, s_w, s_pub, s_a);
+        if (wl < J.w_cnt) long2_panel<C, DIRS>(J, J.w_lo + wl, lane, icp, s_w, s_pub, s_a);
     }
 }
 
@@ -389,7 +338,7 @@ __global__ void __launch_bounds__(32) k_long2_traceback(const LongTb2 *__restric
     if (lane == 0) { J.state[0] = i; J.state[1] = j; J.state[2] = pos; J.state[3] = 1; }
 }
 
-// packed scripts of a batch: k_long_emit per pair
+// packed scripts: one CTA per pair, op + entered cell via two block scans (same as k_finalize, unpacked input)
 struct LongEmit2 { const uint8_t *tmp; int m, n; const int32_t *n_ops; uint8_t *op; int32_t *oi, *oj; };
 
 __global__ void __launch_bounds__(1024) k_long2_emit(const LongEmit2 *__restrict__ jobs) {

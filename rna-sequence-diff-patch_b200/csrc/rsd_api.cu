@@ -1864,25 +1864,15 @@ extern "C" int rsd_db_similarity(rsd_ctx *c, const uint8_t *q_codes, int32_t q_l
 // ------------------------------------------------------------------------------------------------
 // long pair (BASELINE config 4)
 // ------------------------------------------------------------------------------------------------
-// first generation: one pair per launch, whole direction matrix resident.  Still the path of the exact-double and fp64
-// kernels (very large or non-dyadic costs) and of the RSD_LONG_V1 / RSD_LONG_R1 / RSD_LONG_WIDE knobs.
-static int long_pair_v1(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t *b, int64_t n,
-                        int force_mode, int want_script, int64_t max_ops,
-                        uint8_t *op, int32_t *oi, int32_t *oj, int64_t *n_ops, double *dist, int *mode_out) {
-    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
-    if (m < 0 || n < 0 || (m > 0 && !a) || (n > 0 && !b) || !dist) return rsd_fail(RSD_EINVAL, "rsd_long_pair: bad arguments");
-    if (m > 0x3fffffff || n > 0x3fffffff) return rsd_fail(RSD_ERANGE, "rsd_long_pair: sequence too long");
-    if (want_script && (!op || !n_ops || max_ops < m + n)) return rsd_fail(RSD_EINVAL, "rsd_long_pair: script buffers missing or max_ops < m+n");
-    RSD_OK_OR_RETURN(c->ensure_device());
-    uint32_t symmask = 0;
-    for (int64_t i = 0; i < m; ++i) { if (a[i] > 15) return rsd_fail(RSD_EINVAL, "rsd_long_pair: code > 15"); symmask |= 1u << a[i]; }
-    for (int64_t j = 0; j < n; ++j) { if (b[j] > 15) return rsd_fail(RSD_EINVAL, "rsd_long_pair: code > 15"); symmask |= 1u << b[j]; }
+// Pairs whose keys do not fit the 32-bit keys of k_long2 (costs too large for that bound, or not dyadic) run on
+// k_long_fwd, one pair per launch with the whole direction matrix resident.  Called by rsd_long_pairs for one non-empty
+// pair whose arguments and symbols (symmask) it has checked.
+static int long_pair_wide(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t *b, int64_t n, uint32_t symmask, int force_mode,
+                          int want_script, uint8_t *op, int32_t *oi, int32_t *oj, int64_t *n_ops, double *dist, int *mode_out) {
     ModeInfo mi;
     RSD_OK_OR_RETURN(c->classify(symmask, m, n, 4, force_mode == RSD_MODE_I16X2 ? RSD_MODE_I32 : force_mode, mi));
     // integer keys (cost * 2^S + steps) are carried in doubles: they must stay below 2^52
     int S = ceil_log2_i64(m + n + 66);
-    // test knob: a wider steps field makes the 32-bit modular keys wrap on small matrices (cells with i*del + j*ins
-    // beyond 2^(31-S)), so the wrap regime of a 50 kb pair can be checked against the oracle at 3 kb
     if (const char *e = getenv("RSD_LONG_S")) S = std::min(std::max(S, atoi(e)), 30);
     bool f64 = mi.mode == RSD_MODE_F64;
     if (!f64) {
@@ -1891,38 +1881,14 @@ static int long_pair_v1(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t *
     } else if (force_mode == RSD_MODE_I32) return rsd_fail(RSD_EINVAL, "rsd_long_pair: integer mode not exact for these costs");
     if (mode_out) *mode_out = f64 ? RSD_MODE_F64 : RSD_MODE_I32;
     c->timed = false; c->last_ms_override = 0.0;
-    if (m == 0 || n == 0) {                     // border row / column only (SED:146-182): one product, all INS or all DEL
-        *dist = m == 0 ? (double)n * c->ins : (double)m * c->del;
-        if (want_script) {
-            const int64_t k = m + n;
-            for (int64_t x = 0; x < k; ++x) { op[x] = m == 0 ? 0 : 1; if (oi) oi[x] = m == 0 ? 0 : (int32_t)(x + 1); if (oj) oj[x] = m == 0 ? (int32_t)(x + 1) : 0; }
-            *n_ops = k;
-        }
-        return RSD_OK;
-    }
     cudaStream_t st = c->stream;
     RSD_OK_OR_RETURN(c->upload_costs(mi, st));
-    // 32-bit modular keys when every pair of compared candidates stays within 2^30 of each other
-    bool key32_ok = false;
-    if (!f64 && !getenv("RSD_LONG_WIDE")) {
-        long long maxc = std::max<long long>(mi.ic.ins, mi.ic.del);
-        for (int x = 0; x < 16; ++x) for (int y = 0; y < 16; ++y)
-            if ((symmask >> x & 1) && (symmask >> y & 1)) maxc = std::max<long long>(maxc, std::llabs((long long)mi.ic.w[x][y]));
-        key32_ok = S <= 24 && ((64 * maxc + 128) << S) < (1ll << 30);    // covers 32 rows of drift (the per-block key tracking)
-    }
-    // 4 columns per lane: the forward pass is latency-bound (one warp per panel, a dependent chain per
-    // row), so narrow panels = more panels in flight win until the panel pipeline lag dominates
-    // (measured at 50 kb, 32-bit keys, two rows per step: C=2 11.5 ms, C=4 7.8 ms, C=8 8.3 ms; one row per step: 12.8 / 10.5 / 10.9 ms; double-carried keys: 15.4 / 22.8 / 19.9 ms).
-    int C = 4;
-    if (const char *e = getenv("RSD_LONG_C")) { const int v = atoi(e); if (v == 4 || v == 8 || v == 16 || (v == 2 && key32_ok)) C = v; }
+    int C = 4;                                  // columns per lane
+    if (const char *e = getenv("RSD_LONG_C")) { const int v = atoi(e); if (v == 4 || v == 8 || v == 16) C = v; }
     const int n_panels = (int)((n + 32 * C - 1) / (32 * C));
     const int64_t n_pad = (int64_t)n_panels * 32 * C;
     int per_sm = 0;
-    const bool key32 = key32_ok;
-    const bool two_rows = key32 && !getenv("RSD_LONG_R1");      // 2 x C register tile per step (default) or one row per step
-    const void *kfn = two_rows ? (C == 2 ? (const void *)k_long_fwd32x2<2> : C == 4 ? (const void *)k_long_fwd32x2<4> : C == 16 ? (const void *)k_long_fwd32x2<16> : (const void *)k_long_fwd32x2<8>) :
-                      key32 ? (C == 2 ? (const void *)k_long_fwd32<2> : C == 4 ? (const void *)k_long_fwd32<4> : C == 16 ? (const void *)k_long_fwd32<16> : (const void *)k_long_fwd32<8>) :
-                      f64 ? (C == 4 ? (const void *)k_long_fwd<true, 4> : C == 16 ? (const void *)k_long_fwd<true, 16> : (const void *)k_long_fwd<true, 8>)
+    const void *kfn = f64 ? (C == 4 ? (const void *)k_long_fwd<true, 4> : C == 16 ? (const void *)k_long_fwd<true, 16> : (const void *)k_long_fwd<true, 8>)
                           : (C == 4 ? (const void *)k_long_fwd<false, 4> : C == 16 ? (const void *)k_long_fwd<false, 16> : (const void *)k_long_fwd<false, 8>);
     RSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kfn, 32, 0));
     if ((int64_t)per_sm * c->sm_count < n_panels)
@@ -1930,8 +1896,7 @@ static int long_pair_v1(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t *
                         n_panels, per_sm * c->sm_count);
     const size_t dir_words = (size_t)((m + 15) / 16) * (size_t)n_pad;
     RSD_OK_OR_RETURN(c->dirs.ensure(dir_words * 4 + 64));
-    const int64_t bstride = m;
-    RSD_OK_OR_RETURN(c->ps().scratch.ensure((size_t)n_panels * (size_t)bstride * 12 + (size_t)n_panels * 4 + 256));
+    RSD_OK_OR_RETURN(c->ps().scratch.ensure((size_t)n_panels * (size_t)m * 12 + 256));
     RSD_OK_OR_RETURN(c->mat_ab.ensure((size_t)m + n + 64));
     RSD_OK_OR_RETURN(c->out_f64.ensure(64));
     uint8_t *da = (uint8_t *)c->mat_ab.p, *db = da + ((m + 15) / 16) * 16;
@@ -1940,58 +1905,45 @@ static int long_pair_v1(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t *
     LongArgs la{};
     la.a = da; la.m = (int)m; la.b = db; la.n = (int)n; la.n_panels = n_panels; la.n_pad = (int)n_pad;
     la.dirs = (uint32_t *)c->dirs.p;
-    la.bound = c->ps().scratch.p; la.bstride = (int)bstride;
-    la.bound_steps = (int *)((unsigned char *)c->ps().scratch.p + (size_t)n_panels * (size_t)bstride * 8);
-    la.progress = (int *)((unsigned char *)c->ps().scratch.p + (size_t)n_panels * (size_t)bstride * 12);
+    la.bound = c->ps().scratch.p;
+    la.bound_steps = (int *)((unsigned char *)c->ps().scratch.p + (size_t)n_panels * (size_t)m * 8);
     la.dist = (double *)c->out_f64.p;
     la.S = S;
-    la.dbg = nullptr;
-    const bool ltrace = getenv("RSD_TRACE") != nullptr;
-    if (ltrace) { RSD_OK_OR_RETURN(c->misc.ensure((size_t)n_panels * 64)); la.dbg = (unsigned long long *)c->misc.p; }
-    RSD_CUDA(cudaMemsetAsync(la.bound, 0x80, (size_t)n_panels * (size_t)bstride * 8, st));      // sentinel = "not published yet"
-    RSD_CUDA(cudaMemsetAsync(la.progress, 0, sizeof(int) * (size_t)n_panels, st));              // [0] doubles as the watchdog's error flag
-    const IntCosts *dic = c->d_ic; const F64Costs *dfc = c->d_fc;
-    void *args[] = {&la, &dic, &dfc};
-    void *args32[] = {&la, &dic};
-    if (c->timing) RSD_CUDA(cudaEventRecord(c->ev0, st));
-    RSD_CUDA(cudaLaunchCooperativeKernel(kfn, dim3(n_panels), dim3(32), key32 ? args32 : args, 0, st));
-    c->launches += 1;
+    RSD_CUDA(cudaMemsetAsync(la.bound, 0x80, (size_t)n_panels * (size_t)m * 8, st));      // sentinel = "not published yet"
     if (want_script) {
         RSD_OK_OR_RETURN(c->s_tmp.ensure((size_t)(m + n) + 64));
         RSD_OK_OR_RETURN(c->s_nops.ensure(64));
         RSD_OK_OR_RETURN(c->s_op.ensure((size_t)(m + n) + 64));
         if (oi) RSD_OK_OR_RETURN(c->s_oi.ensure(sizeof(int32_t) * (size_t)(m + n) + 64));
         if (oj) RSD_OK_OR_RETURN(c->s_oj.ensure(sizeof(int32_t) * (size_t)(m + n) + 64));
+        RSD_OK_OR_RETURN(c->long_jobs.ensure(sizeof(LongEmit2)));
+        const LongEmit2 em{(const uint8_t *)c->s_tmp.p, (int)m, (int)n, (const int32_t *)c->s_nops.p, (uint8_t *)c->s_op.p,
+                           oi ? (int32_t *)c->s_oi.p : nullptr, oj ? (int32_t *)c->s_oj.p : nullptr};
+        RSD_CUDA(cudaMemcpyAsync(c->long_jobs.p, &em, sizeof em, cudaMemcpyHostToDevice, st));
+    }
+    const IntCosts *dic = c->d_ic; const F64Costs *dfc = c->d_fc;
+    void *args[] = {&la, &dic, &dfc};
+    if (c->timing) RSD_CUDA(cudaEventRecord(c->ev0, st));
+    RSD_CUDA(cudaLaunchCooperativeKernel(kfn, dim3(n_panels), dim3(32), args, 0, st));
+    c->launches += 1;
+    if (want_script) {
         k_long_traceback<<<1, 32, 0, st>>>((int)m, (int)n, (const uint32_t *)c->dirs.p, (int)n_pad, (uint8_t *)c->s_tmp.p, (int32_t *)c->s_nops.p);
-        k_long_emit<<<1, 1024, 0, st>>>((const uint8_t *)c->s_tmp.p, (int)m, (int)n, (const int32_t *)c->s_nops.p, (uint8_t *)c->s_op.p,
-                                        oi ? (int32_t *)c->s_oi.p : nullptr, oj ? (int32_t *)c->s_oj.p : nullptr);
+        k_long2_emit<<<1, 1024, 0, st>>>((const LongEmit2 *)c->long_jobs.p);
         c->launches += 2;
     }
     if (c->timing) { RSD_CUDA(cudaEventRecord(c->ev1, st)); c->timed = true; }
     RSD_CUDA(cudaGetLastError());
     RSD_CUDA(cudaMemcpyAsync(dist, c->out_f64.p, sizeof(double), cudaMemcpyDeviceToHost, st));
-    int32_t stalled = 0;
-    RSD_CUDA(cudaMemcpyAsync(&stalled, la.progress, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (ltrace) {
-        std::vector<unsigned long long> d((size_t)n_panels * 8);
-        RSD_CUDA(cudaMemcpyAsync(d.data(), la.dbg, d.size() * 8, cudaMemcpyDeviceToHost, st));
-        RSD_CUDA(cudaStreamSynchronize(st));
-        for (int w2 = 0; w2 < n_panels; w2 += (w2 < 4 ? 1 : std::max(1, n_panels / 8)))
-            fprintf(stderr, "[rsd trace] panel %d: start +%.3f ms, end +%.3f ms, Mclk: poll %.3f publish %.3f a-loads %.3f rows %.3f\n", w2,
-                    (d[w2 * 8] - d[0]) * 1e-6, (d[w2 * 8 + 1] - d[0]) * 1e-6, d[w2 * 8 + 2] * 1e-6, d[w2 * 8 + 3] * 1e-6, d[w2 * 8 + 4] * 1e-6, d[w2 * 8 + 5] * 1e-6);
-    }
-    int32_t k32 = 0;
     if (want_script) {
+        int32_t k32 = 0;
         RSD_CUDA(cudaMemcpyAsync(&k32, c->s_nops.p, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
         RSD_CUDA(cudaStreamSynchronize(st));
-        if (stalled < 0) return rsd_fail(RSD_ECUDA, "rsd_long_pair: the panel pipeline stalled; no result");
         *n_ops = k32;
         RSD_CUDA(cudaMemcpyAsync(op, c->s_op.p, (size_t)k32, cudaMemcpyDeviceToHost, st));
         if (oi) RSD_CUDA(cudaMemcpyAsync(oi, c->s_oi.p, sizeof(int32_t) * (size_t)k32, cudaMemcpyDeviceToHost, st));
         if (oj) RSD_CUDA(cudaMemcpyAsync(oj, c->s_oj.p, sizeof(int32_t) * (size_t)k32, cudaMemcpyDeviceToHost, st));
     }
     RSD_CUDA(cudaStreamSynchronize(st));
-    if (stalled < 0) return rsd_fail(RSD_ECUDA, "rsd_long_pair: the panel pipeline stalled; no result");
     return RSD_OK;
 }
 

@@ -103,7 +103,7 @@ def test_c4_canonical_script_equals_oracle_digest(R, eng, golden, c4_digest):
 def test_c4_other_kernel_variants_equal_oracle_digest(R, eng, golden, c4_digest, monkeypatch):
     a, b = c4_pair()
     eng.set_costs(golden["default_costs"])
-    for env in ({"RSD_LONG_R1": "1"}, {"RSD_LONG_WIDE": "1"}, {"RSD_LONG_C": "8"}):
+    for env in ({"RSD_LONG_WIDE": "1"}, {"RSD_LONG_C": "8"}):
         for k, v in env.items():
             monkeypatch.setenv(k, v)
         _check_digest(eng.long_pair(a, b), c4_digest["c4_default_costs"])
@@ -165,8 +165,8 @@ def test_c4_shape_properties(R, eng, golden):
 
 
 def test_wide_key_fallback_paths_agree(R, eng, golden, monkeypatch):
-    """The 32-bit modular-key kernel is the default; the double-carried integer key kernel stays as the
-    fallback (forced here through RSD_LONG_WIDE, and reached naturally by costs too large for the 32-bit bound)."""
+    """The 32-bit key kernel (k_long2) is the default; the double-carried integer key kernel is the fallback, forced
+    here through RSD_LONG_WIDE and reached naturally by costs too large for the 32-bit bound."""
     rng = np.random.default_rng(77)
     a = rng.integers(0, 4, size=2600, dtype=np.uint8)
     b = mutate_codes(rng, a)
@@ -177,10 +177,7 @@ def test_wide_key_fallback_paths_agree(R, eng, golden, monkeypatch):
     monkeypatch.setenv("RSD_LONG_WIDE", "1")
     wide = eng.long_pair(a, b)
     monkeypatch.delenv("RSD_LONG_WIDE")
-    monkeypatch.setenv("RSD_LONG_R1", "1")                      # 32-bit keys, one row per step
-    one_row = eng.long_pair(a, b)
-    monkeypatch.delenv("RSD_LONG_R1")
-    for res in (fast, wide, one_row):
+    for res in (fast, wide):
         assert res["mode"] == 2 and res["dist"] == d
         assert np.array_equal(res["op"], ops) and np.array_equal(res["oi"], oi) and np.array_equal(res["oj"], oj)
     # integer costs in the thousands: (32 * maxc + 64) << S exceeds 2^30 -> the wide kernel is chosen by the library

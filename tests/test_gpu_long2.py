@@ -66,7 +66,8 @@ def test_batch_of_pairs_vs_oracle(R, eng, golden, monkeypatch, rings):
 
 def test_batch_with_empty_and_mixed_alphabets(R, eng, golden):
     """empty sides are answered on the host (border row / column, SED:146-182); an ACGU+N pair puts the whole call on
-    the x4 dyadic scale of the default table; a full-IUPAC pair (0.66 / 0.83: not dyadic) sends the call to the fp64 kernels"""
+    the x4 dyadic scale of the default table; next to a full-IUPAC pair (0.66 / 0.83: not dyadic) only that pair goes to
+    the fp64 kernel, the ACGU pair keeps the integer keys of its own symbols"""
     costs = golden["default_costs"]
     eng.set_costs(costs)
     e = np.zeros(0, np.uint8)
@@ -83,7 +84,7 @@ def test_batch_with_empty_and_mixed_alphabets(R, eng, golden):
     assert res[5]["dist"] == 0.0 and res[5]["op"].shape[0] == 0
     iupac = make_pairs(8, [(800, 820)], alpha=15)
     res = eng.long_pairs(pairs[:1] + iupac)
-    assert res[1]["mode"] == 3
+    assert res[0]["mode"] == 2 and res[1]["mode"] == 3
     check(res[0], *pairs[0], costs)
     check(res[1], *iupac[0], costs)
 
@@ -116,7 +117,10 @@ def test_overflow_path_in_the_wrap_regime(R, eng, golden, monkeypatch):
     costs = golden["user_costs"]
     eng.set_costs(costs)
     for a, b in make_pairs(77, [(3000, 3000), (2500, 3300)]):
-        check(eng.long_pair(a, b), a, b, costs)
+        res = eng.long_pair(a, b)
+        assert res["mode"] == 2
+        check(res, a, b, costs)
+        check(eng.long_pair(a, b, want_script=False), a, b, costs, script=False)
 
 
 def test_overflow_budget_too_small_is_an_error(R, eng, golden, monkeypatch):
@@ -150,19 +154,42 @@ def test_overflow_path_equals_one_launch_at_60kb(R, eng, golden, monkeypatch):
             monkeypatch.delenv(k)
 
 
-def test_wrapped_difference_kernels_stay_under_test(R, eng, golden, monkeypatch):
-    """The default kernels hold keys relative to a per-lane base (plain signed compares); the wrapped-difference kernels
-    they replace remain the path for wide keys (RSD_LONG_NOREL forces them): batch, overflow blocks and the wrap regime."""
-    monkeypatch.setenv("RSD_LONG_NOREL", "1")
-    pairs = make_pairs(404, SHAPES[:6])
-    for costs in (golden["default_costs"], golden["user_costs"]):
-        eng.set_costs(costs)
-        for r, (a, b) in zip(eng.long_pairs(pairs), pairs):
-            check(r, a, b, costs)
-    monkeypatch.setenv("RSD_LONG_BUDGET_MB", "2")
-    monkeypatch.setenv("RSD_LONG_S", "21")           # user costs: still inside the 32-bit bound, absolute keys wrap
-    a, b = pairs[0]
-    res = eng.long_pair(a, b)
-    assert res["mode"] == 2
-    check(res, a, b, costs)
-    check(eng.long_pair(a, b, want_script=False), a, b, costs, script=False)
+def _long_batches(err):
+    return sum("long batch:" in line for line in err.splitlines())
+
+
+@pytest.mark.parametrize("script", [True, False])
+def test_mixed_symbol_batch_runs_each_pair_on_its_own_symbols(R, eng, golden, monkeypatch, capfd, script):
+    """A call's cost tables cover the symbols of all its pairs.  A pair that does not fit the 32-bit keys on those tables
+    is planned again on its own symbols: it runs on k_long2 when it fits there (one RSD_TRACE 'long batch:' line per
+    k_long2 batch), and only a pair that does not fit alone goes to the exact-double / fp64 kernel."""
+    monkeypatch.setenv("RSD_TRACE", "1")
+    # (a) default table: the full-IUPAC pair is not dyadic (fp64); each ACGU pair runs alone on k_long2
+    costs = golden["default_costs"]
+    acgu = make_pairs(31, [(3000, 3100), (2000, 2100)])
+    iupac = make_pairs(32, [(1500, 1600)], alpha=15)
+    eng.set_costs(costs)
+    capfd.readouterr()
+    res = eng.long_pairs(acgu + iupac, want_script=script)
+    err = capfd.readouterr().err
+    assert [r["mode"] for r in res] == [2, 2, 3]
+    assert _long_batches(err) == 2, err[-600:]
+    for r, (a, b) in zip(res, acgu + iupac):
+        check(r, a, b, costs, script=script)
+    # (b) integer table where substitutions involving N cost thousands: the ACGU+N pair needs the exact-double kernel
+    # (still integer keys: mode 2), the ACGU pair fits the 32-bit keys of its own symbols
+    def sub(x, y):
+        return 0.0 if x == y else 4000.0 + (x + y).count("A") if "N" in (x, y) else 1.0
+    big_n = {"insert": 1.0, "delete": 1.0, "update": {x: {y: sub(x, y) for y in O.SYMBOLS} for x in O.SYMBOLS}}
+    rng = np.random.default_rng(33)
+    (a0, b0), = make_pairs(34, [(3000, 3000)])
+    with_n = rng.integers(0, 4, size=2500, dtype=np.uint8); with_n[::41] = 14
+    pairs = [(a0, b0), (with_n, mutate_codes(rng, with_n))]
+    eng.set_costs(big_n)
+    capfd.readouterr()
+    res = eng.long_pairs(pairs, want_script=script)
+    err = capfd.readouterr().err
+    assert [r["mode"] for r in res] == [2, 2]
+    assert _long_batches(err) == 1, err[-600:]
+    for r, (a, b) in zip(res, pairs):
+        check(r, a, b, big_n, script=script)

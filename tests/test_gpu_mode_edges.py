@@ -248,16 +248,13 @@ def long_pairs_3000():
     return [(np.array(E.codes_of(x), np.uint8), np.array(E.codes_of(y), np.uint8)) for x, y in zip(a, b)]
 
 
-@pytest.mark.parametrize("norel", [False, True])
 @pytest.mark.parametrize("lanes", [4, 8, 16])
-def test_long_pair_key32_edge(R, eng, monkeypatch, capfd, norel, lanes):
+def test_long_pair_key32_edge(R, eng, monkeypatch, capfd, lanes):
     """3000 x 3000 (S = 13): maxc = 2045 (ins 1022, del 1023) is the largest the 32-bit keys allow and runs k_long2
-    (relative and wrapped-difference keys, 4 / 8 / 16 columns per lane); maxc = 2046 runs the exact-double fallback.
+    (4 / 8 / 16 columns per lane); maxc = 2046 runs the exact-double fallback.
     The path shows in the RSD_TRACE output: only k_long2 batches print a 'long batch:' line."""
     monkeypatch.setenv("RSD_TRACE", "1")
     monkeypatch.setenv("RSD_LONG_C", str(lanes))
-    if norel:
-        monkeypatch.setenv("RSD_LONG_NOREL", "1")
     pairs = long_pairs_3000()
     for (ins, dele), want32 in (((1022, 1023), True), ((1023, 1023), False)):
         costs = E.table(ins, dele, LONG_SUBS)

@@ -11,10 +11,6 @@ L = int(os.environ.get("L", 50000))
 pairs = [c4_pair(seed=20260004 + k, m=L) for k in range(int(os.environ.get("NPAIRS", 16)))]
 eng = R.Engine(0); eng.set_costs(cost_tables.default_costs()); eng.set_timing(True)
 single = eng.long_pair(*pairs[0])
-os.environ["RSD_LONG_V1"] = "1"
-for rep in range(3):
-    eng.long_pair(*pairs[0]); print("first-generation kernel (k_long_fwd32x2), one pair: forward", round(eng.last_kernel_ms(), 3), "ms incl. traceback", flush=True)
-del os.environ["RSD_LONG_V1"]
 # (pairs, rings, columns per lane); 0 = the library's own choice
 configs = [(1, 0, 0), (1, 1, 4), (1, 1, 8), (1, 1, 16), (2, 0, 0), (2, 2, 8), (2, 2, 16), (4, 0, 0), (4, 4, 8), (4, 4, 16), (8, 0, 0), (8, 8, 8), (8, 8, 16),
            (12, 0, 0), (12, 12, 8), (12, 12, 16), (16, 0, 0), (16, 16, 8), (16, 16, 16)]
