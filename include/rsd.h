@@ -50,7 +50,7 @@ enum {
     RSD_ECUDA = 3,      /* a CUDA call failed                                        */
     RSD_ENOMEM = 4,     /* device or host allocation failed                          */
     RSD_ECOSTS = 5,     /* costs out of contract: negative, NaN or infinite          */
-    RSD_ERANGE = 6      /* sequence too long for this entry point                    */
+    RSD_ERANGE = 6      /* sequence too long for this entry point, or output > cap   */
 };
 
 enum {                  /* numeric mode actually used, reported through *mode_out    */
@@ -186,6 +186,19 @@ int rsd_db_search_topk_dev(rsd_ctx *ctx, const uint32_t *q_words_dev, const int6
                            const int32_t *q_len_dev, int64_t n_queries, int64_t max_qlen, int bits,
                            uint32_t q_symmask, int k, int force_mode,
                            int64_t *top_idx_dev, double *top_score_dev, int *mode_out, void *stream);
+/* Range search: replaces the wf_score scan of search_collection (IR:466-477) followed by a filter on
+ * the distance.  For each query q (caller order): every record r of this shard with D(q, r) <= max_dist,
+ * D being the fp64 value rsd_distance_batch returns for (source = query, destination = record); the
+ * bound is inclusive and exact (integer modes compare the scaled distance with floor(max_dist * 2^k)).
+ * CSR output, each query's hits by global index ascending: hit_off[n_queries + 1], hit_idx[total]
+ * (global index), hit_dist[total] = D.  cap is the length of hit_idx / hit_dist: more hits than cap
+ * return RSD_ERANGE with hit_off complete (the total is hit_off[n_queries]) and the hit arrays
+ * unspecified.  max_dist must be >= 0 and not NaN (+inf: every record).  force_mode / mode_out as
+ * in rsd_db_search_topk. */
+int rsd_db_search_range(rsd_ctx *ctx, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
+                        int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, double max_dist,
+                        int force_mode, int64_t cap, int64_t *hit_off, int64_t *hit_idx, double *hit_dist,
+                        int *mode_out);
 /* Set / multiset / TF-vector similarity of one query against the loaded database — the other scorers
  * of search_collection (IRMethods.py:443-477 with the measures of IRMethods.py:49-389; documents'
  * 'tf' vectors are rebuilt on the device from the sequences, what fa_import.py:49 stores).  `method`
@@ -226,6 +239,13 @@ int rsd_multi_db_free(rsd_multi *m);
 int rsd_multi_db_search_topk(rsd_multi *m, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
                              int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, int k, int force_mode,
                              int64_t *top_idx, double *top_score, double *all_scores, int *mode_out);
+/* like rsd_db_search_range (which replaces the wf_score scan of search_collection, IR:466-477, followed
+ * by a filter on the distance), over the whole database: each device searches its shard, and the hits of
+ * a query are the shards' hits in shard order; cap / RSD_ERANGE apply to the total */
+int rsd_multi_db_search_range(rsd_multi *m, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
+                              int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, double max_dist,
+                              int force_mode, int64_t cap, int64_t *hit_off, int64_t *hit_idx, double *hit_dist,
+                              int *mode_out);
 int64_t rsd_multi_launch_count(rsd_multi *m);
 
 /* ---- long pairs (>= ~10 kb): block-tiled wavefront with traceback ----------------------------

@@ -12,10 +12,14 @@
 //   table comes from shared memory with one broadcast LDS.64, and each packed cell is
 //   PRMT (both records' v) + IMAD (packed add, fma pipe) + VIMNMX3.U16x2.
 //   The record's selector registers are built once and reused for every query of the batch.
+// Two epilogues share that body (template RANGE):
 // Top-k: a candidate passes when its key (score desc, global index asc) is not worse than the
 //   current k-th best key of its query (tau).  tau starts at "accept all" and is tightened after
 //   every chunk by k_topk_fold, which also keeps the running top-k list.  The final order is a
 //   total order on (score, index), so the result does not depend on atomic ordering.
+// Range: every record whose scaled integer distance is <= floor(max_dist * 2^k) is appended as (key, D),
+//   key = (query in batch << 32) | (global index - base); no threshold state, no fold.  The append order
+//   depends on the atomics, so each batch's hits are sorted by key on the device (cub radix sort).
 #pragma once
 #include <type_traits>
 #include "k_dist.cuh"
@@ -37,12 +41,23 @@ struct TopkState {
     int k;
 };
 
+// hits of a range search (one query batch): the count may pass cap, the batch then reruns with a larger buffer
+struct RangeHits {
+    unsigned long long *keys;              // [cap] (query in batch << 32) | (global index - base)
+    double *dist;                          // [cap] D
+    unsigned long long *n;                 // hits appended (may exceed cap)
+    int64_t cap;
+    int thr;                               // fast kernel: floor(max_dist * 2^k), clamped to INT_MAX
+    double max_dist;                       // general path: compared with the fp64 distance
+};
+
 // rowtab[q][i] = 8 bytes: v(query symbol i of q, compact symbol 0..6) = max(0, -w) <= 127; byte 7 (PAD) = 0
+template <bool RANGE>
 __global__ void __launch_bounds__(128)
 k_search_twin16(const uint32_t *__restrict__ db_words, const int64_t *__restrict__ db_start,
                 const int32_t *__restrict__ db_len, int64_t rec0, int64_t n_rec, int db_bits,
                 const int64_t *__restrict__ perm, int64_t global_base, const uint2 *__restrict__ rowtab, int QROWS, const int32_t *__restrict__ q_len, int n_queries,
-                SearchTab tab, TopkState tk, double *__restrict__ all_scores, int64_t all_stride, uint32_t one) {
+                SearchTab tab, TopkState tk, double *__restrict__ all_scores, int64_t all_stride, uint32_t one, RangeHits rh) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     uint2 *s_rows = reinterpret_cast<uint2 *>(smem_raw);                     // [n_queries][QROWS]
     double *s_tau = reinterpret_cast<double *>(s_rows + (size_t)n_queries * QROWS);
@@ -50,7 +65,8 @@ k_search_twin16(const uint32_t *__restrict__ db_words, const int64_t *__restrict
     int *s_qlen = reinterpret_cast<int *>(s_taui + n_queries);
     for (int k = threadIdx.x; k < n_queries * QROWS; k += blockDim.x) s_rows[k] = rowtab[k];
     for (int k = threadIdx.x; k < n_queries; k += blockDim.x) {
-        s_tau[k] = tk.tau_s[k]; s_taui[k] = tk.tau_i[k]; s_qlen[k] = q_len[k];
+        if constexpr (!RANGE) { s_tau[k] = tk.tau_s[k]; s_taui[k] = tk.tau_i[k]; }
+        s_qlen[k] = q_len[k];
     }
     __syncthreads();
 
@@ -121,6 +137,27 @@ k_search_twin16(const uint32_t *__restrict__ db_words, const int64_t *__restrict
             }
             const int dA = m * tab.del + baseA - (int)(H[31] & 0xffffu);
             const int dB = m * tab.del + baseB - (int)(H[31] >> 16);
+            if constexpr (RANGE) {
+                const bool cA = live && dA <= rh.thr, cB = hasB && dB <= rh.thr;
+                const unsigned mA = __ballot_sync(RSD_FULL, cA), mB = __ballot_sync(RSD_FULL, cB);
+                if (mA | mB) {
+                    const int lane_id = threadIdx.x & 31;
+                    unsigned long long base = 0;
+                    if (lane_id == 0) base = atomicAdd(rh.n, (unsigned long long)(__popc(mA) + __popc(mB)));
+                    base = __shfl_sync(RSD_FULL, base, 0);
+                    const unsigned below = (1u << lane_id) - 1u;
+                    const unsigned long long qk = (unsigned long long)q << 32;
+                    if (cA) {
+                        const unsigned long long slot = base + __popc(mA & below);
+                        if (slot < (unsigned long long)rh.cap) { rh.keys[slot] = qk | (unsigned long long)(perm[rA] - global_base); rh.dist[slot] = __dmul_rn((double)dA, tab.inv_scale); }
+                    }
+                    if (cB) {
+                        const unsigned long long slot = base + __popc(mA) + __popc(mB & below);
+                        if (slot < (unsigned long long)rh.cap) { rh.keys[slot] = qk | (unsigned long long)(perm[rB] - global_base); rh.dist[slot] = __dmul_rn((double)dB, tab.inv_scale); }
+                    }
+                }
+                continue;
+            }
             // IR:440  score = 1 / (1 + cost)
             const double sA = __ddiv_rn(1.0, __dadd_rn(1.0, __dmul_rn((double)dA, tab.inv_scale)));
             const double sB = __ddiv_rn(1.0, __dadd_rn(1.0, __dmul_rn((double)dB, tab.inv_scale)));
@@ -302,5 +339,40 @@ __global__ void k_score_filter_pairs(const double *__restrict__ dist, int64_t re
             const int slot = base + __popc(peers & ((1u << lane) - 1u));
             if (slot < tk.cap) { tk.cand_s[(size_t)q * tk.cap + slot] = s; tk.cand_i[(size_t)q * tk.cap + slot] = g; }
         }
+    }
+}
+
+// ... or, in a range search, the pairs within max_dist (fp64 compare: the distance of an integer mode is exactly
+// d / 2^k, so d / 2^k <= max_dist decides as d <= floor(max_dist * 2^k) would).  q_base is the query in the batch.
+__global__ void k_range_filter_pairs(const double *__restrict__ dist, int64_t rec0, int64_t n_rec, const int64_t *__restrict__ perm,
+                                     int64_t global_base, int q_base, int n_q, RangeHits rh) {
+    const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= (int64_t)n_q * n_rec) return;
+    const double d = dist[p];
+    if (!(d <= rh.max_dist)) return;
+    const int q = q_base + (int)(p / n_rec); const int64_t r = p % n_rec;
+    // one atomic per (warp, query), as in k_score_filter_pairs
+    const unsigned peers = __match_any_sync(__activemask(), q);
+    const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+    unsigned long long base = 0;
+    if (lane == leader) base = atomicAdd(rh.n, (unsigned long long)__popc(peers));
+    base = __shfl_sync(peers, base, leader);
+    const unsigned long long slot = base + __popc(peers & ((1u << lane) - 1u));
+    if (slot < (unsigned long long)rh.cap) {
+        rh.keys[slot] = ((unsigned long long)q << 32) | (unsigned long long)(perm[rec0 + r] - global_base);
+        rh.dist[slot] = d;
+    }
+}
+
+// after the sort by key: idx[i] = global index of hit i; off[q] = first hit of query q of the batch (off[n_q] = n)
+__global__ void k_range_split(const unsigned long long *__restrict__ keys, int64_t n, int n_q, int64_t global_base,
+                              int64_t *__restrict__ idx, int64_t *__restrict__ off) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) idx[i] = (int64_t)(keys[i] & 0xffffffffull) + global_base;
+    if (i <= n_q) {
+        const unsigned long long want = (unsigned long long)i << 32;
+        int64_t lo = 0, hi = n;
+        while (lo < hi) { const int64_t mid = (lo + hi) / 2; if (keys[mid] < want) lo = mid + 1; else hi = mid; }
+        off[i] = lo;
     }
 }

@@ -25,6 +25,8 @@
 #include "k_long2.cuh"
 #include "k_ingest.cuh"
 
+#include <cub/device/device_radix_sort.cuh>
+
 // ------------------------------------------------------------------------------------------------
 // errors
 // ------------------------------------------------------------------------------------------------
@@ -1487,7 +1489,7 @@ extern "C" int rsd_db_load(rsd_ctx *c, const uint32_t *words, const int64_t *sta
 
 extern "C" int rsd_db_free(rsd_ctx *c) {
     if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
-    if (c->inited && c->pid == getpid()) { cudaSetDevice(c->device); c->db.release(); c->db_perm.release(); c->db_topi.release(); c->db_tops.release(); c->db_aux.release(); c->db_dist.release(); c->sim_scores.release(); c->sim_aux.release(); c->sim_work.release(); }
+    if (c->inited && c->pid == getpid()) { cudaSetDevice(c->device); c->db.release(); c->db_perm.release(); c->db_topi.release(); c->db_tops.release(); c->db_aux.release(); c->db_dist.release(); c->rng_keys.release(); c->rng_dist.release(); c->rng_tmp.release(); c->sim_scores.release(); c->sim_aux.release(); c->sim_work.release(); }
     c->db_loaded = false; c->db_n = 0;
     return RSD_OK;
 }
@@ -1527,14 +1529,18 @@ int rsd_ctx::fast_prefix(uint32_t q_symmask, int64_t max_qlen, int bits, int for
     return RSD_OK;
 }
 
-// queries already on the device; outputs to device buffers (top_idx/top_score [Q][k]) and optionally all scores
+#define RSD_RANGE_HITS0 ((int64_t)1 << 20)
+
+// queries already on the device; outputs to device buffers (top_idx/top_score [Q][k]) and optionally all scores, or,
+// with `ro`, a range search: every record within ro->max_dist of each query, appended to ro batch by batch
 int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len, int64_t n_queries,
                         int64_t max_qlen, int bits, uint32_t q_symmask, int k, int force_mode,
-                        int64_t *top_idx, double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st) {
+                        int64_t *top_idx, double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st, RangeOut *ro) {
     if (!db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_search: no database loaded (rsd_db_load)");
     if (bits != db_bits) return rsd_fail(RSD_EINVAL, "rsd_db_search: query packing (%d bit) differs from the database (%d bit)", bits, db_bits);
     if (k < 0 || k > RSD_TOPK_MAX) return rsd_fail(RSD_EINVAL, "rsd_db_search: k must be in 0..%d (ask for all_scores instead)", RSD_TOPK_MAX);
     if (n_queries < 0 || n_queries > 1 << 20) return rsd_fail(RSD_EINVAL, "rsd_db_search: n_queries out of range");
+    if (ro && db_n > 0xffffffffLL) return rsd_fail(RSD_EINVAL, "rsd_db_search_range: a shard holds at most 2^32 - 1 records");
     const uint32_t symmask = db_symmask | q_symmask;
     ModeInfo mi;                                  // general kernels: every symbol of the database and the queries
     RSD_OK_OR_RETURN(classify(symmask, max_qlen, db_maxlen, bits, force_mode == RSD_MODE_I16X2 ? 0 : force_mode, mi));
@@ -1562,19 +1568,29 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
     const int64_t CH0 = 4096, CH = (int64_t)1 << 21;
     const int QB = fast ? 64 : 16;                           // queries per batch
     const int64_t cap = std::min<int64_t>(std::max<int64_t>(db_n, 1), CH);
-    const size_t per_q = (size_t)cap * 16 + (size_t)std::max(k, 1) * 16 + 64;
-    RSD_OK_OR_RETURN(db_aux.ensure(per_q * QB + (size_t)QB * 64 * 8 + 4096));
     RSD_OK_OR_RETURN(db_topi.ensure((size_t)QB * QROWS * 8 + 64));
-    unsigned char *aux = (unsigned char *)db_aux.p;
     TopkState tk{};
-    tk.k = k; tk.cap = cap;
-    tk.cand_s = (double *)aux; aux += (size_t)QB * cap * 8;
-    tk.cand_i = (int64_t *)aux; aux += (size_t)QB * cap * 8;
-    tk.best_s = (double *)aux; aux += (size_t)QB * std::max(k, 1) * 8;
-    tk.best_i = (int64_t *)aux; aux += (size_t)QB * std::max(k, 1) * 8;
-    tk.tau_s = (double *)aux; aux += (size_t)QB * 8;
-    tk.tau_i = (int64_t *)aux; aux += (size_t)QB * 8;
-    tk.cand_n = (int *)aux; aux += (size_t)QB * 4;
+    if (!ro) {                                     // a range search keeps no top-k state
+        const size_t per_q = (size_t)cap * 16 + (size_t)std::max(k, 1) * 16 + 64;
+        RSD_OK_OR_RETURN(db_aux.ensure(per_q * QB + (size_t)QB * 64 * 8 + 4096));
+        unsigned char *aux = (unsigned char *)db_aux.p;
+        tk.k = k; tk.cap = cap;
+        tk.cand_s = (double *)aux; aux += (size_t)QB * cap * 8;
+        tk.cand_i = (int64_t *)aux; aux += (size_t)QB * cap * 8;
+        tk.best_s = (double *)aux; aux += (size_t)QB * std::max(k, 1) * 8;
+        tk.best_i = (int64_t *)aux; aux += (size_t)QB * std::max(k, 1) * 8;
+        tk.tau_s = (double *)aux; aux += (size_t)QB * 8;
+        tk.tau_i = (int64_t *)aux; aux += (size_t)QB * 8;
+        tk.cand_n = (int *)aux; aux += (size_t)QB * 4;
+    }
+    RangeHits rh{};
+    if (ro) {
+        // the fast kernel compares the scaled integer distance with floor(max_dist * 2^k) (exact: a power-of-two scale)
+        const double t = std::floor(std::ldexp(ro->max_dist, mi_fast.ic.scale_log2));
+        rh.thr = t >= (double)INT32_MAX ? INT32_MAX : (int)t;
+        rh.max_dist = ro->max_dist;
+        RSD_OK_OR_RETURN(range_reserve(std::max<int64_t>(RSD_RANGE_HITS0, range_cap()), QB));
+    }
     uint2 *rowtab = (uint2 *)db_topi.p;
     const int64_t cap_gen = std::min<int64_t>(std::max<int64_t>(n_gen, 1), cap);
     const int64_t gen_pairs_max = (int64_t)1 << 23;                          // (query, record) pairs per launch train of the general path
@@ -1591,6 +1607,11 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
     for (int64_t q0 = 0; q0 < n_queries; q0 += QB) {
         const int nq = (int)std::min<int64_t>(QB, n_queries - q0);
         if (k > 0) { k_topk_init<<<(nq + 63) / 64, 64, 0, st>>>(tk, nq); launches += 1; }
+        if (ro) {
+            rh.keys = (unsigned long long *)rng_keys.p; rh.dist = (double *)rng_dist.p; rh.n = (unsigned long long *)rng_n.p;
+            rh.cap = range_cap();
+            RSD_CUDA(cudaMemsetAsync(rh.n, 0, sizeof(unsigned long long), st));
+        }
         double *alls = all_scores_dev ? all_scores_dev + (size_t)q0 * db_n : nullptr;
         if (fast) {
             // the integer tables of the fast prefix (the general part below uploads its own; stream order keeps them apart)
@@ -1607,16 +1628,16 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
                 // that is a whole number of waves (resident CTAs x 256 records) leaves no partly filled last wave
                 int per_sm = 0;
                 const size_t smem_q = (size_t)nq * QROWS * 8 + (size_t)nq * 20 + 16;
-                if (search_per_sm_nq != nq || search_per_sm_qrows != QROWS) {
-                    RSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_search_twin16, 128, smem_q));
-                    search_per_sm = per_sm; search_per_sm_nq = nq; search_per_sm_qrows = QROWS;
+                if (search_per_sm_nq != nq || search_per_sm_qrows != QROWS || search_per_sm_range != (ro != nullptr)) {
+                    RSD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ro ? k_search_twin16<true> : k_search_twin16<false>, 128, smem_q));
+                    search_per_sm = per_sm; search_per_sm_nq = nq; search_per_sm_qrows = QROWS; search_per_sm_range = ro != nullptr;
                 }
                 per_sm = search_per_sm;
                 wave = (int64_t)std::max(per_sm, 1) * sm_count * 256;
                 if (rest > cap && cap >= wave) main_sz = cap / wave * wave;       // a shard that fits one chunk goes in one launch (finer waves below)
             }
             for (int64_t r0 = 0; r0 < n_fast;) {
-                const bool seed = r0 == 0 && n_fast > CH0;
+                const bool seed = !ro && r0 == 0 && n_fast > CH0;
                 const int64_t nr = std::min<int64_t>(seed ? CH0 : main_sz, n_fast - r0);
                 const int64_t threads = (nr + 1) / 2;
                 const size_t smem = (size_t)nq * QROWS * 8 + (size_t)nq * 20 + 16;
@@ -1628,8 +1649,10 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
                 if (const char *e = getenv("RSD_SEARCH_WAVES")) want_waves = std::max(atoi(e), 1);
                 if (!seed && wave > 0 && nr < want_waves * wave) gy = (unsigned)std::min<int64_t>(std::min(nq, 16), (want_waves * wave + nr - 1) / std::max<int64_t>(nr, 1));
                 const dim3 grid((unsigned)((threads + 127) / 128), gy);
-                k_search_twin16<<<grid, 128, smem, st>>>(dbw, dbs, dbl, r0, nr, db_bits, (const int64_t *)db_perm.p, db_base, rowtab, QROWS,
-                                                                                      q_len + q0, nq, tab, tk, alls, db_n, 1u);
+                if (ro) k_search_twin16<true><<<grid, 128, smem, st>>>(dbw, dbs, dbl, r0, nr, db_bits, (const int64_t *)db_perm.p, db_base, rowtab, QROWS,
+                                                                       q_len + q0, nq, tab, tk, nullptr, db_n, 1u, rh);
+                else k_search_twin16<false><<<grid, 128, smem, st>>>(dbw, dbs, dbl, r0, nr, db_bits, (const int64_t *)db_perm.p, db_base, rowtab, QROWS,
+                                                                     q_len + q0, nq, tab, tk, alls, db_n, 1u, rh);
                 launches += 1;
                 if (k > 0) { k_topk_fold<<<nq, 256, 0, st>>>(tk); launches += 1; }
                 RSD_CUDA(cudaGetLastError());
@@ -1657,7 +1680,8 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
                                       force_mode == RSD_MODE_I16X2 ? 0 : force_mode, (double *)db_dist.p, &mode_unused, st);
                 timing = t_save;
                 if (rc) return rc;
-                k_score_filter_pairs<<<(unsigned)((np + 255) / 256), 256, 0, st>>>((const double *)db_dist.p, r0, nr, (const int64_t *)db_perm.p, db_base, qa, nqb, tk, alls, db_n);
+                if (ro) k_range_filter_pairs<<<(unsigned)((np + 255) / 256), 256, 0, st>>>((const double *)db_dist.p, r0, nr, (const int64_t *)db_perm.p, db_base, qa, nqb, rh);
+                else k_score_filter_pairs<<<(unsigned)((np + 255) / 256), 256, 0, st>>>((const double *)db_dist.p, r0, nr, (const int64_t *)db_perm.p, db_base, qa, nqb, tk, alls, db_n);
                 launches += 1;
             }
             if (k > 0) { k_topk_fold<<<nq, 256, 0, st>>>(tk); launches += 1; }
@@ -1668,8 +1692,61 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
             RSD_CUDA(cudaMemcpyAsync(top_idx + q0 * k, tk.best_i, sizeof(int64_t) * (size_t)nq * k, cudaMemcpyDeviceToDevice, st));
             RSD_CUDA(cudaMemcpyAsync(top_score + q0 * k, tk.best_s, sizeof(double) * (size_t)nq * k, cudaMemcpyDeviceToDevice, st));
         }
+        if (ro) {
+            bool rerun = false;
+            RSD_OK_OR_RETURN(range_collect(nq, QB, *ro, rerun, st));
+            if (rerun) q0 -= QB;                 // the buffer now holds the batch's exact count: the same batch again
+        }
     }
     if (timing) { RSD_CUDA(cudaEventRecord(ev1, st)); timed = true; }
+    return RSD_OK;
+}
+
+// Range search hit buffer: room for `hits` hits (keys and distances, each twice for the sort's double buffer), the
+// counter and qb + 1 offsets.  Starts at RSD_RANGE_HITS0 hits and grows to the exact count of a batch that overflowed.
+int rsd_ctx::range_reserve(int64_t hits, int qb) {
+    RSD_OK_OR_RETURN(rng_keys.ensure(sizeof(unsigned long long) * 2 * (size_t)hits));
+    RSD_OK_OR_RETURN(rng_dist.ensure(sizeof(double) * 2 * (size_t)hits));
+    RSD_OK_OR_RETURN(rng_n.ensure(sizeof(int64_t) * (size_t)(qb + 2)));
+    return RSD_OK;
+}
+
+// After a query batch of a range search: the hit count comes back; a count above the buffer grows it and asks for the
+// batch again (rerun).  Otherwise the hits are sorted by key (query in batch, then collection index: the store order is
+// (tier, length)), split per query, and appended to `ro`.
+int rsd_ctx::range_collect(int nq, int qb, RangeOut &ro, bool &rerun, cudaStream_t st) {
+    unsigned long long n = 0;
+    RSD_CUDA(cudaMemcpyAsync(&n, rng_n.p, sizeof n, cudaMemcpyDeviceToHost, st));
+    RSD_CUDA(cudaStreamSynchronize(st));
+    const int64_t cap_h = range_cap();
+    rerun = (int64_t)n > cap_h;
+    if (rerun) return range_reserve((int64_t)n, qb);
+    cub::DoubleBuffer<unsigned long long> kb((unsigned long long *)rng_keys.p, (unsigned long long *)rng_keys.p + cap_h);
+    cub::DoubleBuffer<double> vb((double *)rng_dist.p, (double *)rng_dist.p + cap_h);
+    if (n > 1) {
+        int end_bit = 32;
+        while ((1 << (end_bit - 32)) < nq) ++end_bit;
+        size_t tmp = 0;
+        RSD_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp, kb, vb, (int64_t)n, 0, end_bit, st));
+        RSD_OK_OR_RETURN(rng_tmp.ensure(tmp));
+        RSD_CUDA(cub::DeviceRadixSort::SortPairs(rng_tmp.p, tmp, kb, vb, (int64_t)n, 0, end_bit, st));
+        launches += 1;
+    }
+    int64_t *off_d = (int64_t *)rng_n.p + 1, *idx_d = (int64_t *)kb.Alternate();
+    const int64_t nt = std::max<int64_t>((int64_t)n, nq + 1);
+    k_range_split<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(kb.Current(), (int64_t)n, nq, db_base, idx_d, off_d);
+    launches += 1;
+    RSD_CUDA(cudaGetLastError());
+    std::vector<int64_t> off((size_t)nq + 1);
+    const size_t h0 = ro.idx.size();
+    ro.idx.resize(h0 + n); ro.dist.resize(h0 + n);
+    RSD_CUDA(cudaMemcpyAsync(off.data(), off_d, sizeof(int64_t) * off.size(), cudaMemcpyDeviceToHost, st));
+    if (n) {
+        RSD_CUDA(cudaMemcpyAsync(ro.idx.data() + h0, idx_d, sizeof(int64_t) * n, cudaMemcpyDeviceToHost, st));
+        RSD_CUDA(cudaMemcpyAsync(ro.dist.data() + h0, vb.Current(), sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+    }
+    RSD_CUDA(cudaStreamSynchronize(st));
+    for (int q = 0; q < nq; ++q) ro.cnt.push_back(off[(size_t)q + 1] - off[(size_t)q]);
     return RSD_OK;
 }
 
@@ -1684,33 +1761,28 @@ extern "C" int rsd_db_search_topk_dev(rsd_ctx *c, const uint32_t *q_words_dev, c
                          top_idx_dev, top_score_dev, nullptr, mode_out, (cudaStream_t)stream);
 }
 
-extern "C" int rsd_db_search_topk(rsd_ctx *c, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
-                                  int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, int k, int force_mode,
-                                  int64_t *top_idx, double *top_score, double *all_scores, int *mode_out) {
-    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
-    if (n_queries < 0 || (n_queries > 0 && (!q_words || !q_start || !q_len))) return rsd_fail(RSD_EINVAL, "rsd_db_search_topk: bad arguments");
-    if (k > 0 && (!top_idx || !top_score)) return rsd_fail(RSD_EINVAL, "rsd_db_search_topk: NULL top-k output");
-    RSD_OK_OR_RETURN(c->ensure_device());
-    if (n_queries == 0) return RSD_OK;
-    cudaStream_t st = c->stream;
-    RSD_OK_OR_RETURN(c->upload_seqs(c->bufQ, q_words, q_start, q_len, n_queries, q_nwords, st));
-    const int kk = std::max(k, 0);
-    RSD_OK_OR_RETURN(c->s_oi.ensure(sizeof(int64_t) * (size_t)n_queries * std::max(kk, 1)));
-    RSD_OK_OR_RETURN(c->s_oj.ensure(sizeof(double) * (size_t)n_queries * std::max(kk, 1)));
-    if (all_scores) RSD_OK_OR_RETURN(c->out_f64.ensure(sizeof(double) * (size_t)n_queries * std::max<int64_t>(c->db_n, 1)));
-    int64_t max_qlen = 0;
-    for (int64_t i = 0; i < n_queries; ++i) max_qlen = std::max<int64_t>(max_qlen, q_len[i]);
+// order (empty: caller order) = the caller's query of every device row; rows [0, n_first) form the first group
+struct QueryGroups {
+    std::vector<int64_t> order;
+    int64_t n_first = 0;
+    uint32_t mask_first = 0, mask_rest = 0;
+};
+
+// the queries are already in c->bufQ; their start / len there are rewritten in group order
+static int group_queries(rsd_ctx *c, const char *who, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
+                         int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, int force_mode, int64_t max_qlen,
+                         QueryGroups &qg) {
     // A query that carries a symbol outside the fast kernel's reach (an ambiguity code whose costs are not dyadic) would
     // send every query of its batch through the general kernels for the whole database.  Queries are therefore grouped:
     // those that leave a fast prefix first, the others after them, one search per group.
-    std::vector<int64_t> order;
-    int64_t n_first = n_queries;
-    uint32_t mask_first = q_symmask, mask_rest = 0;
+    std::vector<int64_t> &order = qg.order;
+    order.clear();
+    qg.n_first = n_queries; qg.mask_first = q_symmask; qg.mask_rest = 0;
     if (n_queries > 1 && force_mode == 0) {
         const int per = 32 / bits;
         std::vector<uint32_t> qm((size_t)n_queries, 0u);
         for (int64_t q = 0; q < n_queries; ++q) {
-            if (q_start[q] < 0 || q_start[q] + ((int64_t)q_len[q] + per - 1) / per > q_nwords) return rsd_fail(RSD_EINVAL, "rsd_db_search_topk: query %lld lies outside the word buffer", (long long)q);
+            if (q_start[q] < 0 || q_start[q] + ((int64_t)q_len[q] + per - 1) / per > q_nwords) return rsd_fail(RSD_EINVAL, "%s: query %lld lies outside the word buffer", who, (long long)q);
             for (int32_t j = 0; j < q_len[q]; ++j) qm[(size_t)q] |= 1u << ((q_words[q_start[q] + j / per] >> ((j % per) * bits)) & ((1u << bits) - 1u));
         }
         std::vector<uint32_t> ok_masks, bad_masks;         // masks already classified (few distinct ones)
@@ -1740,30 +1812,62 @@ extern "C" int rsd_db_search_topk(rsd_ctx *c, const uint32_t *q_words, const int
             if (nf > 0) {
                 order.reserve((size_t)n_queries);
                 for (int64_t q = 0; q < n_queries; ++q) if (friendly[(size_t)q]) order.push_back(q);
-                for (int64_t q = 0; q < n_queries; ++q) if (!friendly[(size_t)q]) { order.push_back(q); mask_rest |= qm[(size_t)q]; }
-                n_first = n_ok; mask_first = mu;
+                for (int64_t q = 0; q < n_queries; ++q) if (!friendly[(size_t)q]) { order.push_back(q); qg.mask_rest |= qm[(size_t)q]; }
+                qg.n_first = n_ok; qg.mask_first = mu;
             }
         }
     }
     if (!order.empty()) {                             // queries in group order on the device (the words stay where they are)
         std::vector<int64_t> ps((size_t)n_queries); std::vector<int32_t> pl((size_t)n_queries);
         for (int64_t r = 0; r < n_queries; ++r) { ps[(size_t)r] = q_start[order[(size_t)r]]; pl[(size_t)r] = q_len[order[(size_t)r]]; }
-        RSD_CUDA(cudaMemcpyAsync(c->bufQ.start.p, ps.data(), sizeof(int64_t) * (size_t)n_queries, cudaMemcpyHostToDevice, st));
-        RSD_CUDA(cudaMemcpyAsync(c->bufQ.len.p, pl.data(), sizeof(int32_t) * (size_t)n_queries, cudaMemcpyHostToDevice, st));
-        RSD_CUDA(cudaStreamSynchronize(st));          // ps / pl are pageable temporaries
+        RSD_CUDA(cudaMemcpyAsync(c->bufQ.start.p, ps.data(), sizeof(int64_t) * (size_t)n_queries, cudaMemcpyHostToDevice, c->stream));
+        RSD_CUDA(cudaMemcpyAsync(c->bufQ.len.p, pl.data(), sizeof(int32_t) * (size_t)n_queries, cudaMemcpyHostToDevice, c->stream));
+        RSD_CUDA(cudaStreamSynchronize(c->stream));          // ps / pl are pageable temporaries
     }
-    int mode_all = 0;
+    return RSD_OK;
+}
+
+// one search_dev per group (rows of c->bufQ); top-k rows go to c->s_oi / c->s_oj, all_scores rows to c->out_f64, and range
+// hits (ro) are appended row by row
+static int search_groups(rsd_ctx *c, const QueryGroups &qg, int64_t n_queries, int64_t max_qlen, int bits, int kk, int force_mode,
+                         bool all_scores, RangeOut *ro, int &mode_all) {
+    mode_all = 0;
     for (int g = 0; g < 2; ++g) {
-        const int64_t g0 = g == 0 ? 0 : n_first, g1 = g == 0 ? n_first : n_queries;
+        const int64_t g0 = g == 0 ? 0 : qg.n_first, g1 = g == 0 ? qg.n_first : n_queries;
         if (g1 <= g0) continue;
         int mo = 0;
         struct Hold { rsd_ctx *c; ~Hold() { c->hold_ev0 = false; } } hold{c};
-        c->hold_ev0 = g == 1 && n_first > 0;
+        c->hold_ev0 = g == 1 && qg.n_first > 0;
         RSD_OK_OR_RETURN(c->search_dev((const uint32_t *)c->bufQ.words.p, (const int64_t *)c->bufQ.start.p + g0, (const int32_t *)c->bufQ.len.p + g0,
-                                       g1 - g0, max_qlen, bits, g == 0 ? mask_first : mask_rest, kk, force_mode, (int64_t *)c->s_oi.p + g0 * kk, (double *)c->s_oj.p + g0 * kk,
-                                       all_scores ? (double *)c->out_f64.p + (size_t)g0 * c->db_n : nullptr, &mo, st));
+                                       g1 - g0, max_qlen, bits, g == 0 ? qg.mask_first : qg.mask_rest, kk, force_mode,
+                                       ro ? nullptr : (int64_t *)c->s_oi.p + g0 * kk, ro ? nullptr : (double *)c->s_oj.p + g0 * kk,
+                                       all_scores ? (double *)c->out_f64.p + (size_t)g0 * c->db_n : nullptr, &mo, c->stream, ro));
         mode_all = std::max(mode_all, mo);
     }
+    return RSD_OK;
+}
+
+extern "C" int rsd_db_search_topk(rsd_ctx *c, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
+                                  int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, int k, int force_mode,
+                                  int64_t *top_idx, double *top_score, double *all_scores, int *mode_out) {
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    if (n_queries < 0 || (n_queries > 0 && (!q_words || !q_start || !q_len))) return rsd_fail(RSD_EINVAL, "rsd_db_search_topk: bad arguments");
+    if (k > 0 && (!top_idx || !top_score)) return rsd_fail(RSD_EINVAL, "rsd_db_search_topk: NULL top-k output");
+    RSD_OK_OR_RETURN(c->ensure_device());
+    if (n_queries == 0) return RSD_OK;
+    cudaStream_t st = c->stream;
+    RSD_OK_OR_RETURN(c->upload_seqs(c->bufQ, q_words, q_start, q_len, n_queries, q_nwords, st));
+    const int kk = std::max(k, 0);
+    RSD_OK_OR_RETURN(c->s_oi.ensure(sizeof(int64_t) * (size_t)n_queries * std::max(kk, 1)));
+    RSD_OK_OR_RETURN(c->s_oj.ensure(sizeof(double) * (size_t)n_queries * std::max(kk, 1)));
+    if (all_scores) RSD_OK_OR_RETURN(c->out_f64.ensure(sizeof(double) * (size_t)n_queries * std::max<int64_t>(c->db_n, 1)));
+    int64_t max_qlen = 0;
+    for (int64_t i = 0; i < n_queries; ++i) max_qlen = std::max<int64_t>(max_qlen, q_len[i]);
+    QueryGroups qg;
+    RSD_OK_OR_RETURN(group_queries(c, "rsd_db_search_topk", q_words, q_start, q_len, n_queries, q_nwords, bits, q_symmask, force_mode, max_qlen, qg));
+    const std::vector<int64_t> &order = qg.order;
+    int mode_all = 0;
+    RSD_OK_OR_RETURN(search_groups(c, qg, n_queries, max_qlen, bits, kk, force_mode, all_scores != nullptr, nullptr, mode_all));
     if (mode_out) *mode_out = mode_all;
     if (order.empty()) {
         if (kk > 0) {
@@ -1783,6 +1887,84 @@ extern "C" int rsd_db_search_topk(rsd_ctx *c, const uint32_t *q_words, const int
     }
     RSD_CUDA(cudaStreamSynchronize(st));
     return RSD_OK;
+}
+
+// Range search of one shard, host queries in, hits out per query in caller order (rsd_db_search_range and every shard of
+// rsd_multi_db_search_range).
+static int range_shard(rsd_ctx *c, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len, int64_t n_queries,
+                       int64_t q_nwords, int bits, uint32_t q_symmask, double max_dist, int force_mode, RangeOut &out, int *mode_out) {
+    RSD_OK_OR_RETURN(c->upload_seqs(c->bufQ, q_words, q_start, q_len, n_queries, q_nwords, c->stream));
+    int64_t max_qlen = 0;
+    for (int64_t i = 0; i < n_queries; ++i) max_qlen = std::max<int64_t>(max_qlen, q_len[i]);
+    QueryGroups qg;
+    RSD_OK_OR_RETURN(group_queries(c, "rsd_db_search_range", q_words, q_start, q_len, n_queries, q_nwords, bits, q_symmask, force_mode, max_qlen, qg));
+    RangeOut ro;
+    ro.max_dist = max_dist;
+    int mode_all = 0;
+    RSD_OK_OR_RETURN(search_groups(c, qg, n_queries, max_qlen, bits, 0, force_mode, false, &ro, mode_all));
+    if (mode_out) *mode_out = mode_all;
+    if (qg.order.empty()) { out = std::move(ro); return RSD_OK; }
+    std::vector<int64_t> row0((size_t)n_queries + 1, 0), row_of((size_t)n_queries);      // device row -> first hit; query -> row
+    for (int64_t r = 0; r < n_queries; ++r) { row0[(size_t)r + 1] = row0[(size_t)r] + ro.cnt[(size_t)r]; row_of[(size_t)qg.order[(size_t)r]] = r; }
+    out.cnt.assign((size_t)n_queries, 0); out.idx.resize(ro.idx.size()); out.dist.resize(ro.dist.size());
+    int64_t h = 0;
+    for (int64_t q = 0; q < n_queries; ++q) {
+        const int64_t r = row_of[(size_t)q], n = ro.cnt[(size_t)r];
+        std::copy_n(ro.idx.begin() + row0[(size_t)r], n, out.idx.begin() + h);
+        std::copy_n(ro.dist.begin() + row0[(size_t)r], n, out.dist.begin() + h);
+        out.cnt[(size_t)q] = n; h += n;
+    }
+    return RSD_OK;
+}
+
+// CSR output of a range search: each query's hits of shard 0, then shard 1, ... (the shards are index-contiguous, so
+// this is collection order).  hit_off is always written; more hits than cap is RSD_ERANGE, never a silent cut.
+static int range_emit(const char *who, const std::vector<RangeOut> &shards, int64_t n_queries, int64_t cap,
+                      int64_t *hit_off, int64_t *hit_idx, double *hit_dist) {
+    hit_off[0] = 0;
+    for (int64_t q = 0; q < n_queries; ++q) {
+        int64_t n = 0;
+        for (const RangeOut &o : shards) n += o.cnt[(size_t)q];
+        hit_off[q + 1] = hit_off[q] + n;
+    }
+    if (hit_off[n_queries] > cap)
+        return rsd_fail(RSD_ERANGE, "%s: %lld hits exceed cap = %lld (hit_off holds every query's count)", who,
+                        (long long)hit_off[n_queries], (long long)cap);
+    std::vector<int64_t> pos(shards.size(), 0);
+    int64_t h = 0;
+    for (int64_t q = 0; q < n_queries; ++q)
+        for (size_t g = 0; g < shards.size(); ++g) {
+            const int64_t n = shards[g].cnt[(size_t)q];
+            if (n) {
+                memcpy(hit_idx + h, shards[g].idx.data() + pos[g], sizeof(int64_t) * (size_t)n);
+                memcpy(hit_dist + h, shards[g].dist.data() + pos[g], sizeof(double) * (size_t)n);
+            }
+            pos[g] += n; h += n;
+        }
+    return RSD_OK;
+}
+
+// argument checks of both range entry points (before any device work)
+static int range_args(const char *who, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len, int64_t n_queries,
+                      double max_dist, int64_t cap, const int64_t *hit_off, const int64_t *hit_idx, const double *hit_dist) {
+    if (n_queries < 0 || (n_queries > 0 && (!q_words || !q_start || !q_len))) return rsd_fail(RSD_EINVAL, "%s: bad arguments", who);
+    if (!(max_dist >= 0.0)) return rsd_fail(RSD_EINVAL, "%s: max_dist must be >= 0 and not NaN (got %g)", who, max_dist);
+    if (cap < 0 || !hit_off || (cap > 0 && (!hit_idx || !hit_dist))) return rsd_fail(RSD_EINVAL, "%s: bad output arrays", who);
+    return RSD_OK;
+}
+
+extern "C" int rsd_db_search_range(rsd_ctx *c, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
+                                   int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, double max_dist,
+                                   int force_mode, int64_t cap, int64_t *hit_off, int64_t *hit_idx, double *hit_dist,
+                                   int *mode_out) {
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    RSD_OK_OR_RETURN(range_args("rsd_db_search_range", q_words, q_start, q_len, n_queries, max_dist, cap, hit_off, hit_idx, hit_dist));
+    RSD_OK_OR_RETURN(c->ensure_device());
+    hit_off[0] = 0;
+    if (n_queries == 0) return RSD_OK;
+    std::vector<RangeOut> out(1);
+    RSD_OK_OR_RETURN(range_shard(c, q_words, q_start, q_len, n_queries, q_nwords, bits, q_symmask, max_dist, force_mode, out[0], mode_out));
+    return range_emit("rsd_db_search_range", out, n_queries, cap, hit_off, hit_idx, hit_dist);
 }
 
 // ------------------------------------------------------------------------------------------------

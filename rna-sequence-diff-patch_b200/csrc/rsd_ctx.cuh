@@ -4,7 +4,9 @@
 #include <stdarg.h>
 #include <stdint.h>
 #include <unistd.h>
+#include <algorithm>
 #include <new>
+#include <vector>
 
 #include "k_plan.cuh"
 
@@ -70,6 +72,14 @@ struct PlanSlot {
     void release() { scratch.release(); pair_bin.release(); bins.release(); groups.release(); dirty = true; }
 };
 
+// Hits of a range search on the host, query by query in the order the search saw the queries: cnt[q] hits each,
+// concatenated in idx / dist, every query's hits by global index ascending.
+struct RangeOut {
+    double max_dist = 0;
+    std::vector<int64_t> cnt, idx;
+    std::vector<double> dist;
+};
+
 struct rsd_ctx {
     int device = 0;
     bool inited = false;
@@ -119,6 +129,10 @@ struct rsd_ctx {
     bool db_loaded = false;
     DevBuf db_dist, db_topi, db_tops, db_aux, db_perm;
     int search_per_sm = 0, search_per_sm_nq = -1, search_per_sm_qrows = -1;      // occupancy of the search kernel, asked once per shape
+    bool search_per_sm_range = false;                                             // ... and epilogue
+    // range search: hit append buffer of one query batch (keys and distances, each two halves for the sort), the
+    // 64-bit hit counter + per-query offsets, the sort's scratch
+    DevBuf rng_keys, rng_dist, rng_n, rng_tmp;
     DevBuf sim_q, sim_scores, sim_aux, sim_codes, sim_work;
 
     int ensure_device();
@@ -138,7 +152,10 @@ struct rsd_ctx {
     int fast_prefix(uint32_t q_symmask, int64_t max_qlen, int bits, int force_mode, ModeInfo &mi_fast, uint32_t lut[4], int64_t &n_fast) const;
     int search_dev(const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len, int64_t n_queries,
                    int64_t max_qlen, int bits, uint32_t q_symmask, int k, int force_mode, int64_t *top_idx,
-                   double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st);
+                   double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st, RangeOut *ro = nullptr);
+    int64_t range_cap() const { return (int64_t)(std::min(rng_keys.cap, rng_dist.cap) / 16); }     // hits the buffer holds
+    int range_reserve(int64_t hits, int qb);
+    int range_collect(int nq, int qb, RangeOut &ro, bool &rerun, cudaStream_t st);
     int script_pipeline(const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int bits, uint32_t symmask,
                         int force_mode, int64_t max_ops, bool with_x, uint8_t *op, int32_t *oi, int32_t *oj,
                         int32_t *n_ops, double *dist, uint8_t *ok, int *mode_out);
@@ -147,7 +164,7 @@ struct rsd_ctx {
         for (PlanSlot &s : slots) s.release();
         DevBuf *all[] = {&out_f64, &mat_vals, &mat_mask, &mat_ab,
                          &long_pool, &long_jobs, &dirs, &s_op, &s_oi, &s_oj, &s_nops, &s_ok, &s_tmp, &p_out, &p_len, &p_err, &misc,
-                         &db_dist, &db_topi, &db_tops, &db_aux, &db_perm, &sim_q, &sim_scores, &sim_aux, &sim_codes, &sim_work};
+                         &db_dist, &db_topi, &db_tops, &db_aux, &db_perm, &rng_keys, &rng_dist, &rng_n, &rng_tmp, &sim_q, &sim_scores, &sim_aux, &sim_codes, &sim_work};
         for (DevBuf *b : all) b->release();
         d_stage.release(); for (int s = 0; s < 2; ++s) { raw_codes[s].release(); sym_start[s].release(); }
         if (h_stage) { cudaFreeHost(h_stage); h_stage = nullptr; h_stage_cap = 0; }

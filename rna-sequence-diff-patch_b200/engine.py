@@ -32,6 +32,33 @@ def costs_to_arrays(costs: dict):
     return float(costs["insert"]), float(costs["delete"]), sub
 
 
+def _db_query(Q: PackedSeqs, db_bits: int) -> PackedSeqs:
+    """The repacking rule of the database searches: 2-bit queries go to 4 bits for a 4-bit database."""
+    Q = Q.repack(db_bits) if Q.bits != db_bits and db_bits == 4 else Q
+    if Q.bits != db_bits:
+        raise ValueError("query symbols do not fit the database packing; reload the database with bits=4")
+    return Q
+
+
+def _search_range(fn, h, Q: PackedSeqs, max_dist: float, force_mode: int, guess: int):
+    """Calls a range entry point (rsd_db_search_range / rsd_multi_db_search_range) with room for `guess` hits; when the
+    hits do not fit (RSD_ERANGE, hit_off complete), once more with the exact total."""
+    nq = Q.n
+    off = np.zeros(nq + 1, np.int64)
+    mode = C.c_int()
+    for attempt in range(2):
+        cap = max(int(guess), 1)
+        idx = np.empty(cap, np.int64); dist = np.empty(cap, np.float64)
+        rc = fn(h, ptr(Q.words, _u32), ptr(Q.start, _i64), ptr(Q.len, _i32), nq, Q.words.shape[0], Q.bits, Q.symmask,
+                float(max_dist), force_mode, cap, ptr(off, _i64), ptr(idx, _i64), ptr(dist, _f64), C.byref(mode))
+        if rc == _lib.RSD_ERANGE and attempt == 0:
+            guess = int(off[nq])
+            continue
+        check(rc)
+        total = int(off[nq])
+        return (off, idx[:total], dist[:total]), mode.value
+
+
 class Engine:
     def __init__(self, device: int = 0):
         self._lib = _lib.load_library()
@@ -186,9 +213,7 @@ class Engine:
 
     def db_search_topk(self, Q: PackedSeqs, k: int, want_scores: bool = False, force_mode: int = 0):
         """-> (top_idx int64[q,k], top_score f64[q,k][, all_scores f64[q, n_db]])."""
-        Q = Q.repack(self._db_bits) if Q.bits != self._db_bits and self._db_bits == 4 else Q
-        if Q.bits != self._db_bits:
-            raise ValueError("query symbols do not fit the database packing; reload the database with bits=4")
+        Q = _db_query(Q, self._db_bits)
         nq = Q.n
         idx = np.zeros((nq, k), np.int64); sc = np.zeros((nq, k), np.float64)
         alls = np.zeros((nq, self._db_n), np.float64) if want_scores else None
@@ -199,6 +224,16 @@ class Engine:
                                            ptr(alls, _f64) if want_scores else None, C.byref(mode)))
         self.last_mode = mode.value
         return (idx, sc, alls) if want_scores else (idx, sc)
+
+    def db_search_range(self, Q: PackedSeqs, max_dist: float, force_mode: int = 0):
+        """Every database record within max_dist (inclusive) of each query, with its exact distance D (the fp64 value of
+        distance_batch(query, record)) -> CSR (offsets int64[q+1], idx int64[total], dist f64[total]): the hits of query q
+        are idx[offsets[q]:offsets[q+1]], by global index ascending.  max_dist = inf returns every record."""
+        Q = _db_query(Q, self._db_bits)
+        res, self.last_mode = _search_range(self._lib.rsd_db_search_range, self._ctx, Q, max_dist, force_mode,
+                                            getattr(self, "_range_total", Q.n * 256))
+        self._range_total = int(res[0][-1])
+        return res
 
     def db_search_topk_dev(self, q_words, q_start, q_len, n_queries, max_qlen, bits, q_symmask, k, top_idx, top_score,
                            stream, force_mode: int = 0):
@@ -338,9 +373,7 @@ class MultiEngine:
         self._db_gen += 1
 
     def db_search_topk(self, Q: PackedSeqs, k: int, want_scores: bool = False, force_mode: int = 0):
-        Q = Q.repack(self._db_bits) if Q.bits != self._db_bits and self._db_bits == 4 else Q
-        if Q.bits != self._db_bits:
-            raise ValueError("query symbols do not fit the database packing; reload the database with bits=4")
+        Q = _db_query(Q, self._db_bits)
         nq = Q.n
         idx = np.zeros((nq, max(k, 1)), np.int64); sc = np.zeros((nq, max(k, 1)), np.float64)
         alls = np.zeros((nq, self._db_n), np.float64) if want_scores else None
@@ -351,6 +384,14 @@ class MultiEngine:
         self.last_mode = mode.value
         idx, sc = idx[:, :k], sc[:, :k]
         return (idx, sc, alls) if want_scores else (idx, sc)
+
+    def db_search_range(self, Q: PackedSeqs, max_dist: float, force_mode: int = 0):
+        """Engine.db_search_range over the whole sharded database."""
+        Q = _db_query(Q, self._db_bits)
+        res, self.last_mode = _search_range(self._lib.rsd_multi_db_search_range, self._h, Q, max_dist, force_mode,
+                                            getattr(self, "_range_total", Q.n * 256))
+        self._range_total = int(res[0][-1])
+        return res
 
     def launch_count(self) -> int:
         return int(self._lib.rsd_multi_launch_count(self._h))

@@ -2,7 +2,8 @@
 
 Mirrors: wf_score IR:435-440, the wf_score branch of search_collection IR:443-447,466-477 (one
 batched GPU scan of the collection instead of one wagnerFisher call per document), and the
-stable descending top-k of performance.py:12-15 / gui.py:573,593; and the other scorers of
+stable descending top-k of performance.py:12-15 / gui.py:573,593; every document within a distance bound
+(range_collection, which the reference lacks); and the other scorers of
 search_collection — set / multiset / TF-vector measures, IR:49-389 — as one GPU pass over the collection
 (similarity_collection)."""
 from __future__ import annotations
@@ -81,6 +82,21 @@ def score_collection(query: str, sequences, costs: dict, engine=None):
     _Resident.load(eng, sequences, upper=True)
     _, _, scores = eng.db_search_topk(pack([query.upper()], bits=4), k=1, want_scores=True)
     return [(s, float(v)) for s, v in zip(sequences, scores[0])]
+
+
+def range_collection(query: str, sequences, max_dist: float, costs: dict, engine=None):
+    """[(index, sequence, D)] for every sequence of the collection with D = distance(query, sequence) <= max_dist
+    (inclusive), in collection order — the wf_score scan of search_collection (IR:466-477) filtered on the distance
+    instead of ranked, with D exact rather than recovered from 1 / (1 + D)."""
+    sequences = list(sequences)
+    if not sequences:
+        return []
+    eng = engine or get_search_engine()
+    eng.set_costs(costs)
+    _validate_collection(query, sequences, costs)
+    _Resident.load(eng, sequences, upper=True)
+    _, idx, dist = eng.db_search_range(pack([query.upper()], bits=4), max_dist)
+    return [(int(i), sequences[i], float(d)) for i, d in zip(idx, dist)]
 
 
 SIM_METHODS = ("set_intersection_similarity", "set_jaccard_similarity", "set_dice_similarity",

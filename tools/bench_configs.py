@@ -208,7 +208,9 @@ def x2(eng, L=1_000_000):
             "direction_matrix_bytes": cells / 4, "checked": "valid path, cost == distance == distance-only pass, patch(A) == B"}
 
 
-def c5(eng, n_rec, nq=64, k=10, reps=3, iupac=False):
+def c5_data(n_rec, nq=64, iupac=False):
+    """The single-process C5 database (24..31 nt, ACGU with one N per 1000 symbols) and nq queries (records with 10 %
+    of their symbols redrawn) -> (codes, off, lens, query codes list, Q packed, db packed)."""
     rng = np.random.default_rng(20260005)
     lens = rng.integers(24, 32, size=n_rec)
     off = np.zeros(n_rec + 1, np.int64); np.cumsum(lens, out=off[1:])
@@ -225,6 +227,11 @@ def c5(eng, n_rec, nq=64, k=10, reps=3, iupac=False):
         qs.append(s); qo.append(qo[-1] + s.shape[0])
     Q = R.pack((np.concatenate(qs), np.array(qo, np.int64)), bits=4)
     db = R.pack((codes, off), bits=4)
+    return codes, off, lens, qs, Q, db
+
+
+def c5(eng, n_rec, nq=64, k=10, reps=3, iupac=False):
+    codes, off, lens, qs, Q, db = c5_data(n_rec, nq, iupac)
     eng.set_costs(DEFAULT); eng.set_timing(True)
     eng.db_load(db)
     cells = float(sum(len(q) for q in qs)) * 0 + float(np.add.outer(np.array([len(q) for q in qs]), np.zeros(1)).sum() * 0)

@@ -86,7 +86,7 @@ def main():
         alpha = [SYM[:4], SYM[:4], SYM[:4] + "N", SYM, SYM[:2], "ACGUYR"][int(rng.integers(0, 6))]
         ckind = ["default", "user", "dyadic", "int", "decimal"][int(rng.integers(0, 5))]
         lkind = ["tiny", "short", "c2", "kb", "skew", "wide"][int(rng.integers(0, 6))]
-        what = ["dist", "dist", "script", "search", "long", "sim"][int(rng.integers(0, 6))]
+        what = ["dist", "dist", "script", "search", "long", "sim", "range"][int(rng.integers(0, 7))]
         costs = random_costs(rng, ckind)
         eng.set_costs(costs)
         force = int(rng.choice([0, 0, 0, 2, 3]))
@@ -190,6 +190,29 @@ def main():
                     ok = ok and r2["dist"] == d2 and np.array_equal(r2["op"], o2) and np.array_equal(r2["oi"], i2) and np.array_equal(r2["oj"], j2)
                 cells += float(m) * b1.shape[0]
                 desc = f"long {m}x{b1.shape[0]} mode={eng.last_mode} knobs={knobs} batch={len(extra) + 1}"
+            elif what == "range":
+                n = int(rng.choice([1, 50, 3000, 40000]))
+                lens = rng.integers(0 if rng.random() < 0.3 else 20, int(rng.choice([32, 33, 60])), size=n)
+                cd, od = make(rng, lens, alpha)
+                nq = int(rng.choice([1, 3, 70]))
+                ql = rng.integers(1, int(rng.choice([32, 65])), size=nq)
+                cq, oq = make(rng, ql, alpha)
+                D = np.stack([O.distance_batch(np.tile(cq[oq[q]:oq[q + 1]], n), np.arange(n + 1, dtype=np.int64) * int(ql[q]), cd, od, costs)
+                              for q in range(nq)])
+                # the bound from the oracle's own distances: an occurring D, the double below it, 0 or inf
+                v = float(rng.choice(D.ravel()))
+                bound = [v, float(np.nextafter(v, -np.inf)) if v > 0 else 0.0, 0.0, float("inf")][int(rng.choice([0, 0, 1, 1, 2, 3]))]
+                eng.db_load(R.pack((cd, od), bits=4))
+                try:
+                    off, idx, dist = eng.db_search_range(R.pack((cq, oq), bits=4), bound, force_mode=0 if force == 2 else force)
+                finally:
+                    eng.db_free()
+                ok = off[0] == 0
+                for q in range(nq):
+                    w = np.flatnonzero(D[q] <= bound)
+                    ok = ok and np.array_equal(idx[off[q]:off[q + 1]], w) and np.array_equal(dist[off[q]:off[q + 1]], D[q, w])
+                cells += float(ql.sum()) * float(lens.sum())
+                desc = f"range n={n} q={nq} max_dist={bound!r} hits={int(off[-1])} mode={eng.last_mode}"
             else:
                 n = int(rng.choice([1, 50, 3000, 40000]))
                 lens = rng.integers(0 if rng.random() < 0.3 else 20, int(rng.choice([32, 33, 60])), size=n)
