@@ -148,7 +148,12 @@ int rsd_script_batch(rsd_ctx *ctx,
 /* ---- batched patch: replaces patching(es, str1) (SED:380-457) for scripts produced by
  * rsd_script_batch (closed form, SURVEY a12).  x = the strings to patch (packed like A), one per
  * pair; out: 1 byte per symbol codes in slot p of stride max_out (>= max(len x + n_ops));
- * err[p] in {0, 1, -1} (SED:389-399); out_len[p] = patched length (0 when -1). */
+ * err[p] in {0, 1, -1} (SED:389-399); out_len[p] = patched length (0 when -1).
+ * Scripts must be paths of their pair: op codes 0/1/2 whose counts end at cell (a_len, b_len), and,
+ * where oi / oj are given (either may be NULL), oj[t] = the destination cell entered by an INS or
+ * UPD, oi[t] = the source cell entered by a DEL or UPD.  Scripts of rsd_script_batch and their
+ * reverses (generate_rev_es) are paths; anything else fails with RSD_EINVAL naming the pair and the
+ * op, checked on the host before any device work.  Hand-edited scripts go through sed.patching. */
 int rsd_patch_batch(rsd_ctx *ctx,
                     const uint8_t *op, const int32_t *oi, const int32_t *oj, const int32_t *n_ops, int64_t max_ops,
                     const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len, int64_t a_nwords,

@@ -1327,24 +1327,74 @@ extern "C" int rsd_script_patch_check_batch(rsd_ctx *c,
                          force_mode, max_ops, op, oi, oj, n_ops, dist, ok, mode_out);
 }
 
+// A script handed to rsd_patch_batch must be a path of its pair (m = a_len, n = b_len): op codes in {INS, DEL, UPD},
+// ending at cell (m, n), and where oi / oj are given, the cell each op enters: oj on INS / UPD, oi on DEL / UPD, the
+// indices the reference's sequential patching reads (SED:380-457).  k_finalize rebuilds the entered cells from prefix
+// sums of the ops, so a script with other counts would read past the pair's sequences (extra inserts also write past
+// its max_out slot), and one whose indices disagree with those sums would be patched unlike the reference.  Scripts of
+// rsd_script_batch, their reverses (eswire.rev_packed; the j-2 source index of a reversed delete is on an INS, which
+// is not checked) and any op sequence with the right counts pass; a hand-edited script goes through sed.patching.
+template <bool I, bool J>
+static bool is_patch_path(const uint8_t *op, const int32_t *oi, const int32_t *oj, int32_t k, int32_t m, int32_t n) {
+    uint32_t bad = 0; int32_t ci = 0, cj = 0;
+    for (int32_t t = 0; t < k; ++t) {       // branch-free: 2x (with oi, oj) to 5x (op only) faster than the loop below
+        const uint32_t o = op[t];
+        ci += o != 0u; cj += o != 1u;
+        bad |= (uint32_t)(o > 2u);
+        if constexpr (I) bad |= (uint32_t)(o != 0u) & (uint32_t)(oi[t] != ci);
+        if constexpr (J) bad |= (uint32_t)(o != 1u) & (uint32_t)(oj[t] != cj);
+    }
+    return !bad && ci == m && cj == n;
+}
+
+static int check_patch_path(int64_t p, const uint8_t *op, const int32_t *oi, const int32_t *oj, int32_t k, int32_t m, int32_t n) {
+    static const char *name[3] = {"INS", "DEL", "UPD"};
+    if (oi ? (oj ? is_patch_path<true, true>(op, oi, oj, k, m, n) : is_patch_path<true, false>(op, oi, oj, k, m, n))
+           : (oj ? is_patch_path<false, true>(op, oi, oj, k, m, n) : is_patch_path<false, false>(op, oi, oj, k, m, n)))
+        return RSD_OK;
+    // not a path: find the first offending op for the message
+    int32_t ci = 0, cj = 0;
+    for (int32_t t = 0; t < k; ++t) {
+        const uint32_t o = op[t];
+        if (o > 2u) return rsd_fail(RSD_EINVAL, "rsd_patch_batch: pair %lld op %d: code %u is not INS (0), DEL (1) or UPD (2)",
+                                    (long long)p, t, o);
+        ci += o != 0u; cj += o != 1u;
+        if (ci > m || cj > n)
+            return rsd_fail(RSD_EINVAL, "rsd_patch_batch: pair %lld op %d (%s) enters cell (%d, %d) outside the %d x %d matrix of the pair",
+                            (long long)p, t, name[o], ci, cj, m, n);
+        if (oi && o != 0u && oi[t] != ci)
+            return rsd_fail(RSD_EINVAL, "rsd_patch_batch: pair %lld op %d (%s): oi = %d, the path enters source cell %d",
+                            (long long)p, t, name[o], oi[t], ci);
+        if (oj && o != 1u && oj[t] != cj)
+            return rsd_fail(RSD_EINVAL, "rsd_patch_batch: pair %lld op %d (%s): oj = %d, the path enters destination cell %d",
+                            (long long)p, t, name[o], oj[t], cj);
+    }
+    if (ci != m || cj != n)
+        return rsd_fail(RSD_EINVAL, "rsd_patch_batch: pair %lld ends after its %d ops at cell (%d, %d), not (%d, %d)",
+                        (long long)p, k, ci, cj, m, n);
+    return RSD_OK;
+}
+
 extern "C" int rsd_patch_batch(rsd_ctx *c,
                                const uint8_t *op, const int32_t *oi, const int32_t *oj, const int32_t *n_ops, int64_t max_ops,
                                const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len, int64_t a_nwords,
                                const uint32_t *b_words, const int64_t *b_start, const int32_t *b_len, int64_t b_nwords,
                                const uint32_t *x_words, const int64_t *x_start, const int32_t *x_len, int64_t x_nwords,
                                int64_t n_pairs, int bits, int64_t max_out, uint8_t *out, int32_t *out_len, int32_t *err) {
-    (void)oi; (void)oj;        // derivable from op (prefix sums); accepted for symmetry with rsd_script_batch
     if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
     if (n_pairs < 0) return rsd_fail(RSD_EINVAL, "rsd_patch_batch: n_pairs < 0");
-    if (n_pairs > 0 && (!op || !n_ops || !a_words || !b_words || !x_words || !out || !out_len || !err))
+    if (n_pairs > 0 && (!op || !n_ops || !a_words || !a_len || !b_words || !b_len || !x_words || !x_len || !out || !out_len || !err))
         return rsd_fail(RSD_EINVAL, "rsd_patch_batch: NULL buffer");
     if (bits != 2 && bits != 4) return rsd_fail(RSD_EINVAL, "rsd: bits must be 2 or 4");
-    RSD_OK_OR_RETURN(c->ensure_device());
-    if (n_pairs == 0) return RSD_OK;
+    // host-side validation first, so that a bad script is refused the same way with or without a device
     for (int64_t p = 0; p < n_pairs; ++p) {
         if (n_ops[p] < 0 || n_ops[p] > max_ops) return rsd_fail(RSD_EINVAL, "rsd_patch_batch: n_ops[%lld] out of range", (long long)p);
         if ((int64_t)x_len[p] + b_len[p] > max_out) return rsd_fail(RSD_EINVAL, "rsd_patch_batch: max_out too small for pair %lld", (long long)p);
+        const size_t row = (size_t)p * (size_t)max_ops;
+        RSD_OK_OR_RETURN(check_patch_path(p, op + row, oi ? oi + row : nullptr, oj ? oj + row : nullptr, n_ops[p], a_len[p], b_len[p]));
     }
+    RSD_OK_OR_RETURN(c->ensure_device());
+    if (n_pairs == 0) return RSD_OK;
     cudaStream_t st = c->stream;
     RSD_OK_OR_RETURN(c->upload_seqs(c->bufA, a_words, a_start, a_len, n_pairs, a_nwords, st));
     RSD_OK_OR_RETURN(c->upload_seqs(c->bufB, b_words, b_start, b_len, n_pairs, b_nwords, st));

@@ -184,7 +184,10 @@ class Engine:
         return res
 
     def patch_batch(self, scripts: dict, A: PackedSeqs, B: PackedSeqs, X: PackedSeqs):
-        """patching(es_p, x_p) for scripts from script_batch -> (out codes uint8[n,max_out], out_len, err)."""
+        """patching(es_p, x_p) for scripts from script_batch -> (out codes uint8[n,max_out], out_len, err).
+        Every script must be a path of its pair (A_p -> B_p), like those of script_batch and their reverses
+        (eswire.rev_packed with A and B swapped): RsdError RSD_EINVAL otherwise, before any device work.  Hand-edited
+        scripts go through sed.patching."""
         (A, B, X), bits = self._common_bits(A, B, X)
         n = A.n
         op, oi, oj, n_ops = scripts["op"], scripts["oi"], scripts["oj"], scripts["n_ops"]
