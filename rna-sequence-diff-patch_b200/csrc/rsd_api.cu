@@ -1130,10 +1130,13 @@ int rsd_ctx::script_pipeline(const int32_t *a_len, const int32_t *b_len, int64_t
     // per-pair direction-word counts and chunking
     // The chunk budget is what the direction buffer already holds when that was sized by an earlier call with
     // outputs of at least this size (cudaMemGetInfo costs ~15 ms with tens of GB allocated — measured); otherwise
-    // 70 % of the free memory, at most 24 GiB of direction words per chunk.
+    // 70 % of the free memory, at most 24 GiB of direction words per chunk.  RSD_SCRIPT_BUDGET_WORDS sets the budget of
+    // this call alone (tests: forces the chunked path on small batches); it neither reads nor updates the measured one.
     const int64_t out_bytes = n_pairs * max_ops * (int64_t)((op ? 1 : 0) + (oi ? 4 : 0) + (oj ? 4 : 0)) + n_pairs * 32;
+    const char *forced_budget = getenv("RSD_SCRIPT_BUDGET_WORDS");
     int64_t budget_words;
-    if (dirs.p && dirs_budget_words > 0 && out_bytes <= dirs_budget_out_bytes) budget_words = dirs_budget_words;
+    if (forced_budget) budget_words = atoll(forced_budget);
+    else if (dirs.p && dirs_budget_words > 0 && out_bytes <= dirs_budget_out_bytes) budget_words = dirs_budget_words;
     else {
         size_t free_b = 0, total_b = 0;
         RSD_CUDA(cudaMemGetInfo(&free_b, &total_b));
@@ -1163,7 +1166,10 @@ int rsd_ctx::script_pipeline(const int32_t *a_len, const int32_t *b_len, int64_t
     for (size_t k = 0; k + 1 < chunk_start.size(); ++k) chunk_max_pairs = std::max(chunk_max_pairs, chunk_start[k + 1] - chunk_start[k]);
 
     const double t_plan = now();
-    if (int rc = dirs.ensure(sizeof(uint32_t) * (size_t)(chunk_max_words + 64))) { dirs_budget_words = 0; return rc; }   // re-measure next time
+    if (int rc = dirs.ensure(sizeof(uint32_t) * (size_t)(chunk_max_words + 64))) {
+        if (!forced_budget) dirs_budget_words = 0;                                          // re-measure next time
+        return rc;
+    }
     RSD_OK_OR_RETURN(misc.ensure(sizeof(int64_t) * (size_t)n_pairs));                      // dir_off
     RSD_OK_OR_RETURN(s_tmp.ensure((size_t)chunk_max_pairs * max_ops + 16));
     RSD_OK_OR_RETURN(s_nops.ensure(sizeof(int32_t) * (size_t)n_pairs));
