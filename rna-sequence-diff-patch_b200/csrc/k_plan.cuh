@@ -38,6 +38,7 @@ struct PlanView {
     int MQ;               // row bins per class for this call: min((max_m >> m_shift) + 2, RSD_MQ_MAX)
     int NSC;              // strip classes for this call: min(max_ns, RSD_NSQ_MAX + 1); classes 1..NSC
     int NB;               // NSC * MQ
+    int band;             // tasks for k_dist_band16: 32 groups each, no tape (every class <= RSD_NSQ_MAX)
     unsigned long long *dbg;
 };
 
@@ -77,6 +78,12 @@ __host__ __device__ __forceinline__ void tape_shape(int nsq, int &P, int &G) {
     // utilisation ratio best/shortest = (bg/bp) / (g0/pmin) >= 1.08 ?
     if ((long long)bg * pmin * 100 < (long long)g0 * bp * RSD_TAPE_GAIN) { bp = pmin; bg = g0; }
     P = bp; G = bg;
+}
+
+// groups per task and passes of the layout the plan is cut for
+__host__ __device__ __forceinline__ void task_shape(const PlanView &pv, int nsq, int &P, int &G) {
+    if (pv.band) { P = 1; G = 32; return; }
+    tape_shape(nsq, P, G);
 }
 
 // trivial pairs are answered here: D = n*ins (m == 0) or m*del (n == 0) — one fp64 multiply,
@@ -161,7 +168,7 @@ __device__ __forceinline__ void plan_scan_block(const PlanView &pv) {      // on
             pv.bin_warp_off[ci] = tasks;
             const int groups = pv.bin_group_off[(ci + 1) * pv.MQ] - pv.bin_group_off[ci * pv.MQ];
             int P, G;
-            tape_shape(pv.NSC - ci, P, G);
+            task_shape(pv, pv.NSC - ci, P, G);
             tasks += (groups + G - 1) / G;
         }
         pv.bin_warp_off[pv.NSC] = tasks;
@@ -235,7 +242,7 @@ __device__ __forceinline__ TapeTask plan_decode(const PlanView &pv, int W) {
     const int ci = lo;
     const int nsq = pv.NSC - ci;
     int P, G;
-    tape_shape(nsq, P, G);
+    task_shape(pv, nsq, P, G);
     const int gbase = __ldg(&pv.bin_group_off[ci * pv.MQ]);
     const int gcount = __ldg(&pv.bin_group_off[(ci + 1) * pv.MQ]) - gbase;
     const int wl = W - __ldg(&pv.bin_warp_off[ci]);

@@ -371,7 +371,7 @@ static int persistent_grid(K kernel, int threads, int sm_count, int &blocks) {
 }
 
 int rsd_ctx::make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_pairs, int C, int allow_twin,
-                       double *d_out, cudaStream_t st, PlanView &pv, int64_t max_m, int64_t max_n) {
+                       double *d_out, cudaStream_t st, PlanView &pv, int64_t max_m, int64_t max_n, int band) {
     PlanSlot &sl = ps();
     RSD_OK_OR_RETURN(sl.pair_bin.ensure(sizeof(int) * (size_t)n_pairs));
     const size_t plan_ints = (size_t)(2 * RSD_PLAN_COPIES) * RSD_NB_MAX + 2 * (RSD_NB_MAX + 1) + 16;
@@ -400,7 +400,7 @@ int rsd_ctx::make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_p
     pv.totals = pv.bin_warp_off + (RSD_NB_MAX + 1);
     pv.work_counter = pv.totals + 4;
     pv.groups = (int2 *)sl.groups.p;
-    pv.C = C; pv.allow_twin = allow_twin;
+    pv.C = C; pv.allow_twin = allow_twin; pv.band = band;
     pv.dbg = getenv("RSD_TRACE_PLAN") ? (unsigned long long *)(pv.totals + 6) : nullptr;      // synchronises after every plan
     // bin counters are zeroed again by the scan phase, which also resets cursors / ticket / odd-twin
     // slots — so a plan is three kernels and no memsets.  A call that failed between count and
@@ -437,6 +437,9 @@ int rsd_ctx::make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_p
 // ------------------------------------------------------------------------------------------------
 // distance batch
 // ------------------------------------------------------------------------------------------------
+// Longest sequence of a batch the int16x2 distance takes the band kernel for by default (DESIGN §4): its hand-off buffer
+// takes 128 bytes per row and warp of the longest sequence, in every plan slot of a call
+#define RSD_BAND_MAX_LEN 512
 int rsd_ctx::distance_plan(const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n,
                            int bits, uint32_t symmask, int force_mode, double *d_out, int *mode_out, cudaStream_t st) {
     if (n_pairs < 0 || n_pairs > INT32_MAX) return rsd_fail(RSD_ERANGE, "rsd: n_pairs out of range");
@@ -450,7 +453,20 @@ int rsd_ctx::distance_plan(const int32_t *a_len, const int32_t *b_len, int64_t n
     if (n_pairs == 0) return RSD_OK;
     if (!costs_preloaded) RSD_OK_OR_RETURN(upload_costs(sl.mi, st));
     const int C = sl.mi.mode == RSD_MODE_F64 ? 16 : 32;
-    return make_plan(a_len, b_len, n_pairs, C, sl.mi.mode == RSD_MODE_I16X2 ? 1 : 0, d_out, st, sl.pv, max_m, max_n);
+    // Layout of the int16x2 kernel.  The band kernel needs ins > 0 and del > 0 (else the band has no bound) and every
+    // pair in a strip class of its own (<= RSD_NSQ_MAX strips).  It takes 64 pairs per warp task, so by default it runs
+    // when the batch gives every resident warp at least one task (measured crossover at C2 shapes: 1.5 * 10^5 pairs =
+    // 2344 tasks on 2368 warps, DESIGN §4) and no sequence is longer than RSD_BAND_MAX_LEN.  RSD_DIST_BAND=0|1 forces
+    // the choice wherever the band kernel applies.
+    bool band = false;
+    const int64_t longest = std::max(max_m, max_n);
+    if (sl.mi.mode == RSD_MODE_I16X2 && sl.mi.ic.ins > 0 && sl.mi.ic.del > 0 && (longest + C - 1) / C <= RSD_NSQ_MAX) {
+        int blocks = 0;
+        RSD_OK_OR_RETURN(persistent_grid(k_dist_band16<32>, 128, sm_count, blocks));
+        band = longest <= RSD_BAND_MAX_LEN && n_pairs >= (int64_t)64 * 4 * blocks;
+        if (const char *e = getenv("RSD_DIST_BAND")) band = atoi(e) != 0;
+    }
+    return make_plan(a_len, b_len, n_pairs, C, sl.mi.mode == RSD_MODE_I16X2 ? 1 : 0, d_out, st, sl.pv, max_m, max_n, band ? 1 : 0);
 }
 
 int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len,
@@ -465,7 +481,27 @@ int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, co
     const int wpb = THREADS / 32;
     int blocks = 0;
     const int stride = (int)max_m;           // two boundary columns of max_m rows per warp (tape passes)
-    if (mi.mode == RSD_MODE_I16X2) {
+    if (mi.mode == RSD_MODE_I16X2 && pv.band) {
+        RSD_OK_OR_RETURN(persistent_grid(k_dist_band16<32>, THREADS, sm_count, blocks));
+        const int rows = (int)std::max<int64_t>(max_m, sl.max_n);       // rows after the orientation choice
+        RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(uint32_t) * 32 * (size_t)rows * blocks * wpb + 16));
+        unsigned long long *trace = nullptr;
+        if (getenv("RSD_TRACE")) {
+            RSD_OK_OR_RETURN(sl.trace.ensure(3 * sizeof(unsigned long long)));
+            trace = (unsigned long long *)sl.trace.p;
+            RSD_CUDA(cudaMemsetAsync(trace, 0, 3 * sizeof(unsigned long long), st));
+        }
+        if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
+        k_dist_band16<32><<<blocks, THREADS, 0, st>>>(pv, A, B, mi.ic, d_out, (uint32_t *)sl.scratch.p, rows, 1u, trace);
+        if (trace) {                      // synchronises after the launch: not for timing runs
+            unsigned long long h[3];
+            RSD_CUDA(cudaMemcpyAsync(h, trace, sizeof h, cudaMemcpyDeviceToHost, st));
+            RSD_CUDA(cudaStreamSynchronize(st));
+            fprintf(stderr, "[rsd trace] k_dist_band16: %lld pairs, cell slots %.4g = %.3f x sum(m*n) %.4g = %.3f x the strip-padded cells %.4g\n",
+                    (long long)sl.n_pairs, (double)h[0], (double)h[0] / std::max(1.0, (double)h[1]), (double)h[1],
+                    (double)h[0] / std::max(1.0, (double)h[2]), (double)h[2]);
+        }
+    } else if (mi.mode == RSD_MODE_I16X2) {
         RSD_OK_OR_RETURN(persistent_grid(k_dist_twin16<32>, THREADS, sm_count, blocks));
         const int stride2 = (int)std::max<int64_t>(max_m, sl.max_n);     // rows after the orientation choice
         RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(uint32_t) * 2 * (size_t)stride2 * blocks * wpb + 16));
@@ -1200,7 +1236,7 @@ int rsd_ctx::script_pipeline(const int32_t *a_len, const int32_t *b_len, int64_t
         SeqView A{dA, sA + p0, lA + p0}, B{dB, sB + p0, lB + p0};
         PlanView pv;
         // trivial pairs (m == 0 or n == 0) get their distance from the planner and an all-INS / all-DEL script from the traceback
-        RSD_OK_OR_RETURN(make_plan(lA + p0, lB + p0, np, C, 0, (double *)out_f64.p + p0, st, pv, max_m, max_n));
+        RSD_OK_OR_RETURN(make_plan(lA + p0, lB + p0, np, C, 0, (double *)out_f64.p + p0, st, pv, max_m, max_n, 0));
         ScriptView sv{(uint32_t *)dirs.p, (const int64_t *)misc.p + p0, (double *)out_f64.p + p0};
         if (f64) {
             if (bits == 2) k_script_fwd<true, 2, 16><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, sv, S, ps().scratch.p, stride, -1);

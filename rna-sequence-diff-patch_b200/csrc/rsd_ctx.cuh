@@ -64,12 +64,12 @@ struct ModeInfo {
 // Plan arrays + hand-off scratch of one batch in flight; the chunks of a host call use one slot each so their
 // kernels may overlap, everything else uses slot 0.
 struct PlanSlot {
-    DevBuf scratch, pair_bin, bins, groups;
+    DevBuf scratch, pair_bin, bins, groups, trace;
     bool dirty = true;           // bin counters need a memset before the next plan
     PlanView pv;
     ModeInfo mi;
     int64_t n_pairs = 0, max_n = 0;
-    void release() { scratch.release(); pair_bin.release(); bins.release(); groups.release(); dirty = true; }
+    void release() { scratch.release(); pair_bin.release(); bins.release(); groups.release(); trace.release(); dirty = true; }
 };
 
 // Hits of a range search on the host, query by query in the order the search saw the queries: cnt[q] hits each,
@@ -141,7 +141,7 @@ struct rsd_ctx {
     int upload_seqs(SeqBufs &sb, const uint32_t *words, const int64_t *start, const int32_t *len, int64_t n,
                     int64_t n_words, cudaStream_t st);
     int make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_pairs, int C, int allow_twin, double *d_out,
-                  cudaStream_t st, PlanView &pv, int64_t max_m, int64_t max_n);
+                  cudaStream_t st, PlanView &pv, int64_t max_m, int64_t max_n, int band);
     int distance_plan(const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n, int bits,
                       uint32_t symmask, int force_mode, double *d_out, int *mode_out, cudaStream_t st);
     int distance_launch(const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len, const uint32_t *b_words,

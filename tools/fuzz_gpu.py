@@ -98,11 +98,17 @@ def main():
                 while float((la.astype(np.float64) * lb).sum()) > budget and n > 1:
                     n //= 2; la, lb = la[:n], lb[:n]
                 ca, oa = make(rng, la, alpha); cb, ob = make(rng, lb, alpha)
-                got = eng.distance_batch(R.pack((ca, oa)), R.pack((cb, ob)), force_mode=force)
+                knobs = {}
+                if rng.random() < 0.6: knobs["RSD_DIST_BAND"] = str(rng.choice([0, 1]))     # int16x2 layout: band / tape
+                os.environ.update(knobs)
+                try:
+                    got = eng.distance_batch(R.pack((ca, oa)), R.pack((cb, ob)), force_mode=force)
+                finally:
+                    for kname in knobs: del os.environ[kname]
                 want = O.distance_batch(ca, oa, cb, ob, costs)
                 ok = np.array_equal(got, want)
                 cells += float((la.astype(np.float64) * lb).sum())
-                desc = f"dist n={n} mode={eng.last_mode}"
+                desc = f"dist n={n} mode={eng.last_mode} knobs={knobs}"
             elif what == "script":
                 n = int(rng.choice([1, 5, 200, 2000]))
                 if lkind in ("kb", "wide", "skew"):
