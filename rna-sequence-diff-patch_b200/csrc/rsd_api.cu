@@ -91,7 +91,6 @@ int rsd_ctx::ensure_device() {
     RSD_CUDA(cudaEventCreate(&ev_begin));
     RSD_CUDA(cudaEventCreate(&ev0));
     RSD_CUDA(cudaEventCreate(&ev1));
-    cur_ev0 = ev0; cur_ev1 = ev1;
     for (int k = 0; k < RSD_MAX_CHUNKS; ++k) {
         RSD_CUDA(cudaEventCreate(&ev_t0[k])); RSD_CUDA(cudaEventCreate(&ev_t1[k]));
         RSD_CUDA(cudaEventCreateWithFlags(&ev_done[k], cudaEventDisableTiming));
@@ -370,9 +369,8 @@ static int persistent_grid(K kernel, int threads, int sm_count, int &blocks) {
     return RSD_OK;
 }
 
-int rsd_ctx::make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_pairs, int C, int allow_twin,
+int rsd_ctx::make_plan(PlanSlot &sl, const int32_t *d_alen, const int32_t *d_blen, int64_t n_pairs, int C, int allow_twin,
                        double *d_out, cudaStream_t st, PlanView &pv, int64_t max_m, int64_t max_n, int band) {
-    PlanSlot &sl = ps();
     RSD_OK_OR_RETURN(sl.pair_bin.ensure(sizeof(int) * (size_t)n_pairs));
     const size_t plan_ints = (size_t)(2 * RSD_PLAN_COPIES) * RSD_NB_MAX + 2 * (RSD_NB_MAX + 1) + 16;
     {
@@ -440,18 +438,18 @@ int rsd_ctx::make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_p
 // Longest sequence of a batch the int16x2 distance takes the band kernel for by default (DESIGN §4): its hand-off buffer
 // takes 128 bytes per row and warp of the longest sequence, in every plan slot of a call
 #define RSD_BAND_MAX_LEN 512
-int rsd_ctx::distance_plan(const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n,
-                           int bits, uint32_t symmask, int force_mode, double *d_out, int *mode_out, cudaStream_t st) {
+// Plans a batch into `sl`: its numeric mode, the kernel layout and the plan arrays.  load_costs = false when the caller
+// has already uploaded the cost tables of this classification.
+int rsd_ctx::distance_plan(PlanSlot &sl, const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n,
+                           int bits, uint32_t symmask, int force_mode, bool load_costs, double *d_out, int *mode_out, cudaStream_t st) {
     if (n_pairs < 0 || n_pairs > INT32_MAX) return rsd_fail(RSD_ERANGE, "rsd: n_pairs out of range");
     if (bits != 2 && bits != 4) return rsd_fail(RSD_EINVAL, "rsd: bits must be 2 or 4");
     if (bits == 2 && (symmask & ~0xFu)) return rsd_fail(RSD_EINVAL, "rsd: 2-bit packing with symbols outside ACGU");
-    PlanSlot &sl = ps();
     RSD_OK_OR_RETURN(classify(symmask, max_m, max_n, bits, force_mode, sl.mi));
     if (mode_out) *mode_out = sl.mi.mode;
-    timed = false; last_ms_override = 0.0;
     sl.n_pairs = n_pairs; sl.max_n = max_n;
     if (n_pairs == 0) return RSD_OK;
-    if (!costs_preloaded) RSD_OK_OR_RETURN(upload_costs(sl.mi, st));
+    if (load_costs) RSD_OK_OR_RETURN(upload_costs(sl.mi, st));
     const int C = sl.mi.mode == RSD_MODE_F64 ? 16 : 32;
     // Layout of the int16x2 kernel.  The band kernel needs ins > 0 and del > 0 (else the band has no bound) and every
     // pair in a strip class of its own (<= RSD_NSQ_MAX strips).  It takes 64 pairs per warp task, so by default it runs
@@ -466,13 +464,13 @@ int rsd_ctx::distance_plan(const int32_t *a_len, const int32_t *b_len, int64_t n
         band = longest <= RSD_BAND_MAX_LEN && n_pairs >= (int64_t)64 * 4 * blocks;
         if (const char *e = getenv("RSD_DIST_BAND")) band = atoi(e) != 0;
     }
-    return make_plan(a_len, b_len, n_pairs, C, sl.mi.mode == RSD_MODE_I16X2 ? 1 : 0, d_out, st, sl.pv, max_m, max_n, band ? 1 : 0);
+    return make_plan(sl, a_len, b_len, n_pairs, C, sl.mi.mode == RSD_MODE_I16X2 ? 1 : 0, d_out, st, sl.pv, max_m, max_n, band ? 1 : 0);
 }
 
-int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len,
+// The distance kernel of the batch planned into `sl`.  Events t0 / t1 (when not null) are recorded around the launch.
+int rsd_ctx::distance_launch(PlanSlot &sl, const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len,
                              const uint32_t *b_words, const int64_t *b_start, const int32_t *b_len,
-                             int64_t max_m, int bits, double *d_out, cudaStream_t st) {
-    PlanSlot &sl = ps();
+                             int64_t max_m, int bits, double *d_out, cudaStream_t st, cudaEvent_t t0, cudaEvent_t t1) {
     if (sl.n_pairs == 0) return RSD_OK;
     const ModeInfo &mi = sl.mi;
     const PlanView &pv = sl.pv;
@@ -480,7 +478,6 @@ int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, co
     constexpr int THREADS = 128;
     const int wpb = THREADS / 32;
     int blocks = 0;
-    const int stride = (int)max_m;           // two boundary columns of max_m rows per warp (tape passes)
     if (mi.mode == RSD_MODE_I16X2 && pv.band) {
         RSD_OK_OR_RETURN(persistent_grid(k_dist_band16<32>, THREADS, sm_count, blocks));
         const int rows = (int)std::max<int64_t>(max_m, sl.max_n);       // rows after the orientation choice
@@ -491,7 +488,7 @@ int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, co
             trace = (unsigned long long *)sl.trace.p;
             RSD_CUDA(cudaMemsetAsync(trace, 0, 3 * sizeof(unsigned long long), st));
         }
-        if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
+        if (t0) RSD_CUDA(cudaEventRecord(t0, st));
         k_dist_band16<32><<<blocks, THREADS, 0, st>>>(pv, A, B, mi.ic, d_out, (uint32_t *)sl.scratch.p, rows, 1u, trace);
         if (trace) {                      // synchronises after the launch: not for timing runs
             unsigned long long h[3];
@@ -505,34 +502,23 @@ int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, co
         RSD_OK_OR_RETURN(persistent_grid(k_dist_twin16<32>, THREADS, sm_count, blocks));
         const int stride2 = (int)std::max<int64_t>(max_m, sl.max_n);     // rows after the orientation choice
         RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(uint32_t) * 2 * (size_t)stride2 * blocks * wpb + 16));
-        if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
+        if (t0) RSD_CUDA(cudaEventRecord(t0, st));
         k_dist_twin16<32><<<blocks, THREADS, 0, st>>>(pv, A, B, mi.ic, d_out, (uint32_t *)sl.scratch.p, stride2, 1u);
-    } else if (mi.mode == RSD_MODE_I32) {
-        if (bits == 2) {
-            RSD_OK_OR_RETURN(persistent_grid(k_dist_gen<int, 2, 32>, THREADS, sm_count, blocks));
-            RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(int) * 2 * (size_t)stride * blocks * wpb + 16));
-            if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
-            k_dist_gen<int, 2, 32><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, d_out, (int *)sl.scratch.p, stride);
-        } else {
-            RSD_OK_OR_RETURN(persistent_grid(k_dist_gen<int, 4, 32>, THREADS, sm_count, blocks));
-            RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(int) * 2 * (size_t)stride * blocks * wpb + 16));
-            if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
-            k_dist_gen<int, 4, 32><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, d_out, (int *)sl.scratch.p, stride);
-        }
     } else {
-        if (bits == 2) {
-            RSD_OK_OR_RETURN(persistent_grid(k_dist_gen<double, 2, 16>, THREADS, sm_count, blocks));
-            RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(double) * 2 * (size_t)stride * blocks * wpb + 16));
-            if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
-            k_dist_gen<double, 2, 16><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, d_out, (double *)sl.scratch.p, stride);
-        } else {
-            RSD_OK_OR_RETURN(persistent_grid(k_dist_gen<double, 4, 16>, THREADS, sm_count, blocks));
-            RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(double) * 2 * (size_t)stride * blocks * wpb + 16));
-            if (timing) RSD_CUDA(cudaEventRecord(cur_ev0, st));
-            k_dist_gen<double, 4, 16><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, d_out, (double *)sl.scratch.p, stride);
-        }
+        // general kernels: two boundary columns of max_m rows per warp (tape passes); `elem` has the scratch element type
+        auto launch_gen = [&](auto kernel, auto elem) -> int {
+            using T = decltype(elem);
+            const int stride = (int)max_m;
+            RSD_OK_OR_RETURN(persistent_grid(kernel, THREADS, sm_count, blocks));
+            RSD_OK_OR_RETURN(sl.scratch.ensure(sizeof(T) * 2 * (size_t)stride * blocks * wpb + 16));
+            if (t0) RSD_CUDA(cudaEventRecord(t0, st));
+            kernel<<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, d_out, (T *)sl.scratch.p, stride);
+            return RSD_OK;
+        };
+        if (mi.mode == RSD_MODE_I32) RSD_OK_OR_RETURN(launch_gen(bits == 2 ? k_dist_gen<int, 2, 32> : k_dist_gen<int, 4, 32>, 0));
+        else RSD_OK_OR_RETURN(launch_gen(bits == 2 ? k_dist_gen<double, 2, 16> : k_dist_gen<double, 4, 16>, 0.0));
     }
-    if (timing) { RSD_CUDA(cudaEventRecord(cur_ev1, st)); timed = true; }
+    if (t1) RSD_CUDA(cudaEventRecord(t1, st));
     launches += 1;
     RSD_CUDA(cudaGetLastError());
     return RSD_OK;
@@ -541,10 +527,10 @@ int rsd_ctx::distance_launch(const uint32_t *a_words, const int64_t *a_start, co
 int rsd_ctx::distance_dev(const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len,
                           const uint32_t *b_words, const int64_t *b_start, const int32_t *b_len,
                           int64_t n_pairs, int64_t max_m, int64_t max_n, int bits, uint32_t symmask,
-                          int force_mode, double *d_out, int *mode_out, cudaStream_t st) {
-    cur_slot = 0;
-    RSD_OK_OR_RETURN(distance_plan(a_len, b_len, n_pairs, max_m, max_n, bits, symmask, force_mode, d_out, mode_out, st));
-    return distance_launch(a_words, a_start, a_len, b_words, b_start, b_len, max_m, bits, d_out, st);
+                          int force_mode, double *d_out, int *mode_out, cudaStream_t st, cudaEvent_t t0, cudaEvent_t t1) {
+    PlanSlot &sl = slots[0];
+    RSD_OK_OR_RETURN(distance_plan(sl, a_len, b_len, n_pairs, max_m, max_n, bits, symmask, force_mode, true, d_out, mode_out, st));
+    return distance_launch(sl, a_words, a_start, a_len, b_words, b_start, b_len, max_m, bits, d_out, st, t0, t1);
 }
 
 extern "C" int rsd_distance_batch_dev(rsd_ctx *c,
@@ -554,8 +540,13 @@ extern "C" int rsd_distance_batch_dev(rsd_ctx *c,
                                       int force_mode, double *out, int *mode_out, void *stream) {
     if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
     RSD_OK_OR_RETURN(c->ensure_device());
-    return c->distance_dev(a_words, a_start, a_len, b_words, b_start, b_len, n_pairs, max_m, max_n, bits, symmask,
-                           force_mode, out, mode_out, (cudaStream_t)stream);
+    // the kernel alone is timed
+    c->timed = false; c->last_ms_override = 0.0;
+    const bool timed = c->timing && n_pairs > 0;
+    RSD_OK_OR_RETURN(c->distance_dev(a_words, a_start, a_len, b_words, b_start, b_len, n_pairs, max_m, max_n, bits, symmask,
+                                     force_mode, out, mode_out, (cudaStream_t)stream, timed ? c->ev0 : nullptr, timed ? c->ev1 : nullptr));
+    c->timed = timed;
+    return RSD_OK;
 }
 
 static int64_t max_len(const int32_t *len, int64_t n) {
@@ -698,20 +689,18 @@ static int distance_host(rsd_ctx *c, const SideIn in[2], int64_t n_pairs, int64_
     }
     bounds[n_chunks] = n_pairs;
     t_len = now();
+    // the chunk kernels are timed (ev_t0 / ev_t1 of each chunk) and their times summed
     const bool timing = c->timing;
     float kernel_ms = 0.f;
-    struct SlotReset { rsd_ctx *c; ~SlotReset() { c->cur_slot = 0; c->costs_preloaded = false; c->cur_ev0 = c->ev0; c->cur_ev1 = c->ev1; } } slot_reset{c};
-    c->costs_preloaded = true;
+    c->timed = false; c->last_ms_override = 0.0;
     RSD_CUDA(cudaStreamWaitEvent(st, c->ev_len, 0));
     auto enqueue_plans = [&]() -> int {
         for (int k = 0; k < n_chunks; ++k) {
             const int64_t p0 = bounds[k], p1 = bounds[k + 1];
             if (p1 <= p0) continue;
-            c->cur_slot = k;
-            RSD_OK_OR_RETURN(c->distance_plan((const int32_t *)dS[0]->len.p + p0, (const int32_t *)dS[1]->len.p + p0, p1 - p0, max_m, max_n, bits,
-                                              symmask, force_mode, (double *)c->out_f64.p + p0, mode_out, st));
+            RSD_OK_OR_RETURN(c->distance_plan(c->slots[k], (const int32_t *)dS[0]->len.p + p0, (const int32_t *)dS[1]->len.p + p0, p1 - p0, max_m, max_n,
+                                              bits, symmask, force_mode, false, (double *)c->out_f64.p + p0, mode_out, st));
         }
-        c->cur_slot = 0;
         RSD_CUDA(cudaEventRecord(c->ev_plans, st));
         RSD_CUDA(cudaStreamWaitEvent(c->stream2, c->ev_plans, 0));
         return RSD_OK;
@@ -721,11 +710,9 @@ static int distance_host(rsd_ctx *c, const SideIn in[2], int64_t n_pairs, int64_
     // chunk's blocks move in while the last tasks of the previous chunk drain, so a chunk boundary costs no idle SMs
     auto launch_chunk = [&](int k, cudaStream_t sk) -> int {
         const int64_t p0 = bounds[k], p1 = bounds[k + 1];
-        c->cur_slot = k;
-        c->cur_ev0 = c->ev_t0[k]; c->cur_ev1 = c->ev_t1[k];
-        RSD_OK_OR_RETURN(c->distance_launch((const uint32_t *)dS[0]->words.p, (const int64_t *)dS[0]->start.p + p0, (const int32_t *)dS[0]->len.p + p0,
+        RSD_OK_OR_RETURN(c->distance_launch(c->slots[k], (const uint32_t *)dS[0]->words.p, (const int64_t *)dS[0]->start.p + p0, (const int32_t *)dS[0]->len.p + p0,
                                             (const uint32_t *)dS[1]->words.p, (const int64_t *)dS[1]->start.p + p0, (const int32_t *)dS[1]->len.p + p0,
-                                            max_m, bits, (double *)c->out_f64.p + p0, sk));
+                                            max_m, bits, (double *)c->out_f64.p + p0, sk, timing ? c->ev_t0[k] : nullptr, timing ? c->ev_t1[k] : nullptr));
         // results go back on their own stream, behind nothing but the chunk's kernel
         RSD_CUDA(cudaEventRecord(c->ev_done[k], sk));
         RSD_CUDA(cudaStreamWaitEvent(c->d2h_stream, c->ev_done[k], 0));
@@ -804,7 +791,7 @@ static int distance_host(rsd_ctx *c, const SideIn in[2], int64_t n_pairs, int64_
         }
         for (int s = 0; s < 2; ++s) if (in[s].canonical()) {
             auto job = [&in, &tab, &neg_len, n_pairs, sh, nblk, b_first, s] { block_sums(in[s].len, n_pairs, sh, b_first, nblk, tab[s][0], in[s].codes ? tab[s][1] : nullptr, &neg_len); };
-            if (b_first < nblk) { if (n_pairs >= (1 << 17) && !getenv("RSD_NO_HELPERS")) helpers[s] = std::thread(job); else job(); }
+            if (b_first < nblk) { if (n_pairs >= (1 << 17)) helpers[s] = std::thread(job); else job(); }
         }
         int64_t sent0[2] = {0, 0};                       // symbols of chunk 0 already on their way
         for (int s = 0; s < 2; ++s) if (in[s].canonical()) {
@@ -913,7 +900,7 @@ static int distance_host(rsd_ctx *c, const SideIn in[2], int64_t n_pairs, int64_
             RSD_CUDA(cudaEventElapsedTime(&ms, c->ev_t0[k], c->ev_t1[k]));
             kernel_ms += ms;
         }
-        c->timed = false; c->last_ms_override = kernel_ms;
+        c->last_ms_override = kernel_ms;
         if (trace) {
             for (int k = 0; k < n_chunks; ++k) {
                 if (bounds[k + 1] <= bounds[k]) continue;
@@ -940,17 +927,21 @@ static void unpack_symbols(const uint32_t *words, int64_t word0, int32_t len, in
     if (j < len) { uint32_t x = words[word0 + j / per]; for (; j < len; ++j) { out[j] = (uint8_t)(x & msk); x >>= bits; } }
 }
 
-// Batches whose cells lie mostly in pairs of several thousand symbols: the panel-wavefront kernels (rsd_long_pairs,
-// distance only) run them at 2.7 TCUPS where one warp per pair with tape passes manages 1.0 / 0.5 / 0.25 TCUPS at
-// 5 / 10 / 20 kb (tools/dbg_mid_pairs.py).  -> 1 routed (out filled), 0 not applicable, < 0 error.
-static int distance_route_long(rsd_ctx *c, const SideIn in[2], int64_t n_pairs, int bits, int force_mode, double *out, int *mode_out) {
-    if (n_pairs > 65536 || force_mode == RSD_MODE_I16X2 || getenv("RSD_DIST_NO_LONG")) return 0;      // (a forced int16x2 mode keeps its own applicability error)
-    int64_t T = 6144;                                  // by wall time the tape-pass kernel still wins at 4-5 kb (tools/dbg_crossover.py)
-    if (const char *e = getenv("RSD_DIST_LONG_MIN")) T = std::max<int64_t>(atoll(e), 1);
+// Per-pair edit scripts of a batch that route_long sends to the panel kernels: rows of max_ops entries (rsd_script_batch).
+struct LongScripts { int64_t max_ops; uint8_t *op; int32_t *oi, *oj, *n_ops; };
+
+// Batches whose cells lie mostly in pairs of at least T symbols go to the panel-wavefront kernels (rsd_long_pairs).  One
+// warp per pair with tape passes, the design of k_dist_* / k_script_fwd for 1-2 kb pairs, runs distances at 1.0 / 0.5 /
+// 0.25 TCUPS and scripts at 450 / 240 / 35 GCUPS at 5 / 10 / 20 kb, where the panel pipeline runs at 2.7 and 1.0-1.4
+// TCUPS (tools/dbg_mid_pairs.py).  With `scripts` the scripts come back too; T <= 0 never routes; `who` prefixes the
+// messages.  -> 1 routed (out filled), 0 not applicable, < 0 error.
+static int route_long(rsd_ctx *c, const char *who, int64_t T, const SideIn in[2], int64_t n_pairs, int bits, int force_mode,
+                      const LongScripts *scripts, double *out, int *mode_out) {
+    if (T <= 0 || n_pairs > 65536 || force_mode == RSD_MODE_I16X2) return 0;      // (a forced int16x2 mode keeps its own applicability error)
     double cells_all = 0, cells_long = 0; int64_t total[2] = {0, 0};
     for (int64_t p = 0; p < n_pairs; ++p) {
         const int32_t m = in[0].len[p], n = in[1].len[p];
-        if (m < 0 || n < 0) return -rsd_fail(RSD_EINVAL, "rsd_distance_batch: negative length");
+        if (m < 0 || n < 0) return -rsd_fail(RSD_EINVAL, "%s: negative length", who);
         const double cells = (double)m * (double)n;
         cells_all += cells; total[0] += m; total[1] += n;
         if (std::max(m, n) >= T) cells_long += cells;
@@ -959,28 +950,50 @@ static int distance_route_long(rsd_ctx *c, const SideIn in[2], int64_t n_pairs, 
     const int per = 32 / bits;
     std::vector<uint8_t> codes[2];
     std::vector<const uint8_t *> ptr[2]; std::vector<int64_t> len64[2];
+    int64_t at[2] = {0, 0}, wat[2] = {0, 0};          // symbol / word offset of the canonical layouts
     for (int s = 0; s < 2; ++s) {
         ptr[s].resize((size_t)n_pairs); len64[s].resize((size_t)n_pairs);
         if (!in[s].codes) codes[s].resize((size_t)total[s] + 16);
-        int64_t at = 0, wat = 0;                      // symbol / word offset of the canonical layouts
-        for (int64_t p = 0; p < n_pairs; ++p) {
+    }
+    for (int64_t p = 0; p < n_pairs; ++p) {
+        for (int s = 0; s < 2; ++s) {
             const int32_t len = in[s].len[p];
             len64[s][(size_t)p] = len;
-            if (in[s].codes) { ptr[s][(size_t)p] = in[s].codes + at; at += len; continue; }
-            const int64_t st0 = in[s].start ? in[s].start[p] : wat;
+            if (in[s].codes) { ptr[s][(size_t)p] = in[s].codes + at[s]; at[s] += len; continue; }
+            const int64_t st0 = in[s].start ? in[s].start[p] : wat[s];
             const int64_t nw = ((int64_t)len + per - 1) / per;
-            if (st0 < 0 || st0 + nw > in[s].nwords) return -rsd_fail(RSD_EINVAL, "rsd_distance_batch: pair %lld lies outside the word buffer", (long long)p);
-            ptr[s][(size_t)p] = codes[s].data() + at;
-            unpack_symbols(in[s].words, st0, len, bits, codes[s].data() + at); at += len;
-            wat += nw;
+            if (st0 < 0 || st0 + nw > in[s].nwords) return -rsd_fail(RSD_EINVAL, "%s: pair %lld lies outside the word buffer", who, (long long)p);
+            ptr[s][(size_t)p] = codes[s].data() + at[s];
+            unpack_symbols(in[s].words, st0, len, bits, codes[s].data() + at[s]); at[s] += len;
+            wat[s] += nw;
         }
+        if (scripts && (int64_t)in[0].len[p] + in[1].len[p] > scripts->max_ops)
+            return -rsd_fail(RSD_EINVAL, "%s: max_ops too small for pair %lld", who, (long long)p);
+    }
+    const size_t n_rows = scripts ? (size_t)n_pairs : 0;
+    std::vector<int64_t> mo(n_rows, scripts ? scripts->max_ops : 0), no64(n_rows, 0);
+    std::vector<uint8_t *> pop(n_rows); std::vector<int32_t *> poi(n_rows), poj(n_rows);
+    for (size_t p = 0; p < n_rows; ++p) {
+        const size_t row = p * (size_t)scripts->max_ops;
+        pop[p] = scripts->op + row;
+        poi[p] = scripts->oi ? scripts->oi + row : nullptr; poj[p] = scripts->oj ? scripts->oj + row : nullptr;
     }
     std::vector<int> modes((size_t)n_pairs, 0);
-    const int rc = rsd_long_pairs(c, (int)n_pairs, ptr[0].data(), len64[0].data(), ptr[1].data(), len64[1].data(), force_mode == RSD_MODE_I16X2 ? 0 : force_mode, 0,
-                                  nullptr, nullptr, nullptr, nullptr, nullptr, out, modes.data());
+    const int rc = rsd_long_pairs(c, (int)n_pairs, ptr[0].data(), len64[0].data(), ptr[1].data(), len64[1].data(), force_mode, scripts != nullptr,
+                                  mo.data(), pop.data(), poi.data(), poj.data(), no64.data(), out, modes.data());
     if (rc) return -rc;
+    for (size_t p = 0; p < n_rows; ++p) scripts->n_ops[p] = (int32_t)no64[p];
     if (mode_out) { int mm = 0; for (int x : modes) mm = std::max(mm, x); *mode_out = mm; }
     return 1;
+}
+
+// Length threshold of route_long for an entry point: 0 (never route) when the knob `off` is set, else the knob `min` or
+// the default.  By wall time the tape-pass distance kernels still win at 4-5 kb (tools/dbg_crossover.py).
+constexpr int64_t DIST_LONG_MIN = 6144, SCRIPT_LONG_MIN = 4096;
+static int64_t long_min(const char *off, const char *min, int64_t dflt) {
+    if (getenv(off)) return 0;
+    const char *e = getenv(min);
+    return e ? std::max<int64_t>(atoll(e), 1) : dflt;
 }
 
 extern "C" int rsd_distance_batch(rsd_ctx *c,
@@ -996,7 +1009,8 @@ extern "C" int rsd_distance_batch(rsd_ctx *c,
     RSD_OK_OR_RETURN(c->ensure_device());
     if (n_pairs == 0) return RSD_OK;
     const SideIn in[2] = {{a_words, a_start, a_len, a_nwords, nullptr}, {b_words, b_start, b_len, b_nwords, nullptr}};
-    if (const int r = distance_route_long(c, in, n_pairs, bits, force_mode, out, mode_out)) return r > 0 ? RSD_OK : -r;
+    const int64_t T = long_min("RSD_DIST_NO_LONG", "RSD_DIST_LONG_MIN", DIST_LONG_MIN);
+    if (const int r = route_long(c, "rsd_distance_batch", T, in, n_pairs, bits, force_mode, nullptr, out, mode_out)) return r > 0 ? RSD_OK : -r;
     return distance_host(c, in, n_pairs, max_m_hint, max_n_hint, bits, symmask, force_mode, out, mode_out);
 }
 
@@ -1015,7 +1029,8 @@ extern "C" int rsd_distance_batch_codes(rsd_ctx *c, const uint8_t *a_codes, cons
     if (n_pairs == 0) return RSD_OK;
     // (negative lengths are caught by the block sums of distance_host: no extra pass over the 8 bytes per pair)
     const SideIn in[2] = {{nullptr, nullptr, a_len, 0, a_codes}, {nullptr, nullptr, b_len, 0, b_codes}};
-    if (const int r = distance_route_long(c, in, n_pairs, bits, force_mode, out, mode_out)) return r > 0 ? RSD_OK : -r;
+    const int64_t T = long_min("RSD_DIST_NO_LONG", "RSD_DIST_LONG_MIN", DIST_LONG_MIN);
+    if (const int r = route_long(c, "rsd_distance_batch", T, in, n_pairs, bits, force_mode, nullptr, out, mode_out)) return r > 0 ? RSD_OK : -r;
     return distance_host(c, in, n_pairs, max_m_hint, max_n_hint, bits, symmask, force_mode, out, mode_out);
 }
 
@@ -1056,25 +1071,26 @@ extern "C" int rsd_ubench(rsd_ctx *c, int which, double *ops_per_s) {
     if (!c || !ops_per_s) return rsd_fail(RSD_EINVAL, "rsd_ubench: NULL argument");
     RSD_OK_OR_RETURN(c->ensure_device());
     cudaStream_t st = c->stream;
-    RSD_OK_OR_RETURN(c->ps().scratch.ensure(64));
+    DevBuf &scratch = c->slots[0].scratch;
+    RSD_OK_OR_RETURN(scratch.ensure(64));
     const int threads = 256, blocks = c->sm_count * 8, iters = 2000;
     const uint32_t y = 0x00010003u, z = 0x00070002u;
     float best = 1e30f;
     for (int rep = 0; rep < 4; ++rep) {
         RSD_CUDA(cudaEventRecord(c->ev0, st));
         switch (which) {
-            case 0: k_ubench_u32<0><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 1: k_ubench_u32<1><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 2: k_ubench_u32<2><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 3: k_ubench_u32<3><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 4: k_ubench_f64<<<blocks, threads, 0, st>>>(iters, 1.5, (double *)c->ps().scratch.p); break;
-            case 5: k_ubench_u32<5><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 6: k_ubench_u32<6><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 7: k_ubench_mix<<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 8: k_ubench_u32<8><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 9: k_ubench_u32<9><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 10: k_ubench_u32<10><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
-            case 11: k_ubench_u32<11><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)c->ps().scratch.p); break;
+            case 0: k_ubench_u32<0><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 1: k_ubench_u32<1><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 2: k_ubench_u32<2><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 3: k_ubench_u32<3><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 4: k_ubench_f64<<<blocks, threads, 0, st>>>(iters, 1.5, (double *)scratch.p); break;
+            case 5: k_ubench_u32<5><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 6: k_ubench_u32<6><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 7: k_ubench_mix<<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 8: k_ubench_u32<8><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 9: k_ubench_u32<9><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 10: k_ubench_u32<10><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
+            case 11: k_ubench_u32<11><<<blocks, threads, 0, st>>>(iters, y, z, (uint32_t *)scratch.p); break;
             default: return rsd_fail(RSD_EINVAL, "rsd_ubench: unknown kind %d", which);
         }
         RSD_CUDA(cudaEventRecord(c->ev1, st));
@@ -1218,13 +1234,13 @@ int rsd_ctx::script_pipeline(const int32_t *a_len, const int32_t *b_len, int64_t
 
     constexpr int THREADS = 128;
     const int wpb = THREADS / 32;
+    const auto fwd = f64 ? (bits == 2 ? k_script_fwd<true, 2, 16> : k_script_fwd<true, 4, 16>)
+                         : (bits == 2 ? k_script_fwd<false, 2, 32> : k_script_fwd<false, 4, 32>);
     int blocks = 0;
-    if (f64) { if (bits == 2) RSD_OK_OR_RETURN(persistent_grid(k_script_fwd<true, 2, 16>, THREADS, sm_count, blocks));
-               else RSD_OK_OR_RETURN(persistent_grid(k_script_fwd<true, 4, 16>, THREADS, sm_count, blocks)); }
-    else { if (bits == 2) RSD_OK_OR_RETURN(persistent_grid(k_script_fwd<false, 2, 32>, THREADS, sm_count, blocks));
-           else RSD_OK_OR_RETURN(persistent_grid(k_script_fwd<false, 4, 32>, THREADS, sm_count, blocks)); }
+    RSD_OK_OR_RETURN(persistent_grid(fwd, THREADS, sm_count, blocks));
     const int stride = (int)max_m;       // two boundary columns of max_m rows per warp (tape passes)
-    RSD_OK_OR_RETURN(ps().scratch.ensure((size_t)(f64 ? 12 : 4) * 2 * (size_t)stride * blocks * wpb + 64));
+    PlanSlot &sl = slots[0];
+    RSD_OK_OR_RETURN(sl.scratch.ensure((size_t)(f64 ? 12 : 4) * 2 * (size_t)stride * blocks * wpb + 64));
 
     const uint32_t *dA = (const uint32_t *)bufA.words.p, *dB = (const uint32_t *)bufB.words.p;
     const int64_t *sA = (const int64_t *)bufA.start.p, *sB = (const int64_t *)bufB.start.p;
@@ -1236,15 +1252,9 @@ int rsd_ctx::script_pipeline(const int32_t *a_len, const int32_t *b_len, int64_t
         SeqView A{dA, sA + p0, lA + p0}, B{dB, sB + p0, lB + p0};
         PlanView pv;
         // trivial pairs (m == 0 or n == 0) get their distance from the planner and an all-INS / all-DEL script from the traceback
-        RSD_OK_OR_RETURN(make_plan(lA + p0, lB + p0, np, C, 0, (double *)out_f64.p + p0, st, pv, max_m, max_n, 0));
+        RSD_OK_OR_RETURN(make_plan(sl, lA + p0, lB + p0, np, C, 0, (double *)out_f64.p + p0, st, pv, max_m, max_n, 0));
         ScriptView sv{(uint32_t *)dirs.p, (const int64_t *)misc.p + p0, (double *)out_f64.p + p0};
-        if (f64) {
-            if (bits == 2) k_script_fwd<true, 2, 16><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, sv, S, ps().scratch.p, stride, -1);
-            else k_script_fwd<true, 4, 16><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, sv, S, ps().scratch.p, stride, -1);
-        } else {
-            if (bits == 2) k_script_fwd<false, 2, 32><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, sv, S, ps().scratch.p, stride, -1);
-            else k_script_fwd<false, 4, 32><<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, sv, S, ps().scratch.p, stride, -1);
-        }
+        fwd<<<blocks, THREADS, 0, st>>>(pv, A, B, d_ic, d_fc, sv, S, sl.scratch.p, stride, -1);
         k_traceback<<<(unsigned)((np + 63) / 64), 64, 0, st>>>(lA + p0, lB + p0, np, (const uint32_t *)dirs.p,
                                                                (const int64_t *)misc.p + p0, C, (uint8_t *)s_tmp.p, max_ops,
                                                                (int32_t *)s_nops.p + p0);
@@ -1303,47 +1313,12 @@ static int script_common(rsd_ctx *c, const uint32_t *a_words, const int64_t *a_s
     if (max_ops < 1) return rsd_fail(RSD_EINVAL, "rsd_script: max_ops must be >= 1");
     RSD_OK_OR_RETURN(c->ensure_device());
     if (n_pairs == 0) { if (mode_out) *mode_out = 0; return RSD_OK; }
-    // A batch whose cells lie mostly in pairs of several thousand symbols goes to the panel-wavefront kernels
-    // (rsd_long_pairs): one warp per pair with tape passes, the design of k_script_fwd for 1-2 kb pairs, falls to
-    // 450 / 240 / 35 GCUPS at 5 / 10 / 20 kb, where the panel pipeline runs at 1.0-1.4 TCUPS with the same scripts
-    // (tools/dbg_mid_pairs.py).  Not for the round-trip-checking variant (ok != NULL), which patches on the device.
-    if (!ok && n_pairs <= 65536 && force_mode != RSD_MODE_I16X2 && !getenv("RSD_SCRIPT_NO_LONG")) {
-        int64_t T = 4096;
-        if (const char *e = getenv("RSD_SCRIPT_LONG_MIN")) T = std::max<int64_t>(atoll(e), 1);
-        double cells_all = 0, cells_long = 0; int64_t total = 0;
-        for (int64_t p = 0; p < n_pairs; ++p) {
-            if (a_len[p] < 0 || b_len[p] < 0) return rsd_fail(RSD_EINVAL, "rsd_script: negative length");
-            const double cells = (double)a_len[p] * (double)b_len[p];
-            cells_all += cells; total += (int64_t)a_len[p] + b_len[p];
-            if (std::max(a_len[p], b_len[p]) >= T) cells_long += cells;
-        }
-        if (cells_long > 0.5 * cells_all) {
-            const int per = 32 / bits;
-            std::vector<uint8_t> codes((size_t)total + 16);
-            std::vector<const uint8_t *> pa((size_t)n_pairs), pb((size_t)n_pairs);
-            std::vector<int64_t> lm((size_t)n_pairs), ln((size_t)n_pairs), mo((size_t)n_pairs), no64((size_t)n_pairs, 0);
-            std::vector<uint8_t *> pop((size_t)n_pairs); std::vector<int32_t *> poi((size_t)n_pairs), poj((size_t)n_pairs);
-            std::vector<int> modes((size_t)n_pairs, 0);
-            size_t at = 0;
-            for (int64_t p = 0; p < n_pairs; ++p) {
-                for (int side = 0; side < 2; ++side) {
-                    const uint32_t *w = side ? b_words : a_words; const int64_t st0 = side ? b_start[p] : a_start[p];
-                    const int32_t len = side ? b_len[p] : a_len[p]; const int64_t nw = side ? b_nwords : a_nwords;
-                    if (st0 < 0 || st0 + ((int64_t)len + per - 1) / per > nw) return rsd_fail(RSD_EINVAL, "rsd_script: pair %lld lies outside the word buffer", (long long)p);
-                    (side ? pb : pa)[(size_t)p] = codes.data() + at;
-                    unpack_symbols(w, st0, len, bits, codes.data() + at); at += (size_t)len;
-                }
-                lm[(size_t)p] = a_len[p]; ln[(size_t)p] = b_len[p]; mo[(size_t)p] = max_ops;
-                if ((int64_t)a_len[p] + b_len[p] > max_ops) return rsd_fail(RSD_EINVAL, "rsd_script: max_ops too small for pair %lld", (long long)p);
-                pop[(size_t)p] = op + (size_t)p * max_ops;
-                poi[(size_t)p] = oi ? oi + (size_t)p * max_ops : nullptr; poj[(size_t)p] = oj ? oj + (size_t)p * max_ops : nullptr;
-            }
-            RSD_OK_OR_RETURN(rsd_long_pairs(c, (int)n_pairs, pa.data(), lm.data(), pb.data(), ln.data(), force_mode == RSD_MODE_I16X2 ? 0 : force_mode, 1, mo.data(),
-                                            pop.data(), poi.data(), poj.data(), no64.data(), dist, modes.data()));
-            for (int64_t p = 0; p < n_pairs; ++p) n_ops[p] = (int32_t)no64[(size_t)p];
-            if (mode_out) { int mm = 0; for (int x : modes) mm = std::max(mm, x); *mode_out = mm; }
-            return RSD_OK;
-        }
+    // not for the round-trip-checking variant (ok != NULL), which patches on the device
+    if (!ok) {
+        const SideIn in[2] = {{a_words, a_start, a_len, a_nwords, nullptr}, {b_words, b_start, b_len, b_nwords, nullptr}};
+        const LongScripts scripts{max_ops, op, oi, oj, n_ops};
+        const int64_t T = long_min("RSD_SCRIPT_NO_LONG", "RSD_SCRIPT_LONG_MIN", SCRIPT_LONG_MIN);
+        if (const int r = route_long(c, "rsd_script", T, in, n_pairs, bits, force_mode, &scripts, dist, mode_out)) return r > 0 ? RSD_OK : -r;
     }
     RSD_OK_OR_RETURN(c->upload_seqs(c->bufA, a_words, a_start, a_len, n_pairs, a_nwords, c->stream));
     RSD_OK_OR_RETURN(c->upload_seqs(c->bufB, b_words, b_start, b_len, n_pairs, b_nwords, c->stream));
@@ -1624,10 +1599,12 @@ int rsd_ctx::fast_prefix(uint32_t q_symmask, int64_t max_qlen, int bits, int for
 #define RSD_RANGE_HITS0 ((int64_t)1 << 20)
 
 // queries already on the device; outputs to device buffers (top_idx/top_score [Q][k]) and optionally all scores, or,
-// with `ro`, a range search: every record within ro->max_dist of each query, appended to ro batch by batch
+// with `ro`, a range search: every record within ro->max_dist of each query, appended to ro batch by batch.  Timed from
+// ev0 to ev1; record_start = false keeps the ev0 of an earlier search (the first query group of a host call).
 int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len, int64_t n_queries,
                         int64_t max_qlen, int bits, uint32_t q_symmask, int k, int force_mode,
-                        int64_t *top_idx, double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st, RangeOut *ro) {
+                        int64_t *top_idx, double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st, RangeOut *ro,
+                        bool record_start) {
     if (!db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_search: no database loaded (rsd_db_load)");
     if (bits != db_bits) return rsd_fail(RSD_EINVAL, "rsd_db_search: query packing (%d bit) differs from the database (%d bit)", bits, db_bits);
     if (k < 0 || k > RSD_TOPK_MAX) return rsd_fail(RSD_EINVAL, "rsd_db_search: k must be in 0..%d (ask for all_scores instead)", RSD_TOPK_MAX);
@@ -1695,7 +1672,7 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
     tab.ins = mi_fast.ic.ins; tab.del = mi_fast.ic.del; tab.inv_scale = 1.0 / (double)(1 << mi_fast.ic.scale_log2);
     tab.compact_lut_lo = lut_lo; tab.compact_lut_hi = lut_hi;
     const uint32_t *dbw = (const uint32_t *)db.words.p; const int64_t *dbs = (const int64_t *)db.start.p; const int32_t *dbl = (const int32_t *)db.len.p;
-    if (timing && !hold_ev0) RSD_CUDA(cudaEventRecord(ev0, st));        // (the second query group of a host call keeps the first one's start)
+    if (timing && record_start) RSD_CUDA(cudaEventRecord(ev0, st));
     for (int64_t q0 = 0; q0 < n_queries; q0 += QB) {
         const int nq = (int)std::min<int64_t>(QB, n_queries - q0);
         if (k > 0) { k_topk_init<<<(nq + 63) / 64, 64, 0, st>>>(tk, nq); launches += 1; }
@@ -1767,11 +1744,8 @@ int rsd_ctx::search_dev(const uint32_t *q_words, const int64_t *q_start, const i
                 k_fill_pairs_view<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(q_start + q0, q_len + q0, qa, nqb, dbs, dbl, r0, nr, va_s, va_l, vb_s, vb_l);
                 launches += 1;
                 int mode_unused = 0;
-                const bool t_save = timing; timing = false;
-                int rc = distance_dev(q_words, va_s, va_l, dbw, vb_s, vb_l, np, max_qlen, db_maxlen, bits, symmask,
-                                      force_mode == RSD_MODE_I16X2 ? 0 : force_mode, (double *)db_dist.p, &mode_unused, st);
-                timing = t_save;
-                if (rc) return rc;
+                RSD_OK_OR_RETURN(distance_dev(q_words, va_s, va_l, dbw, vb_s, vb_l, np, max_qlen, db_maxlen, bits, symmask,
+                                              force_mode == RSD_MODE_I16X2 ? 0 : force_mode, (double *)db_dist.p, &mode_unused, st, nullptr, nullptr));
                 if (ro) k_range_filter_pairs<<<(unsigned)((np + 255) / 256), 256, 0, st>>>((const double *)db_dist.p, r0, nr, (const int64_t *)db_perm.p, db_base, qa, nqb, rh);
                 else k_score_filter_pairs<<<(unsigned)((np + 255) / 256), 256, 0, st>>>((const double *)db_dist.p, r0, nr, (const int64_t *)db_perm.p, db_base, qa, nqb, tk, alls, db_n);
                 launches += 1;
@@ -1850,7 +1824,7 @@ extern "C" int rsd_db_search_topk_dev(rsd_ctx *c, const uint32_t *q_words_dev, c
     RSD_OK_OR_RETURN(c->ensure_device());
     if (k < 1) return rsd_fail(RSD_EINVAL, "rsd_db_search_topk_dev: k must be >= 1");
     return c->search_dev(q_words_dev, q_start_dev, q_len_dev, n_queries, max_qlen, bits, q_symmask, k, force_mode,
-                         top_idx_dev, top_score_dev, nullptr, mode_out, (cudaStream_t)stream);
+                         top_idx_dev, top_score_dev, nullptr, mode_out, (cudaStream_t)stream, nullptr, true);
 }
 
 // order (empty: caller order) = the caller's query of every device row; rows [0, n_first) form the first group
@@ -1928,12 +1902,10 @@ static int search_groups(rsd_ctx *c, const QueryGroups &qg, int64_t n_queries, i
         const int64_t g0 = g == 0 ? 0 : qg.n_first, g1 = g == 0 ? qg.n_first : n_queries;
         if (g1 <= g0) continue;
         int mo = 0;
-        struct Hold { rsd_ctx *c; ~Hold() { c->hold_ev0 = false; } } hold{c};
-        c->hold_ev0 = g == 1 && qg.n_first > 0;
         RSD_OK_OR_RETURN(c->search_dev((const uint32_t *)c->bufQ.words.p, (const int64_t *)c->bufQ.start.p + g0, (const int32_t *)c->bufQ.len.p + g0,
                                        g1 - g0, max_qlen, bits, g == 0 ? qg.mask_first : qg.mask_rest, kk, force_mode,
                                        ro ? nullptr : (int64_t *)c->s_oi.p + g0 * kk, ro ? nullptr : (double *)c->s_oj.p + g0 * kk,
-                                       all_scores ? (double *)c->out_f64.p + (size_t)g0 * c->db_n : nullptr, &mo, c->stream, ro));
+                                       all_scores ? (double *)c->out_f64.p + (size_t)g0 * c->db_n : nullptr, &mo, c->stream, ro, g0 == 0));
         mode_all = std::max(mode_all, mo);
     }
     return RSD_OK;
@@ -2170,7 +2142,8 @@ static int long_pair_wide(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t
                         n_panels, per_sm * c->sm_count);
     const size_t dir_words = (size_t)((m + 15) / 16) * (size_t)n_pad;
     RSD_OK_OR_RETURN(c->dirs.ensure(dir_words * 4 + 64));
-    RSD_OK_OR_RETURN(c->ps().scratch.ensure((size_t)n_panels * (size_t)m * 12 + 256));
+    DevBuf &scratch = c->slots[0].scratch;
+    RSD_OK_OR_RETURN(scratch.ensure((size_t)n_panels * (size_t)m * 12 + 256));
     RSD_OK_OR_RETURN(c->mat_ab.ensure((size_t)m + n + 64));
     RSD_OK_OR_RETURN(c->out_f64.ensure(64));
     uint8_t *da = (uint8_t *)c->mat_ab.p, *db = da + ((m + 15) / 16) * 16;
@@ -2179,8 +2152,8 @@ static int long_pair_wide(rsd_ctx *c, const uint8_t *a, int64_t m, const uint8_t
     LongArgs la{};
     la.a = da; la.m = (int)m; la.b = db; la.n = (int)n; la.n_panels = n_panels; la.n_pad = (int)n_pad;
     la.dirs = (uint32_t *)c->dirs.p;
-    la.bound = c->ps().scratch.p;
-    la.bound_steps = (int *)((unsigned char *)c->ps().scratch.p + (size_t)n_panels * (size_t)m * 8);
+    la.bound = scratch.p;
+    la.bound_steps = (int *)((unsigned char *)scratch.p + (size_t)n_panels * (size_t)m * 8);
     la.dist = (double *)c->out_f64.p;
     la.S = S;
     RSD_CUDA(cudaMemsetAsync(la.bound, 0x80, (size_t)n_panels * (size_t)m * 8, st));      // sentinel = "not published yet"

@@ -87,11 +87,10 @@ struct rsd_ctx {
     int sm_count = 0;
     cudaStream_t stream = nullptr, stream2 = nullptr, copy_stream = nullptr, d2h_stream = nullptr;
     cudaEvent_t ev_sync = nullptr, ev_chunk[RSD_MAX_CHUNKS] = {}, ev_t0[RSD_MAX_CHUNKS] = {}, ev_t1[RSD_MAX_CHUNKS] = {}, ev_done[RSD_MAX_CHUNKS] = {};
-    cudaEvent_t cur_ev0 = nullptr, cur_ev1 = nullptr, ev_begin = nullptr, ev_len = nullptr, ev_plans = nullptr, ev_tab = nullptr;
+    cudaEvent_t ev_begin = nullptr, ev_len = nullptr, ev_plans = nullptr, ev_tab = nullptr;
     double last_ms_override = 0.0;
-    bool costs_preloaded = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    bool timing = false, timed = false, hold_ev0 = false;
+    bool timing = false, timed = false;
     int64_t launches = 0;
 
     bool have_costs = false;
@@ -106,8 +105,6 @@ struct rsd_ctx {
     void *h_stage = nullptr; size_t h_stage_cap = 0;
     DevBuf d_stage, raw_codes[2], sym_start[2];
     PlanSlot slots[RSD_MAX_CHUNKS];
-    int cur_slot = 0;
-    PlanSlot &ps() { return slots[cur_slot]; }
     DevBuf mat_vals, mat_mask, mat_ab;
     // script / patch
     int64_t dirs_budget_words = 0, dirs_budget_out_bytes = 0;     // chunk budget of the script path, measured once
@@ -140,19 +137,21 @@ struct rsd_ctx {
     int upload_costs(const ModeInfo &mi, cudaStream_t st);
     int upload_seqs(SeqBufs &sb, const uint32_t *words, const int64_t *start, const int32_t *len, int64_t n,
                     int64_t n_words, cudaStream_t st);
-    int make_plan(const int32_t *d_alen, const int32_t *d_blen, int64_t n_pairs, int C, int allow_twin, double *d_out,
+    int make_plan(PlanSlot &sl, const int32_t *d_alen, const int32_t *d_blen, int64_t n_pairs, int C, int allow_twin, double *d_out,
                   cudaStream_t st, PlanView &pv, int64_t max_m, int64_t max_n, int band);
-    int distance_plan(const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n, int bits,
-                      uint32_t symmask, int force_mode, double *d_out, int *mode_out, cudaStream_t st);
-    int distance_launch(const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len, const uint32_t *b_words,
-                        const int64_t *b_start, const int32_t *b_len, int64_t max_m, int bits, double *d_out, cudaStream_t st);
+    int distance_plan(PlanSlot &sl, const int32_t *a_len, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n, int bits,
+                      uint32_t symmask, int force_mode, bool load_costs, double *d_out, int *mode_out, cudaStream_t st);
+    int distance_launch(PlanSlot &sl, const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len, const uint32_t *b_words,
+                        const int64_t *b_start, const int32_t *b_len, int64_t max_m, int bits, double *d_out, cudaStream_t st,
+                        cudaEvent_t t0, cudaEvent_t t1);
     int distance_dev(const uint32_t *a_words, const int64_t *a_start, const int32_t *a_len, const uint32_t *b_words,
                      const int64_t *b_start, const int32_t *b_len, int64_t n_pairs, int64_t max_m, int64_t max_n,
-                     int bits, uint32_t symmask, int force_mode, double *d_out, int *mode_out, cudaStream_t st);
+                     int bits, uint32_t symmask, int force_mode, double *d_out, int *mode_out, cudaStream_t st,
+                     cudaEvent_t t0, cudaEvent_t t1);
     int fast_prefix(uint32_t q_symmask, int64_t max_qlen, int bits, int force_mode, ModeInfo &mi_fast, uint32_t lut[4], int64_t &n_fast) const;
     int search_dev(const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len, int64_t n_queries,
                    int64_t max_qlen, int bits, uint32_t q_symmask, int k, int force_mode, int64_t *top_idx,
-                   double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st, RangeOut *ro = nullptr);
+                   double *top_score, double *all_scores_dev, int *mode_out, cudaStream_t st, RangeOut *ro, bool record_start);
     int64_t range_cap() const { return (int64_t)(std::min(rng_keys.cap, rng_dist.cap) / 16); }     // hits the buffer holds
     int range_reserve(int64_t hits, int qb);
     int range_collect(int nq, int qb, RangeOut &ro, bool &rerun, cudaStream_t st);
