@@ -219,6 +219,14 @@ enum {
 };
 int rsd_db_similarity(rsd_ctx *ctx, const uint8_t *q_codes, int32_t q_len, int method, int k,
                       int64_t *top_idx, double *top_score, double *all_scores);
+/* rsd_db_similarity for a batch of queries: query q is q_codes[q_off[q] .. q_off[q+1]) (codes 0..14, q_off[0] == 0,
+ * non-decreasing, each length <= INT32_MAX).  top_idx / top_score [n_queries][k] (k in 0..RSD_TOPK_MAX; -1 / 0.0 past
+ * the rankable records, NaN never ranked); all_scores (may be NULL) [n_queries][db_n] in record order.
+ * Row q is bit for bit what rsd_db_similarity returns for query q alone.  The records are read once per query batch
+ * (up to 64 queries, fewer when device memory is short or RSD_SIM_QBATCH asks for fewer), not once per query.
+ * Arguments are checked on the host before any device work (RSD_EINVAL); n_queries == 0 writes nothing. */
+int rsd_db_similarity_batch(rsd_ctx *ctx, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                            int method, int k, int64_t *top_idx, double *top_score, double *all_scores);
 /* merge G shards' top-k lists (each n_queries*k, shard-major) with the same key — the reduction
  * run after the gather (host side, O(G*k) per query) */
 int rsd_topk_merge(const int64_t *idx, const double *score, int n_shards, int64_t n_queries, int k,
@@ -226,9 +234,9 @@ int rsd_topk_merge(const int64_t *idx, const double *score, int n_shards, int64_
 
 /* ---- database search over several GPUs of one box, ONE process -------------------------------------------
  * Replaces the process fan-out under IRMethods.create_search_threads / search_collection (IR:443-515) on the
- * wf_score path: the database is cut into contiguous shards balanced by symbols, one per device; the query batch
- * goes to every device; each device keeps a local top-k; the lists (Q * k * 16 bytes per device) are gathered
- * with ONE grouped ncclAllGather over NVLink and merged with the key (score desc, index asc) — identical to the
+ * wf_score path and for the similarity measures: the database is cut into contiguous shards balanced by symbols,
+ * one per device; the query batch goes to every device; each device keeps a local top-k; the lists (Q * k * 16
+ * bytes per device) are gathered with ONE grouped ncclAllGather over NVLink and merged with the key (score desc, index asc) — identical to the
  * stable descending sort over the whole collection because shards are index-contiguous.  NCCL is bound at run
  * time (dlopen), only when more than one distinct device is used.  devices == NULL / n_devices == 0: all visible
  * devices.  A device may be listed several times (shards emulated on one GPU; the gather is then plain copies). */
@@ -244,6 +252,10 @@ int rsd_multi_db_free(rsd_multi *m);
 int rsd_multi_db_search_topk(rsd_multi *m, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
                              int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, int k, int force_mode,
                              int64_t *top_idx, double *top_score, double *all_scores, int *mode_out);
+/* like rsd_db_similarity_batch, over the whole database: every device scores its shard, the local top-k lists go
+ * through the same gather and merge as rsd_multi_db_search_topk; all_scores (optional) is [n_queries][n_records] */
+int rsd_multi_db_similarity(rsd_multi *m, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                            int method, int k, int64_t *top_idx, double *top_score, double *all_scores);
 /* like rsd_db_search_range (which replaces the wf_score scan of search_collection, IR:466-477, followed
  * by a filter on the distance), over the whole database: each device searches its shard, and the hits of
  * a query are the shards' hits in shard order; cap / RSD_ERANGE apply to the total */

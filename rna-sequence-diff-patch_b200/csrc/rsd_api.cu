@@ -2107,6 +2107,145 @@ extern "C" int rsd_db_similarity(rsd_ctx *c, const uint8_t *q_codes, int32_t q_l
     return RSD_OK;
 }
 
+// the host-side checks of a similarity query batch (every entry point, before any device work)
+static int sim_batch_args(const char *fn, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries, int method, int k,
+                          const int64_t *top_idx, const double *top_score) {
+    if (method < 0 || method >= RSD_SIM_COUNT) return rsd_fail(RSD_EINVAL, "%s: unknown method %d", fn, method);
+    if (k < 0 || k > RSD_TOPK_MAX) return rsd_fail(RSD_EINVAL, "%s: k must be in 0..%d", fn, RSD_TOPK_MAX);
+    if (n_queries < 0 || (n_queries > 0 && !q_off)) return rsd_fail(RSD_EINVAL, "%s: bad query", fn);
+    if (n_queries == 0) return RSD_OK;
+    if (k > 0 && (!top_idx || !top_score)) return rsd_fail(RSD_EINVAL, "%s: NULL top-k output", fn);
+    if (q_off[0] != 0) return rsd_fail(RSD_EINVAL, "%s: q_off[0] must be 0", fn);
+    for (int64_t q = 0; q < n_queries; ++q) {
+        const int64_t len = q_off[q + 1] - q_off[q];
+        if (len < 0 || len > INT32_MAX) return rsd_fail(RSD_EINVAL, "%s: bad query offsets at query %lld", fn, (long long)q);
+    }
+    if (q_off[n_queries] > 0 && !q_codes) return rsd_fail(RSD_EINVAL, "%s: bad query", fn);
+    for (int64_t i = 0; i < q_off[n_queries]; ++i)
+        if (q_codes[i] >= 15) return rsd_fail(RSD_EINVAL, "%s: query code %u at %lld is not a symbol", fn, q_codes[i], (long long)i);
+    return RSD_OK;
+}
+
+// Queries q_codes[q_off[q] .. q_off[q+1]) (host) up to the context's sim_codes / sim_off.
+static int sim_upload_queries(rsd_ctx *c, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries) {
+    const int64_t total = q_off[n_queries];
+    RSD_OK_OR_RETURN(c->sim_codes.ensure((size_t)total + 16));
+    RSD_OK_OR_RETURN(c->sim_off.ensure(sizeof(int64_t) * (size_t)(n_queries + 1)));
+    if (total) RSD_CUDA(cudaMemcpyAsync(c->sim_codes.p, q_codes, (size_t)total, cudaMemcpyHostToDevice, c->stream));
+    RSD_CUDA(cudaMemcpyAsync(c->sim_off.p, q_off, sizeof(int64_t) * (size_t)(n_queries + 1), cudaMemcpyHostToDevice, c->stream));
+    return RSD_OK;
+}
+
+// The similarity of n_queries queries (on the device: sim_codes / sim_off) against the loaded shard, in query batches of
+// QB: each batch is one pass over the records into scores [QB][db_n], then the top-k of each query with the chunk
+// sequence of rsd_db_similarity (a 4096-record seed chunk, then chunks of min(db_n, 2^20)).  Outputs: top_idx_dev /
+// top_score_dev [n_queries][k] on the device (k > 0); all_scores (host, may be NULL): query q's db_n scores at
+// all_scores + q * all_stride + all_col.  Timed (rsd_set_timing) from the first kernel to the last copy.
+static int sim_batch_dev(rsd_ctx *c, int64_t n_queries, int method, int k, int64_t *top_idx_dev, double *top_score_dev,
+                         double *all_scores, int64_t all_stride, int64_t all_col) {
+    cudaStream_t st = c->stream;
+    const int64_t n = c->db_n;
+    const int64_t CH0 = 4096, cap = std::min<int64_t>(std::max<int64_t>(n, 1), (int64_t)1 << 20);
+    // QB: at most RSD_SIM_QB queries, and what half of the free device memory holds (the buffers this call reuses count
+    // as free); RSD_SIM_QBATCH lowers it
+    const size_t per_q = sizeof(double) * (size_t)std::max<int64_t>(n, 1) + sizeof(SimQuery) + 64
+                       + (k > 0 ? (size_t)cap * 16 + (size_t)k * 16 : 0);
+    size_t free_b = 0, total_b = 0;
+    RSD_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    const size_t room = free_b / 2 + c->sim_scores.cap + c->sim_aux.cap + c->sim_q.cap;
+    int64_t qb = std::min<int64_t>({n_queries, (int64_t)RSD_SIM_QB, (int64_t)(room / per_q)});
+    if (const char *e = getenv("RSD_SIM_QBATCH")) qb = std::min<int64_t>(qb, atoi(e));
+    qb = std::max<int64_t>(qb, 1);
+    RSD_OK_OR_RETURN(c->sim_q.ensure(sizeof(SimQuery) * (size_t)qb));
+    RSD_OK_OR_RETURN(c->sim_scores.ensure(sizeof(double) * (size_t)qb * (size_t)std::max<int64_t>(n, 1)));
+    RSD_OK_OR_RETURN(c->sim_work.ensure(sizeof(int) * (size_t)(n + 16)));
+    TopkState tk{};
+    if (k > 0) {
+        RSD_OK_OR_RETURN(c->sim_aux.ensure((size_t)qb * ((size_t)cap * 16 + (size_t)k * 16 + 24) + 256));
+        unsigned char *aux = (unsigned char *)c->sim_aux.p;
+        tk.k = k; tk.cap = cap;
+        tk.cand_s = (double *)aux; aux += (size_t)qb * cap * 8;
+        tk.cand_i = (int64_t *)aux; aux += (size_t)qb * cap * 8;
+        tk.best_s = (double *)aux; aux += (size_t)qb * k * 8;
+        tk.best_i = (int64_t *)aux; aux += (size_t)qb * k * 8;
+        tk.tau_s = (double *)aux; aux += (size_t)qb * 8;
+        tk.tau_i = (int64_t *)aux; aux += (size_t)qb * 8;
+        tk.cand_n = (int *)aux;
+    }
+    const uint32_t *dbw = (const uint32_t *)c->db.words.p; const int64_t *dbs = (const int64_t *)c->db.start.p; const int32_t *dbl = (const int32_t *)c->db.len.p;
+    const int64_t *perm = (const int64_t *)c->db_perm.p;
+    const uint8_t *codes = (const uint8_t *)c->sim_codes.p;
+    const int64_t *off = (const int64_t *)c->sim_off.p;
+    SimQuery *simq = (SimQuery *)c->sim_q.p;
+    double *scores = (double *)c->sim_scores.p;
+    int *wl_n = (int *)c->sim_work.p, *wl = wl_n + 4;
+    if (c->timing) RSD_CUDA(cudaEventRecord(c->ev0, st));
+    for (int64_t q0 = 0; q0 < n_queries; q0 += qb) {
+        const int nq = (int)std::min<int64_t>(qb, n_queries - q0);
+        k_sim_query_batch<<<nq, 32, 0, st>>>(codes, off + q0, simq);
+        c->launches += 1;
+        if (n > 0) {
+            if (method < RSD_SIM_COSINE) {
+                k_sim_small_batch<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dbw, dbs, dbl, n, c->db_bits, perm, c->db_base, simq, nq, method, scores, n);
+                c->launches += 1;
+            } else {
+                // plain A/G/C/U records: one thread each; the rest (ambiguity codes, > 60000 symbols) through the worklist
+                RSD_CUDA(cudaMemsetAsync(wl_n, 0, sizeof(int), st));
+                k_sim_tf_thread_batch<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(dbw, dbs, dbl, n, c->db_bits, perm, c->db_base, simq, nq, method,
+                                                                               scores, n, wl, wl_n);
+                const unsigned grid = (unsigned)std::min<int64_t>((n + 3) / 4, (int64_t)c->sm_count * 16);
+                k_sim_tf_batch<<<grid, 128, 0, st>>>(dbw, dbs, dbl, c->db_bits, perm, c->db_base, simq, nq, method, scores, n, wl, wl_n);
+                c->launches += 2;
+            }
+        }
+        if (k > 0) {
+            k_topk_init<<<(nq + 63) / 64, 64, 0, st>>>(tk, nq);
+            c->launches += 1;
+            for (int64_t r0 = 0; r0 < n;) {
+                const int64_t nr = std::min<int64_t>(r0 == 0 ? std::min(CH0, cap) : cap, n - r0);
+                k_sim_filter_batch<<<dim3((unsigned)((nr + 255) / 256), (unsigned)nq), 256, 0, st>>>(scores, n, r0, nr, c->db_base, tk);
+                k_topk_fold<<<nq, 256, 0, st>>>(tk);
+                c->launches += 2;
+                r0 += nr;
+            }
+            RSD_CUDA(cudaMemcpyAsync(top_idx_dev + q0 * k, tk.best_i, sizeof(int64_t) * (size_t)nq * k, cudaMemcpyDeviceToDevice, st));
+            RSD_CUDA(cudaMemcpyAsync(top_score_dev + q0 * k, tk.best_s, sizeof(double) * (size_t)nq * k, cudaMemcpyDeviceToDevice, st));
+        }
+        RSD_CUDA(cudaGetLastError());
+        if (all_scores && n > 0) {
+            // a [nq][n] block: contiguous in the caller's [Q][n] rows, or placed at column all_col of wider rows (a shard)
+            if (all_stride == n) RSD_CUDA(cudaMemcpyAsync(all_scores + q0 * n + all_col, scores, sizeof(double) * (size_t)nq * n, cudaMemcpyDeviceToHost, st));
+            else RSD_CUDA(cudaMemcpy2DAsync(all_scores + q0 * all_stride + all_col, sizeof(double) * (size_t)all_stride, scores, sizeof(double) * (size_t)n,
+                                            sizeof(double) * (size_t)n, (size_t)nq, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    if (c->timing) { RSD_CUDA(cudaEventRecord(c->ev1, st)); c->timed = true; }
+    return RSD_OK;
+}
+
+extern "C" int rsd_db_similarity_batch(rsd_ctx *c, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                                       int method, int k, int64_t *top_idx, double *top_score, double *all_scores) {
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    RSD_OK_OR_RETURN(sim_batch_args("rsd_db_similarity_batch", q_codes, q_off, n_queries, method, k, top_idx, top_score));
+    RSD_OK_OR_RETURN(c->ensure_device());
+    if (n_queries == 0) return RSD_OK;
+    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_similarity_batch: no database loaded (rsd_db_load)");
+    cudaStream_t st = c->stream;
+    c->timed = false; c->last_ms_override = 0.0;
+    const size_t cells = (size_t)n_queries * (size_t)std::max(k, 1);
+    RSD_OK_OR_RETURN(c->sim_top.ensure(sizeof(int64_t) * 2 * cells));
+    int64_t *ti = (int64_t *)c->sim_top.p; double *ts = (double *)(ti + cells);
+    RSD_OK_OR_RETURN(sim_upload_queries(c, q_codes, q_off, n_queries));
+    RSD_OK_OR_RETURN(sim_batch_dev(c, n_queries, method, k, ti, ts, all_scores, c->db_n, 0));
+    if (k > 0) {
+        RSD_CUDA(cudaMemcpyAsync(top_idx, ti, sizeof(int64_t) * (size_t)n_queries * k, cudaMemcpyDeviceToHost, st));
+        RSD_CUDA(cudaMemcpyAsync(top_score, ts, sizeof(double) * (size_t)n_queries * k, cudaMemcpyDeviceToHost, st));
+    }
+    RSD_CUDA(cudaGetLastError());
+    RSD_CUDA(cudaStreamSynchronize(st));
+    return RSD_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // long pair (BASELINE config 4)
 // ------------------------------------------------------------------------------------------------

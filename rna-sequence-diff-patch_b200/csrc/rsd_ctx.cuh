@@ -131,6 +131,7 @@ struct rsd_ctx {
     // 64-bit hit counter + per-query offsets, the sort's scratch
     DevBuf rng_keys, rng_dist, rng_n, rng_tmp;
     DevBuf sim_q, sim_scores, sim_aux, sim_codes, sim_work;
+    DevBuf sim_off, sim_top;               // rsd_db_similarity_batch: query offsets, [2][Q][k] top-k lists
 
     int ensure_device();
     int classify(uint32_t symmask, int64_t max_m, int64_t max_n, int bits, int force_mode, ModeInfo &mi) const;
@@ -163,7 +164,7 @@ struct rsd_ctx {
         for (PlanSlot &s : slots) s.release();
         DevBuf *all[] = {&out_f64, &mat_vals, &mat_mask, &mat_ab,
                          &long_pool, &long_jobs, &dirs, &s_op, &s_oi, &s_oj, &s_nops, &s_ok, &s_tmp, &p_out, &p_len, &p_err, &misc,
-                         &db_dist, &db_topi, &db_tops, &db_aux, &db_perm, &rng_keys, &rng_dist, &rng_n, &rng_tmp, &sim_q, &sim_scores, &sim_aux, &sim_codes, &sim_work};
+                         &db_dist, &db_topi, &db_tops, &db_aux, &db_perm, &rng_keys, &rng_dist, &rng_n, &rng_tmp, &sim_q, &sim_scores, &sim_aux, &sim_codes, &sim_work, &sim_off, &sim_top};
         for (DevBuf *b : all) b->release();
         d_stage.release(); for (int s = 0; s < 2; ++s) { raw_codes[s].release(); sym_start[s].release(); }
         if (h_stage) { cudaFreeHost(h_stage); h_stage = nullptr; h_stage_cap = 0; }

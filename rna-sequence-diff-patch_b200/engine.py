@@ -40,6 +40,39 @@ def _db_query(Q: PackedSeqs, db_bits: int) -> PackedSeqs:
     return Q
 
 
+def _sim_method(method) -> int:
+    if isinstance(method, str):
+        if method not in Engine.SIM_METHODS:
+            raise _lib.RsdError(_lib.RSD_EINVAL, f"unknown similarity method {method!r}")
+        return Engine.SIM_METHODS.index(method)
+    return int(method)
+
+
+def _sim_queries(queries):
+    """A similarity query batch -> (codes uint8, offsets int64[q+1]): a (codes, offsets) tuple as pack takes it, or a
+    list of code arrays (or of strings, encoded)."""
+    if isinstance(queries, tuple):
+        codes, off = queries
+        return np.ascontiguousarray(codes, np.uint8), np.ascontiguousarray(off, np.int64)
+    parts = [encode(x) if isinstance(x, str) else np.asarray(x, np.uint8).reshape(-1) for x in queries]
+    off = np.zeros(len(parts) + 1, np.int64)
+    np.cumsum([p.shape[0] for p in parts], out=off[1:])
+    codes = np.concatenate(parts) if parts else np.zeros(0, np.uint8)
+    return np.ascontiguousarray(codes, np.uint8), off
+
+
+def _similarity_batch(fn, h, db_n: int, queries, method, k: int, want_scores: bool):
+    """Calls rsd_db_similarity_batch / rsd_multi_db_similarity -> (all_scores [q, n] | None, top_idx [q, k], top_score [q, k])."""
+    codes, off = _sim_queries(queries)
+    nq = off.shape[0] - 1
+    cc = codes if codes.shape[0] else np.zeros(1, np.uint8)
+    alls = np.zeros((nq, db_n), np.float64) if want_scores else None
+    idx = np.full((nq, max(k, 1)), -1, np.int64); sc = np.zeros((nq, max(k, 1)), np.float64)
+    check(fn(h, ptr(cc, _u8), ptr(off, _i64), nq, _sim_method(method), int(k), ptr(idx, _i64), ptr(sc, _f64),
+             ptr(alls, _f64) if want_scores and db_n and nq else None))
+    return alls, idx[:, :k], sc[:, :k]
+
+
 def _search_range(fn, h, Q: PackedSeqs, max_dist: float, force_mode: int, guess: int):
     """Calls a range entry point (rsd_db_search_range / rsd_multi_db_search_range) with room for `guess` hits; when the
     hits do not fit (RSD_ERANGE, hit_off complete), once more with the exact total."""
@@ -254,7 +287,7 @@ class Engine:
     def db_similarity(self, query_codes: np.ndarray, method, k: int = 0, want_scores: bool = True):
         """IR:443-477 for the measures of IR:49-389 against the loaded database.
         -> (all_scores f64[n_db] | None, top_idx int64[k], top_score f64[k])."""
-        mid = self.SIM_METHODS.index(method) if isinstance(method, str) else int(method)
+        mid = _sim_method(method)
         q = np.ascontiguousarray(query_codes, np.uint8)
         qq = q if q.shape[0] else np.zeros(1, np.uint8)
         alls = np.zeros(self._db_n, np.float64) if want_scores else None
@@ -262,6 +295,12 @@ class Engine:
         check(self._lib.rsd_db_similarity(self._ctx, ptr(qq, _u8), int(q.shape[0]), mid, int(k), ptr(idx, _i64), ptr(sc, _f64),
                                           ptr(alls, _f64) if want_scores and self._db_n else None))
         return alls, idx[:k], sc[:k]
+
+    def db_similarity_batch(self, queries, method, k: int = 0, want_scores: bool = True):
+        """db_similarity for a batch of queries in one pass over the database per query batch: `queries` is a list of
+        code arrays or a (codes, offsets) tuple, as pack takes it.  Row q equals db_similarity(queries[q], ...) bit for bit.
+        -> (all_scores f64[q, n_db] | None, top_idx int64[q, k], top_score f64[q, k])."""
+        return _similarity_batch(self._lib.rsd_db_similarity_batch, self._ctx, getattr(self, "_db_n", 0), queries, method, k, want_scores)
 
     def topk_merge(self, idx: np.ndarray, score: np.ndarray):
         return topk_merge(idx, score)
@@ -328,7 +367,8 @@ class Engine:
 class MultiEngine:
     """Database search over several GPUs from one process (include/rsd.h, rsd_multi_*): contiguous shards, the
     query batch on every device, local top-k, one NCCL all-gather of the lists, merge.  Same search interface as
-    Engine (set_costs / db_load / db_search_topk / db_free), so ir.score_collection runs on either."""
+    Engine (set_costs / db_load / db_search_topk / db_search_range / db_similarity[_batch] / db_free), so
+    ir.score_collection and ir.similarity_collection run on either."""
 
     def __init__(self, devices=None):
         self._lib = _lib.load_library()
@@ -395,6 +435,15 @@ class MultiEngine:
                                             getattr(self, "_range_total", Q.n * 256))
         self._range_total = int(res[0][-1])
         return res
+
+    def db_similarity(self, query_codes: np.ndarray, method, k: int = 0, want_scores: bool = True):
+        """Engine.db_similarity over the whole sharded database."""
+        alls, idx, sc = self.db_similarity_batch([np.asarray(query_codes, np.uint8)], method, k, want_scores)
+        return (alls[0] if want_scores else None), idx[0], sc[0]
+
+    def db_similarity_batch(self, queries, method, k: int = 0, want_scores: bool = True):
+        """Engine.db_similarity_batch over the whole sharded database."""
+        return _similarity_batch(self._lib.rsd_multi_db_similarity, self._h, self._db_n, queries, method, k, want_scores)
 
     def launch_count(self) -> int:
         return int(self._lib.rsd_multi_launch_count(self._h))

@@ -8,13 +8,14 @@ search_collection — set / multiset / TF-vector measures, IR:49-389 — as one 
 (similarity_collection)."""
 from __future__ import annotations
 
+import weakref
 from operator import itemgetter
 
 import numpy as np
 
 from . import sed
 from .encoding import pack
-from .engine import get_engine, get_search_engine
+from .engine import get_search_engine
 
 
 def wf_score(seq1: str, seq2: str, costs: dict) -> float:
@@ -40,32 +41,38 @@ def _validate_collection(query: str, sequences, costs: dict):
 
 
 class _Resident:
-    """The collection last loaded by score_collection / similarity_collection: a session that searches the same
-    collection again (gui.py:532-600: every search re-reads collection.find({})) pays rsd_db_load once."""
-    engine = None
-    sequences = None
-    gen = -1
+    """The collection each engine holds, as loaded by score_collection / range_collection / similarity_collection: a
+    session that searches the same collection again (gui.py:532-600: every search re-reads collection.find({})) pays
+    rsd_db_load once per engine.  The copy is keyed on its content (the documents after the case rule of the measure
+    that loaded them), so wf_score (upper case) and the other measures (as stored) share it when the collection has no
+    lower-case letters."""
+    held = weakref.WeakKeyDictionary()      # engine -> (load generation, documents as given, upper, documents as loaded)
 
     @classmethod
     def load(cls, eng, sequences, upper: bool):
-        if (cls.engine is eng and cls.gen == getattr(eng, "_db_gen", 0) and cls.sequences is not None
-                and cls.sequences[0] == upper and cls.sequences[1] == sequences):
-            return
-        if cls.engine is not None and cls.engine is not eng:
-            cls.drop()                                   # the collection moves to another engine: free the old copy
-        cls.engine, cls.sequences = None, None
-        eng.db_load(pack([s.upper() for s in sequences] if upper else sequences, bits=4))
-        cls.engine, cls.sequences, cls.gen = eng, (upper, sequences), eng._db_gen
+        h = cls.held.get(eng)
+        if h is not None and h[0] == getattr(eng, "_db_gen", 0):
+            if (h[2] == upper and h[1] == sequences) or h[3] == (_upper(sequences) if upper else sequences):
+                return
+        content = _upper(sequences) if upper else sequences
+        cls.held.pop(eng, None)
+        eng.db_load(pack(content, bits=4))
+        cls.held[eng] = (eng._db_gen, sequences, upper, content)
 
     @classmethod
     def drop(cls):
-        if cls.engine is not None and cls.gen == getattr(cls.engine, "_db_gen", 0):
-            cls.engine.db_free()
-        cls.engine, cls.sequences = None, None
+        for eng, (gen, *_) in list(cls.held.items()):
+            if gen == getattr(eng, "_db_gen", 0):
+                eng.db_free()
+        cls.held.clear()
+
+
+def _upper(sequences):
+    return [s.upper() for s in sequences]
 
 
 def release_collection():
-    """Free the device copy of the collection kept by the last search (optional; the next search reloads)."""
+    """Free the device copies of the collection kept by the searches (optional; the next search reloads)."""
     _Resident.drop()
 
 
@@ -108,14 +115,15 @@ def similarity_collection(query: str, sequences, method: str, engine=None):
     """[(sequence, method(query, sequence))] in collection order for one of SIM_METHODS — what
     search_collection(query, 'tf', collection, <method>) returns (IR:449-477), one GPU pass.  The documents'
     stored 'tf' vectors are rebuilt from the sequences on the device (they are convert_to_tf_vector(sequence),
-    fa_import.py:49).  Unknown symbols raise KeyError (the reference: KeyError IR:106 / ValueError IR:155)."""
+    fa_import.py:49).  Unknown symbols raise KeyError (the reference: KeyError IR:106 / ValueError IR:155).  Sharded over
+    every visible GPU like score_collection."""
     if method not in SIM_METHODS:
         raise ValueError(f"unknown similarity method {method!r}")
     sequences = list(sequences)
     if not sequences:
         return []
     from .encoding import encode
-    eng = engine or get_engine()
+    eng = engine or get_search_engine()
     qc = encode(query)
     _Resident.load(eng, sequences, upper=False)
     scores, _, _ = eng.db_similarity(qc, method)

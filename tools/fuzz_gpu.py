@@ -86,7 +86,7 @@ def main():
         alpha = [SYM[:4], SYM[:4], SYM[:4] + "N", SYM, SYM[:2], "ACGUYR"][int(rng.integers(0, 6))]
         ckind = ["default", "user", "dyadic", "int", "decimal"][int(rng.integers(0, 5))]
         lkind = ["tiny", "short", "c2", "kb", "skew", "wide"][int(rng.integers(0, 6))]
-        what = ["dist", "dist", "script", "search", "long", "sim", "range"][int(rng.integers(0, 7))]
+        what = ["dist", "dist", "script", "search", "long", "sim", "range", "simb"][int(rng.integers(0, 8))]
         costs = random_costs(rng, ckind)
         eng.set_costs(costs)
         force = int(rng.choice([0, 0, 0, 2, 3]))
@@ -153,6 +153,43 @@ def main():
                 finally:
                     eng.db_free()
                 desc = f"sim n={n} bits={bits} qlen={len(q)} mode=0"
+            elif what == "simb":
+                # a similarity query batch (rsd_db_similarity_batch) with a random query count and RSD_SIM_QBATCH, top-k too
+                n = int(rng.choice([1, 40, 400, 5000]))
+                lens = rng.integers(0, int(rng.choice([8, 40, 300])), size=n)
+                cd, od = make(rng, lens, alpha)
+                docs = [O.decode(cd[od[k]:od[k + 1]]) for k in range(n)]
+                nq = int(rng.integers(1, 80))
+                cq, oq = make(rng, rng.integers(0, 40, size=nq), alpha)
+                queries = [O.decode(cq[oq[q]:oq[q + 1]]) for q in range(nq)]
+                method = str(rng.choice(IO.METHODS))
+                k = int(rng.choice([0, 1, 7, 128]))
+                bits = 2 if (set(alpha) <= set("AGCU") and rng.random() < 0.5) else 4
+                knobs = {"RSD_SIM_QBATCH": str(int(rng.integers(1, 20)))} if rng.random() < 0.7 else {}
+                eng.db_load(R.pack((cd, od), bits=bits))
+                os.environ.update(knobs)
+                try:
+                    alls, idx, sc = eng.db_similarity_batch((cq, oq), method, k)
+                finally:
+                    for kname in knobs: del os.environ[kname]
+                    eng.db_free()
+                dreps = [IO.represent(d2, method) for d2 in docs]
+                ok = alls.shape == (nq, n)
+                for q in range(nq):
+                    qa = IO.represent(queries[q], method)
+                    want = np.zeros(n)
+                    for k2, d2 in enumerate(dreps):
+                        try:
+                            want[k2] = IO.score(method, qa, d2)
+                        except ZeroDivisionError:              # set measures of two empty sequences: the device returns NaN
+                            want[k2] = np.nan
+                    ok = ok and bool(np.array_equal(np.isnan(alls[q]), np.isnan(want))
+                                     and np.array_equal(alls[q][~np.isnan(want)].view(np.uint64), want[~np.isnan(want)].view(np.uint64)))
+                    valid = np.flatnonzero(~np.isnan(want))
+                    top = valid[np.argsort(-want[valid], kind="stable")][:k]
+                    wi = np.full(k, -1, np.int64); ws = np.zeros(k); wi[:top.shape[0]] = top; ws[:top.shape[0]] = want[top]
+                    ok = ok and np.array_equal(idx[q], wi) and np.array_equal(sc[q], ws)
+                desc = f"simb n={n} q={nq} method={method} k={k} bits={bits} knobs={knobs}"
             elif what == "long":
                 m, n2 = int(rng.integers(1, 5000)), int(rng.integers(1, 5000))
                 al = np.array([SYM.index(ch) for ch in alpha], np.uint8)
