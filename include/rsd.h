@@ -227,6 +227,23 @@ int rsd_db_similarity(rsd_ctx *ctx, const uint8_t *q_codes, int32_t q_len, int m
  * Arguments are checked on the host before any device work (RSD_EINVAL); n_queries == 0 writes nothing. */
 int rsd_db_similarity_batch(rsd_ctx *ctx, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
                             int method, int k, int64_t *top_idx, double *top_score, double *all_scores);
+/* The idf and tf-idf vector types of search_collection (IRMethods.py:458-465; the vectors of IRMethods.py:189-225).
+ * The idf vector of a sequence is idf[p] = log10(N / df[p]) (0 where df[p] == 0) at each distinct literal bigram p of
+ * it, 0 elsewhere; tf-idf is the matrix product tf . idf.  df[p] is the sum over the collection, in collection order,
+ * of compare_pair_to_seq(p, document) (IRMethods.py:225-252), N the number of records.  The table is built on the
+ * device on first use after rsd_db_load and kept until the next rsd_db_load / rsd_db_free; idf is computed on the host
+ * from df exactly as Python's math.log(N / df, 10).  A database loaded with global_index_base != 0 is one shard of a
+ * collection whose other records it does not know: these calls refuse it (RSD_EINVAL); use rsd_multi for shards. */
+enum { RSD_VEC_IDF = 1, RSD_VEC_TFIDF = 2 };
+/* df[225], idf[225] (either may be NULL) of the loaded database, row-major [15][15] in table order; builds the table
+ * when needed */
+int rsd_db_idf_table(rsd_ctx *ctx, double *df, double *idf);
+/* rsd_db_similarity_batch over the idf (RSD_VEC_IDF) or tf-idf (RSD_VEC_TFIDF) vectors of the query and the records;
+ * method in RSD_SIM_COSINE..RSD_SIM_DICE (the set and multiset measures have no vector type: RSD_EINVAL).  Same
+ * outputs, batching and argument checks as rsd_db_similarity_batch; the scores equal the reference's bit for bit. */
+int rsd_db_vector_similarity_batch(rsd_ctx *ctx, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                                   int vector_type, int method, int k, int64_t *top_idx, double *top_score,
+                                   double *all_scores);
 /* merge G shards' top-k lists (each n_queries*k, shard-major) with the same key — the reduction
  * run after the gather (host side, O(G*k) per query) */
 int rsd_topk_merge(const int64_t *idx, const double *score, int n_shards, int64_t n_queries, int k,
@@ -256,6 +273,13 @@ int rsd_multi_db_search_topk(rsd_multi *m, const uint32_t *q_words, const int64_
  * through the same gather and merge as rsd_multi_db_search_topk; all_scores (optional) is [n_queries][n_records] */
 int rsd_multi_db_similarity(rsd_multi *m, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
                             int method, int k, int64_t *top_idx, double *top_score, double *all_scores);
+/* rsd_db_idf_table over the whole database: the df sums run through the shards in order (device 0's partial sums
+ * continue on device 1, ...), and every device gets the one idf table */
+int rsd_multi_db_idf_table(rsd_multi *m, double *df, double *idf);
+/* rsd_db_vector_similarity_batch over the whole database, scored and gathered like rsd_multi_db_similarity */
+int rsd_multi_db_vector_similarity(rsd_multi *m, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                                   int vector_type, int method, int k, int64_t *top_idx, double *top_score,
+                                   double *all_scores);
 /* like rsd_db_search_range (which replaces the wf_score scan of search_collection, IR:466-477, followed
  * by a filter on the distance), over the whole database: each device searches its shard, and the hits of
  * a query are the shards' hits in shard order; cap / RSD_ERANGE apply to the total */

@@ -63,6 +63,8 @@ SIGNATURES = {
     "rsd_db_search_range": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, C.c_double, ci, i64, i64p, i64p, f64p, intp]),
     "rsd_db_similarity": (ci, [vp, u8p, C.c_int32, ci, ci, i64p, f64p, f64p]),
     "rsd_db_similarity_batch": (ci, [vp, u8p, i64p, i64, ci, ci, i64p, f64p, f64p]),
+    "rsd_db_idf_table": (ci, [vp, f64p, f64p]),
+    "rsd_db_vector_similarity_batch": (ci, [vp, u8p, i64p, i64, ci, ci, ci, i64p, f64p, f64p]),
     "rsd_topk_merge": (ci, [i64p, f64p, ci, i64, ci, i64p, f64p]),
     "rsd_multi_create": (ci, [intp, ci, C.POINTER(vp)]),
     "rsd_multi_destroy": (ci, [vp]),
@@ -72,6 +74,8 @@ SIGNATURES = {
     "rsd_multi_db_free": (ci, [vp]),
     "rsd_multi_db_search_topk": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, ci, ci, i64p, f64p, f64p, intp]),
     "rsd_multi_db_similarity": (ci, [vp, u8p, i64p, i64, ci, ci, i64p, f64p, f64p]),
+    "rsd_multi_db_idf_table": (ci, [vp, f64p, f64p]),
+    "rsd_multi_db_vector_similarity": (ci, [vp, u8p, i64p, i64, ci, ci, ci, i64p, f64p, f64p]),
     "rsd_multi_db_search_range": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, C.c_double, ci, i64, i64p, i64p, f64p, intp]),
     "rsd_multi_launch_count": (i64, [vp]),
     "rsd_long_pair": (ci, [vp, u8p, i64, u8p, i64, ci, ci, i64, u8p, i32p, i32p, i64p, f64p, intp]),

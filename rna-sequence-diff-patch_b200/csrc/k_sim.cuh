@@ -22,6 +22,15 @@
 //                            query TF vectors staged in shared memory RSD_SIM_QT at a time
 //   k_sim_tf_batch           one warp per worklist record: TF matrix in shared memory once, then every query
 //   k_sim_filter_batch       the top-k candidates of one score range, query = blockIdx.y
+//
+// idf and tf-idf vectors (search_collection with vector_type 'idf' / 'tf-idf', IR:189-225 and IR:458-465): the batch
+// kernels above take the vector type VT as a template argument; the query and record matrices are then the idf vector
+// (idf[p] at every distinct literal bigram p of the sequence) or the tf-idf product tf . idf, and everything after
+// that -- centring, norms, the measures, the top-k -- is the 'tf' code unchanged.  idf[p] = log10(N / df[p]) comes
+// from the collection's document-frequency table, built once per loaded database:
+//   k_idf_inv    collection index -> stored record (inverse of db_perm)
+//   k_idf_pres   literal-bigram presence sets of a chunk of records, in collection order
+//   k_idf_chain  the 225 df sums over that chunk, each one serial fp64 chain in collection order
 #pragma once
 #include "../../include/rsd.h"
 #include "rsd_common.cuh"
@@ -86,10 +95,50 @@ __device__ __forceinline__ void tf_build(double *v, int len, G get) {
     }
 }
 
-// the representations of one query (one warp; v = 225 doubles of shared memory)
-__device__ __forceinline__ void sim_query_build(double *v, const uint8_t *__restrict__ q, int len, SimQuery *out) {
+#define RSD_VEC_TF 0              // the 'tf' vectors; RSD_VEC_IDF / RSD_VEC_TFIDF are declared in include/rsd.h
+
+// One warp turns the TF matrix v of a sequence (tf_build) into its idf (VT == RSD_VEC_IDF) or tf-idf vector
+// (RSD_VEC_TFIDF).  IR:189-216: the idf vector is idf[p] at every distinct literal bigram p of the sequence and 0
+// elsewhere.  IR:219-223: tf-idf = np.dot(tf, idf), which numpy's BLAS evaluates per element as a fused multiply-add
+// chain over k = 0..14 ascending from +0.0.  w = 225 doubles and pres = 8 words of shared memory for this warp.
+template <int VT, typename G>
+__device__ __forceinline__ void vec_from_tf(double *v, double *w, uint32_t *pres, int len, G get, const double *__restrict__ idf) {
+    const int lane = threadIdx.x & 31;
+    if (lane < 8) pres[lane] = 0u;
+    __syncwarp();
+    for (int i = lane; i + 1 < len; i += 32) {
+        const int e = get(i) * 15 + get(i + 1);
+        atomicOr(&pres[e >> 5], 1u << (e & 31));
+    }
+    __syncwarp();
+    double *iv = VT == RSD_VEC_IDF ? v : w;
+    for (int e = lane; e < RSD_TF; e += 32) iv[e] = (pres[e >> 5] >> (e & 31) & 1u) ? idf[e] : 0.0;
+    __syncwarp();
+    if constexpr (VT == RSD_VEC_TFIDF) {
+        double o[8];
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+            const int e = lane + 32 * t, i = e / 15, j = e % 15;
+            double acc = 0.0;
+            if (e < RSD_TF)
+                for (int k = 0; k < 15; ++k) acc = __fma_rn(v[i * 15 + k], w[k * 15 + j], acc);
+            o[t] = acc;
+        }
+        __syncwarp();
+#pragma unroll
+        for (int t = 0; t < 8; ++t) if (lane + 32 * t < RSD_TF) v[lane + 32 * t] = o[t];
+        __syncwarp();
+    }
+}
+
+// the representations of one query (one warp; v = 225 doubles of shared memory).  VT != RSD_VEC_TF: tf / tfc / tf_sq /
+// tfc_sq hold the query's idf or tf-idf vector instead of its TF matrix (vec_from_tf; w, pres, idf as there).
+template <int VT = RSD_VEC_TF>
+__device__ __forceinline__ void sim_query_build(double *v, const uint8_t *__restrict__ q, int len, SimQuery *out,
+                                                double *w = nullptr, uint32_t *pres = nullptr, const double *__restrict__ idf = nullptr) {
     const int lane = threadIdx.x;
     tf_build(v, len, [&](int i) { return (int)q[i]; });
+    if constexpr (VT != RSD_VEC_TF) vec_from_tf<VT>(v, w, pres, len, [&](int i) { return (int)q[i]; }, idf);
     const double total = np_sum225([&](int e) { return v[e]; });
     const double avg = __ddiv_rn(total, 225.0);                                                  // np.average
     for (int e = lane; e < RSD_TF; e += 32) { out->tf[e] = v[e]; out->tfc[e] = __dadd_rn(v[e], -avg); }
@@ -114,11 +163,15 @@ __global__ void __launch_bounds__(32) k_sim_query(const uint8_t *__restrict__ q,
     sim_query_build(v, q, len, out);
 }
 
-// one CTA per query of a batch: query q is codes[off[q] .. off[q+1]) -> out[q]
-__global__ void __launch_bounds__(32) k_sim_query_batch(const uint8_t *__restrict__ codes, const int64_t *__restrict__ off, SimQuery *out) {
+// one CTA per query of a batch: query q is codes[off[q] .. off[q+1]) -> out[q]; vector type VT (idf: the table, VT != 0)
+template <int VT>
+__global__ void __launch_bounds__(32) k_sim_query_batch(const uint8_t *__restrict__ codes, const int64_t *__restrict__ off, SimQuery *out,
+                                                        const double *__restrict__ idf) {
     __shared__ double v[RSD_TF];
+    __shared__ double w[VT == RSD_VEC_TFIDF ? RSD_TF : 1];
+    __shared__ uint32_t pres[8];
     const int q = blockIdx.x;
-    sim_query_build(v, codes + off[q], (int)(off[q + 1] - off[q]), out + q);
+    sim_query_build<VT>(v, codes + off[q], (int)(off[q + 1] - off[q]), out + q, w, pres, idf);
 }
 
 // One thread per stored record: set_* (IR:54-91) and multi_* (IR:110-145) measures.
@@ -366,11 +419,20 @@ k_sim_small_batch(const uint32_t *__restrict__ db_words, const int64_t *__restri
 // terms is +0; every partial sum of the pairwise order is then >= +0, and adding +0 to it changes nothing.  The 16
 // corner products keep their accumulator and their place in the order (np_sum225_thread with a compile-time test).
 // Pearson's query vector is centred (negative entries) and the Euclidean / Manhattan terms are not zero: full sums.
+//
+// VT = RSD_VEC_IDF / RSD_VEC_TFIDF (idf = the 225-entry table): the record's idf vector is idf[p] at its literal bigrams,
+// all in the corner.  Its tf-idf entry (i, j) of the corner is the fused chain sum_k tf[i][k] * idf_vec[k][j] over
+// k = 0..3: the terms k >= 4 are fma(0, x, acc) with x finite and >= +0, and every acc of the chain is >= +0, so each
+// leaves acc unchanged; every entry outside the corner is a chain of such terms from +0.0, so +0.  Two things of the
+// 'tf' case do not carry over: np.average of the vector is a real pairwise sum (np_sum225_thread), and the query
+// entries are >= +0 only while every idf entry is (a_nonneg, checked on the host when the table is built); otherwise
+// num of cosine / Tanimoto / Dice is the full sum.
+template <int VT>
 __global__ void __launch_bounds__(128)
 k_sim_tf_thread_batch(const uint32_t *__restrict__ db_words, const int64_t *__restrict__ db_start, const int32_t *__restrict__ db_len,
                       int64_t n_rec, int db_bits, const int64_t *__restrict__ perm, int64_t global_base,
                       const SimQuery *__restrict__ Q, int nq, int method, double *__restrict__ scores, int64_t stride,
-                      int *__restrict__ worklist, int *__restrict__ worklist_n) {
+                      int *__restrict__ worklist, int *__restrict__ worklist_n, const double *__restrict__ idf, int a_nonneg) {
     __shared__ double s_a[RSD_SIM_QT][RSD_TF];
     __shared__ double s_asq[RSD_SIM_QT];
     __shared__ uint16_t s_cnt[16][128];
@@ -398,14 +460,32 @@ k_sim_tf_thread_batch(const uint32_t *__restrict__ db_words, const int64_t *__re
         if (!plain) worklist[atomicAdd(worklist_n, 1)] = (int)r;
     }
     double b[16];
+    if constexpr (VT == RSD_VEC_TF) {
 #pragma unroll
-    for (int e = 0; e < 16; ++e) b[e] = plain ? (double)s_cnt[e][tid] : 0.0;
+        for (int e = 0; e < 16; ++e) b[e] = plain ? (double)s_cnt[e][tid] : 0.0;
+    } else {
+        double iv[16];                                                         // the record's idf vector (corner)
+#pragma unroll
+        for (int e = 0; e < 16; ++e) iv[e] = plain && s_cnt[e][tid] ? __ldg(&idf[e / 4 * 15 + e % 4]) : 0.0;
+#pragma unroll
+        for (int e = 0; e < 16; ++e) {
+            if constexpr (VT == RSD_VEC_IDF) b[e] = iv[e];
+            else {
+                double acc = 0.0;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) acc = __fma_rn((double)s_cnt[e / 4 * 4 + k][tid], iv[k * 4 + e % 4], acc);
+                b[e] = plain ? acc : 0.0;
+            }
+        }
+    }
     auto corner = [](int e) { return e / 15 < 4 && e % 15 < 4; };
     auto bv = [&](int e) -> double { return corner(e) ? b[e / 15 * 4 + e % 15] : 0.0; };
+    const bool skip_zero = VT == RSD_VEC_TF || a_nonneg;                      // num: the 209 non-corner terms are +0
     double avg = 0.0, b_sq = 0.0;
     if (plain) {
         if (pearson) {
-            avg = __ddiv_rn((double)(len > 0 ? len - 1 : 0), 225.0);                  // the counts sum exactly (k_sim_tf_thread)
+            if constexpr (VT == RSD_VEC_TF) avg = __ddiv_rn((double)(len > 0 ? len - 1 : 0), 225.0);   // the counts sum exactly (k_sim_tf_thread)
+            else avg = __ddiv_rn(np_sum225_thread(bv), 225.0);
             b_sq = np_sum225_thread([&](int e) { const double x = __dadd_rn(bv(e), -avg); return __dmul_rn(x, x); });
         } else if (method == RSD_SIM_COSINE || method == RSD_SIM_TANIMOTO || method == RSD_SIM_DICE) {
             b_sq = np_sum225_thread([&](int e) { return __dmul_rn(bv(e), bv(e)); });
@@ -436,7 +516,7 @@ k_sim_tf_thread_batch(const uint32_t *__restrict__ db_words, const int64_t *__re
                 const double d = np_sum225_thread([&](int e) { return fabs(__dadd_rn(a[e], -bv(e))); });
                 v = __ddiv_rn(1.0, __dadd_rn(1.0, __dsqrt_rn(d)));
             } else {
-                const double num = np_sum225_thread([&](int e) { return corner(e) ? __dmul_rn(a[e], bv(e)) : 0.0; });
+                const double num = np_sum225_thread([&](int e) { return corner(e) || !skip_zero ? __dmul_rn(a[e], bv(e)) : 0.0; });
                 if (method == RSD_SIM_COSINE) v = __ddiv_rn(num, __dsqrt_rn(__dmul_rn(a_sq, b_sq)));
                 else if (method == RSD_SIM_TANIMOTO) v = __ddiv_rn(num, __dadd_rn(__dadd_rn(a_sq, b_sq), -num));
                 else v = __ddiv_rn(__dmul_rn(2.0, num), __dadd_rn(a_sq, b_sq));
@@ -448,12 +528,16 @@ k_sim_tf_thread_batch(const uint32_t *__restrict__ db_words, const int64_t *__re
 
 // One warp per worklist record, nq queries (k_sim_tf for a batch): the record's TF matrix (centred for Pearson) and
 // its own sums once in shared memory, then the per-query sums with the query vectors read from SimQuery; the final
-// divisions run one query per lane.
+// divisions run one query per lane.  VT != RSD_VEC_TF: the record's idf / tf-idf vector instead (vec_from_tf).
+template <int VT>
 __global__ void __launch_bounds__(128)
 k_sim_tf_batch(const uint32_t *__restrict__ db_words, const int64_t *__restrict__ db_start, const int32_t *__restrict__ db_len,
                int db_bits, const int64_t *__restrict__ perm, int64_t global_base, const SimQuery *__restrict__ Q, int nq, int method,
-               double *__restrict__ scores, int64_t stride, const int *__restrict__ worklist, const int *__restrict__ worklist_n) {
+               double *__restrict__ scores, int64_t stride, const int *__restrict__ worklist, const int *__restrict__ worklist_n,
+               const double *__restrict__ idf) {
     __shared__ double s_v[4][RSD_TF];
+    __shared__ double s_w[4][VT == RSD_VEC_TFIDF ? RSD_TF : 1];
+    __shared__ uint32_t s_pres[4][8];
     __shared__ double s_sum[4][RSD_SIM_QB];                   // per query: num, or the distance sum
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const bool pearson = method == RSD_SIM_PEARSON, dist = method == RSD_SIM_EUCLIDEAN || method == RSD_SIM_MANHATTAN;
@@ -465,6 +549,7 @@ k_sim_tf_batch(const uint32_t *__restrict__ db_words, const int64_t *__restrict_
         const int len = db_len[r];
         const int64_t st = db_start[r];
         tf_build(v, len, [&](int i) { return (int)pk_get(db_words, st, i, db_bits); });
+        if constexpr (VT != RSD_VEC_TF) vec_from_tf<VT>(v, s_w[wib], s_pres[wib], len, [&](int i) { return (int)pk_get(db_words, st, i, db_bits); }, idf);
         if (pearson) {
             const double avg = __ddiv_rn(np_sum225([&](int e) { return v[e]; }), 225.0);
             for (int e = lane; e < RSD_TF; e += 32) v[e] = __dadd_rn(v[e], -avg);
@@ -506,4 +591,104 @@ __global__ void k_sim_filter_batch(const double *__restrict__ scores, int64_t st
         const int slot = atomicAdd(&tk.cand_n[q], 1);
         if (slot < tk.cap) { tk.cand_s[(size_t)q * tk.cap + slot] = s; tk.cand_i[(size_t)q * tk.cap + slot] = g; }
     }
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// document-frequency table of the idf vectors (IR:189-216)
+// ------------------------------------------------------------------------------------------------------------------
+// compare_pair_to_seq(p, doc) (IR:225-252) depends only on the set of literal bigrams of the document: it is the
+// largest product wa * wb over the expansions (a, b) of p (possibilities(p[0]) x possibilities(p[1]), IR:255-287, at
+// most 8 x 8; p itself is the expansion of product 1) whose bigram a + b occurs, and 0 when none occurs.  The host
+// lists every pair's expansions by product, largest first (IdfExp), so the value is the product of the first one present.
+#define RSD_IDF_EXP 64
+#define RSD_IDF_T 160             // records per tile of k_idf_chain (one per worker thread)
+
+struct IdfExp {
+    int n[RSD_TF];                        // expansions of pair p
+    uint8_t e[RSD_TF][RSD_IDF_EXP];       // their bigrams (a * 15 + b)
+    double w[RSD_TF][RSD_IDF_EXP];        // their products wa * wb, non-increasing
+};
+
+// inv[perm[r] - global_base] = r: the stored record of every collection index of the shard
+__global__ void k_idf_inv(const int64_t *__restrict__ perm, int64_t global_base, int64_t n, int64_t *__restrict__ inv) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < n) inv[perm[r] - global_base] = r;
+}
+
+// The literal-bigram presence sets (225 bits in 8 words) of the records i0 .. i0 + n - 1 of the shard, in collection
+// order: pres[8 * i + word].  One thread per record.
+__global__ void __launch_bounds__(256)
+k_idf_pres(const uint32_t *__restrict__ db_words, const int64_t *__restrict__ db_start, const int32_t *__restrict__ db_len, int db_bits,
+           const int64_t *__restrict__ inv, int64_t i0, int64_t n, uint32_t *__restrict__ pres) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t r = inv[i0 + i];
+    const int len = db_len[r];
+    const int64_t st = db_start[r];
+    uint32_t m[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    if (len > 0) {
+        uint32_t prev = pk_get(db_words, st, 0, db_bits);
+        for (int j = 1; j < len; ++j) {
+            const uint32_t cur = pk_get(db_words, st, j, db_bits);
+            const uint32_t e = prev * 15u + cur;
+#pragma unroll
+            for (int w = 0; w < 8; ++w) m[w] |= (e >> 5 == (uint32_t)w) ? 1u << (e & 31u) : 0u;      // registers, no local array
+            prev = cur;
+        }
+    }
+    uint4 *o = reinterpret_cast<uint4 *>(pres + 8 * i);
+    o[0] = make_uint4(m[0], m[1], m[2], m[3]);
+    o[1] = make_uint4(m[4], m[5], m[6], m[7]);
+}
+
+// df[p] += compare_pair_to_seq(p, record i) for i = 0 .. n - 1 in that order (IR:205-212: `df = df + v` over
+// collection.find({})).  Each of the 225 sums is one dependent chain of __dadd_rn -- the order decides the bits, so no
+// tree or atomic reduction.  CTA = row a of the table (pairs a * 15 + j, j = 0..14), 32 + RSD_IDF_T threads: lane j of
+// warp 0 runs the chain of pair j over one tile of values while the other RSD_IDF_T threads compute the next tile's
+// values (one record each, all 15 pairs) into the other shared buffer.  df carries the sums from launch to launch.
+__global__ void __launch_bounds__(32 + RSD_IDF_T)
+k_idf_chain(const uint32_t *__restrict__ pres, int64_t n, const IdfExp *__restrict__ X, double *__restrict__ df) {
+    constexpr int TP = RSD_IDF_T + 1;                         // row stride: the 15 chain lanes read 15 different banks
+    __shared__ double s_val[2][15 * TP];
+    __shared__ double s_w[15][RSD_IDF_EXP];
+    __shared__ uint8_t s_e[15][RSD_IDF_EXP];
+    __shared__ int s_n[15];
+    const int a = blockIdx.x, tid = threadIdx.x;
+    for (int x = tid; x < 15 * RSD_IDF_EXP; x += blockDim.x) {
+        const int j = x / RSD_IDF_EXP, m = x % RSD_IDF_EXP;
+        s_w[j][m] = X->w[a * 15 + j][m]; s_e[j][m] = X->e[a * 15 + j][m];
+    }
+    if (tid < 15) s_n[tid] = X->n[a * 15 + tid];
+    double acc = tid < 15 ? df[a * 15 + tid] : 0.0;
+    __syncthreads();
+    const int64_t n_tiles = (n + RSD_IDF_T - 1) / RSD_IDF_T;
+    for (int64_t t = 0; t <= n_tiles; ++t) {
+        if (tid < 32) {
+            if (t > 0 && tid < 15) {                            // the chains over tile t - 1
+                const double *val = s_val[(t - 1) & 1] + tid * TP;
+                const int cnt = (int)min((int64_t)RSD_IDF_T, n - (t - 1) * RSD_IDF_T);
+#pragma unroll 8
+                for (int x = 0; x < cnt; ++x) acc = __dadd_rn(acc, val[x]);
+            }
+        } else if (t < n_tiles) {                               // the values of tile t
+            const int x = tid - 32;
+            const int64_t i = t * RSD_IDF_T + x;
+            if (i < n) {
+                const uint4 p0 = reinterpret_cast<const uint4 *>(pres + 8 * i)[0], p1 = reinterpret_cast<const uint4 *>(pres + 8 * i)[1];
+                double *val = s_val[t & 1] + x;
+                for (int j = 0; j < 15; ++j) {
+                    double v = 0.0;
+                    for (int m = 0; m < s_n[j]; ++m) {
+                        const int e = s_e[j][m], q = e >> 5;
+                        const uint4 h = q < 4 ? p0 : p1;           // selects, so the set stays in registers
+                        const uint32_t word = (q & 3) == 0 ? h.x : (q & 3) == 1 ? h.y : (q & 3) == 2 ? h.z : h.w;
+                        if (word >> (e & 31) & 1u) { v = s_w[j][m]; break; }
+                    }
+                    val[j * TP] = v;
+                }
+            }
+        }
+        __syncthreads();
+    }
+    if (tid < 15) df[a * 15 + tid] = acc;
 }

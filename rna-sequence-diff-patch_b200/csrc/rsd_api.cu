@@ -1452,6 +1452,7 @@ extern "C" int rsd_db_load(rsd_ctx *c, const uint32_t *words, const int64_t *sta
     if (bits != 2 && bits != 4) return rsd_fail(RSD_EINVAL, "rsd: bits must be 2 or 4");
     if (bits == 2 && (symmask & ~0xFu)) return rsd_fail(RSD_EINVAL, "rsd_db_load: 2-bit packing with symbols outside ACGU");
     RSD_OK_OR_RETURN(c->ensure_device());
+    c->idf_ready = false;
     // Records are stored sorted by length (stable, so equal lengths keep collection order): the warps of
     // the search kernel then hold records of one length and skip the padding columns.  perm[r] is the
     // collection index of stored record r; every key and every all_scores row uses it.
@@ -1556,8 +1557,8 @@ extern "C" int rsd_db_load(rsd_ctx *c, const uint32_t *words, const int64_t *sta
 
 extern "C" int rsd_db_free(rsd_ctx *c) {
     if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
-    if (c->inited && c->pid == getpid()) { cudaSetDevice(c->device); c->db.release(); c->db_perm.release(); c->db_topi.release(); c->db_tops.release(); c->db_aux.release(); c->db_dist.release(); c->rng_keys.release(); c->rng_dist.release(); c->rng_tmp.release(); c->sim_scores.release(); c->sim_aux.release(); c->sim_work.release(); }
-    c->db_loaded = false; c->db_n = 0;
+    if (c->inited && c->pid == getpid()) { cudaSetDevice(c->device); c->db.release(); c->db_perm.release(); c->db_topi.release(); c->db_tops.release(); c->db_aux.release(); c->db_dist.release(); c->rng_keys.release(); c->rng_dist.release(); c->rng_tmp.release(); c->sim_scores.release(); c->sim_aux.release(); c->sim_work.release(); c->idf_work.release(); }
+    c->db_loaded = false; c->db_n = 0; c->idf_ready = false;
     return RSD_OK;
 }
 
@@ -2140,8 +2141,9 @@ static int sim_upload_queries(rsd_ctx *c, const uint8_t *q_codes, const int64_t 
 // QB: each batch is one pass over the records into scores [QB][db_n], then the top-k of each query with the chunk
 // sequence of rsd_db_similarity (a 4096-record seed chunk, then chunks of min(db_n, 2^20)).  Outputs: top_idx_dev /
 // top_score_dev [n_queries][k] on the device (k > 0); all_scores (host, may be NULL): query q's db_n scores at
-// all_scores + q * all_stride + all_col.  Timed (rsd_set_timing) from the first kernel to the last copy.
-static int sim_batch_dev(rsd_ctx *c, int64_t n_queries, int method, int k, int64_t *top_idx_dev, double *top_score_dev,
+// all_scores + q * all_stride + all_col.  Timed (rsd_set_timing) from the first kernel to the last copy.  vt: the
+// vector type (RSD_VEC_TF, or RSD_VEC_IDF / RSD_VEC_TFIDF with the context's idf table uploaded, idf_upload).
+static int sim_batch_dev(rsd_ctx *c, int vt, int64_t n_queries, int method, int k, int64_t *top_idx_dev, double *top_score_dev,
                          double *all_scores, int64_t all_stride, int64_t all_col) {
     cudaStream_t st = c->stream;
     const int64_t n = c->db_n;
@@ -2179,10 +2181,16 @@ static int sim_batch_dev(rsd_ctx *c, int64_t n_queries, int method, int k, int64
     SimQuery *simq = (SimQuery *)c->sim_q.p;
     double *scores = (double *)c->sim_scores.p;
     int *wl_n = (int *)c->sim_work.p, *wl = wl_n + 4;
+    const double *idf = vt == RSD_VEC_TF ? nullptr : (const double *)c->idf_dev.p;
+    const int a_nonneg = c->idf_nonneg;
+    auto k_query = vt == RSD_VEC_IDF ? k_sim_query_batch<RSD_VEC_IDF> : vt == RSD_VEC_TFIDF ? k_sim_query_batch<RSD_VEC_TFIDF> : k_sim_query_batch<RSD_VEC_TF>;
+    auto k_thread = vt == RSD_VEC_IDF ? k_sim_tf_thread_batch<RSD_VEC_IDF> : vt == RSD_VEC_TFIDF ? k_sim_tf_thread_batch<RSD_VEC_TFIDF>
+                                                                                                 : k_sim_tf_thread_batch<RSD_VEC_TF>;
+    auto k_warp = vt == RSD_VEC_IDF ? k_sim_tf_batch<RSD_VEC_IDF> : vt == RSD_VEC_TFIDF ? k_sim_tf_batch<RSD_VEC_TFIDF> : k_sim_tf_batch<RSD_VEC_TF>;
     if (c->timing) RSD_CUDA(cudaEventRecord(c->ev0, st));
     for (int64_t q0 = 0; q0 < n_queries; q0 += qb) {
         const int nq = (int)std::min<int64_t>(qb, n_queries - q0);
-        k_sim_query_batch<<<nq, 32, 0, st>>>(codes, off + q0, simq);
+        k_query<<<nq, 32, 0, st>>>(codes, off + q0, simq, idf);
         c->launches += 1;
         if (n > 0) {
             if (method < RSD_SIM_COSINE) {
@@ -2191,10 +2199,10 @@ static int sim_batch_dev(rsd_ctx *c, int64_t n_queries, int method, int k, int64
             } else {
                 // plain A/G/C/U records: one thread each; the rest (ambiguity codes, > 60000 symbols) through the worklist
                 RSD_CUDA(cudaMemsetAsync(wl_n, 0, sizeof(int), st));
-                k_sim_tf_thread_batch<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(dbw, dbs, dbl, n, c->db_bits, perm, c->db_base, simq, nq, method,
-                                                                               scores, n, wl, wl_n);
+                k_thread<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(dbw, dbs, dbl, n, c->db_bits, perm, c->db_base, simq, nq, method,
+                                                                  scores, n, wl, wl_n, idf, a_nonneg);
                 const unsigned grid = (unsigned)std::min<int64_t>((n + 3) / 4, (int64_t)c->sm_count * 16);
-                k_sim_tf_batch<<<grid, 128, 0, st>>>(dbw, dbs, dbl, c->db_bits, perm, c->db_base, simq, nq, method, scores, n, wl, wl_n);
+                k_warp<<<grid, 128, 0, st>>>(dbw, dbs, dbl, c->db_bits, perm, c->db_base, simq, nq, method, scores, n, wl, wl_n, idf);
                 c->launches += 2;
             }
         }
@@ -2223,20 +2231,16 @@ static int sim_batch_dev(rsd_ctx *c, int64_t n_queries, int method, int k, int64
     return RSD_OK;
 }
 
-extern "C" int rsd_db_similarity_batch(rsd_ctx *c, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
-                                       int method, int k, int64_t *top_idx, double *top_score, double *all_scores) {
-    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
-    RSD_OK_OR_RETURN(sim_batch_args("rsd_db_similarity_batch", q_codes, q_off, n_queries, method, k, top_idx, top_score));
-    RSD_OK_OR_RETURN(c->ensure_device());
-    if (n_queries == 0) return RSD_OK;
-    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_similarity_batch: no database loaded (rsd_db_load)");
+// a query batch against the loaded database after its arguments were checked: queries up, sim_batch_dev, results down
+static int sim_batch_host(rsd_ctx *c, int vt, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries, int method, int k,
+                          int64_t *top_idx, double *top_score, double *all_scores) {
     cudaStream_t st = c->stream;
     c->timed = false; c->last_ms_override = 0.0;
     const size_t cells = (size_t)n_queries * (size_t)std::max(k, 1);
     RSD_OK_OR_RETURN(c->sim_top.ensure(sizeof(int64_t) * 2 * cells));
     int64_t *ti = (int64_t *)c->sim_top.p; double *ts = (double *)(ti + cells);
     RSD_OK_OR_RETURN(sim_upload_queries(c, q_codes, q_off, n_queries));
-    RSD_OK_OR_RETURN(sim_batch_dev(c, n_queries, method, k, ti, ts, all_scores, c->db_n, 0));
+    RSD_OK_OR_RETURN(sim_batch_dev(c, vt, n_queries, method, k, ti, ts, all_scores, c->db_n, 0));
     if (k > 0) {
         RSD_CUDA(cudaMemcpyAsync(top_idx, ti, sizeof(int64_t) * (size_t)n_queries * k, cudaMemcpyDeviceToHost, st));
         RSD_CUDA(cudaMemcpyAsync(top_score, ts, sizeof(double) * (size_t)n_queries * k, cudaMemcpyDeviceToHost, st));
@@ -2244,6 +2248,160 @@ extern "C" int rsd_db_similarity_batch(rsd_ctx *c, const uint8_t *q_codes, const
     RSD_CUDA(cudaGetLastError());
     RSD_CUDA(cudaStreamSynchronize(st));
     return RSD_OK;
+}
+
+extern "C" int rsd_db_similarity_batch(rsd_ctx *c, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                                       int method, int k, int64_t *top_idx, double *top_score, double *all_scores) {
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    RSD_OK_OR_RETURN(sim_batch_args("rsd_db_similarity_batch", q_codes, q_off, n_queries, method, k, top_idx, top_score));
+    RSD_OK_OR_RETURN(c->ensure_device());
+    if (n_queries == 0) return RSD_OK;
+    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_similarity_batch: no database loaded (rsd_db_load)");
+    return sim_batch_host(c, RSD_VEC_TF, q_codes, q_off, n_queries, method, k, top_idx, top_score, all_scores);
+}
+
+// ------------------------------------------------------------------------------------------------
+// idf / tf-idf vectors (IR:189-225, searched by IR:458-465)
+// ------------------------------------------------------------------------------------------------
+// possibilities(symbol) (IR:255-287): a base first with probability 1, then every ambiguity code that may stand for it
+// (IR:20-46 order) with that code's weight; an ambiguity code: the bases it may stand for, each 1 / (their number),
+// then the code itself with probability 1.
+static int idf_possibilities(int s, int *sym, double *prob) {
+    static const double W[15][4] = {
+        {1, 0, 0, 0}, {0, 1, 0, 0}, {0, 0, 1, 0}, {0, 0, 0, 1},
+        {0, 0, 0.5, 0.5}, {0.5, 0.5, 0, 0}, {0.5, 0, 0, 0.5}, {0, 0.5, 0.5, 0}, {0, 0.5, 0, 0.5}, {0.5, 0, 0.5, 0},
+        {0.33, 0.33, 0, 0.33}, {0.33, 0.33, 0.33, 0}, {0.33, 0, 0.33, 0.33}, {0, 0.33, 0.33, 0.33}, {0.25, 0.25, 0.25, 0.25}};
+    int n = 0;
+    if (s < 4) {
+        sym[n] = s; prob[n++] = 1.0;
+        for (int x = 4; x < 15; ++x) if (W[x][s] != 0) { sym[n] = x; prob[n++] = W[x][s]; }
+        return n;
+    }
+    for (int b = 0; b < 4; ++b) if (W[s][b] != 0) sym[n++] = b;
+    for (int i = 0; i < n; ++i) prob[i] = 1.0 / (double)n;
+    sym[n] = s; prob[n++] = 1.0;
+    return n;
+}
+
+// the expansions of every pair (IdfExp, k_sim.cuh), built once per process
+static const IdfExp &idf_expansions() {
+    static const IdfExp X = [] {
+        IdfExp x{};
+        for (int p = 0; p < RSD_TF; ++p) {
+            int sa[8], sb[8]; double pa[8], pb[8];
+            const int na = idf_possibilities(p / 15, sa, pa), nb = idf_possibilities(p % 15, sb, pb);
+            std::vector<std::pair<double, int>> ex;
+            for (int i = 0; i < na; ++i) for (int j = 0; j < nb; ++j) ex.push_back({pa[i] * pb[j], sa[i] * 15 + sb[j]});
+            std::stable_sort(ex.begin(), ex.end(), [](const std::pair<double, int> &u, const std::pair<double, int> &v) { return u.first > v.first; });
+            x.n[p] = (int)ex.size();
+            for (size_t m = 0; m < ex.size(); ++m) { x.w[p][m] = ex[m].first; x.e[p][m] = (uint8_t)ex[m].second; }
+        }
+        return x;
+    }();
+    return X;
+}
+
+// Continues the 225 df sums (host df, in and out) over the records of the shard loaded in c, in collection order.
+static int idf_df_shard(rsd_ctx *c, double *df) {
+    cudaStream_t st = c->stream;
+    const int64_t n = c->db_n;
+    RSD_OK_OR_RETURN(c->idf_dev.ensure(sizeof(double) * 2 * RSD_TF));
+    double *d_df = (double *)c->idf_dev.p + RSD_TF;
+    RSD_CUDA(cudaMemcpyAsync(d_df, df, sizeof(double) * RSD_TF, cudaMemcpyHostToDevice, st));
+    if (n > 0) {
+        RSD_OK_OR_RETURN(c->idf_exp.ensure(sizeof(IdfExp)));
+        RSD_CUDA(cudaMemcpyAsync(c->idf_exp.p, &idf_expansions(), sizeof(IdfExp), cudaMemcpyHostToDevice, st));
+        // chunks of 2^20 records: the presence sets take 32 bytes per record of the chunk
+        const int64_t CH = std::min<int64_t>(n, (int64_t)1 << 20);
+        RSD_OK_OR_RETURN(c->idf_work.ensure(32 * (size_t)CH + sizeof(int64_t) * (size_t)n));
+        uint32_t *pres = (uint32_t *)c->idf_work.p;            // first: the kernels access it as 16-byte uint4
+        int64_t *inv = (int64_t *)(pres + 8 * CH);
+        const uint32_t *dbw = (const uint32_t *)c->db.words.p; const int64_t *dbs = (const int64_t *)c->db.start.p; const int32_t *dbl = (const int32_t *)c->db.len.p;
+        k_idf_inv<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const int64_t *)c->db_perm.p, c->db_base, n, inv);
+        c->launches += 1;
+        for (int64_t i0 = 0; i0 < n; i0 += CH) {
+            const int64_t nn = std::min(CH, n - i0);
+            k_idf_pres<<<(unsigned)((nn + 255) / 256), 256, 0, st>>>(dbw, dbs, dbl, c->db_bits, inv, i0, nn, pres);
+            k_idf_chain<<<15, 32 + RSD_IDF_T, 0, st>>>(pres, nn, (const IdfExp *)c->idf_exp.p, d_df);
+            c->launches += 2;
+        }
+    }
+    RSD_CUDA(cudaGetLastError());
+    RSD_CUDA(cudaMemcpyAsync(df, d_df, sizeof(double) * RSD_TF, cudaMemcpyDeviceToHost, st));
+    RSD_CUDA(cudaStreamSynchronize(st));
+    return RSD_OK;
+}
+
+// IR:213-214: idf[p] = 0 if df[p] == 0 else math.log(N / df[p], 10), which CPython evaluates as log(N / df) / log(10.0)
+// with the C library's log -- computed here on the host for that reason (the device log rounds differently).  Returns
+// whether every entry is finite and >= +0 (always, as df[p] <= N; k_sim_tf_thread_batch relies on it when it holds).
+static bool idf_from_df(const double *df, int64_t N, double *idf) {
+    volatile double ten = 10.0;                    // evaluated at run time like CPython's, not folded by the compiler
+    const double l10 = std::log((double)ten);
+    bool nonneg = true;
+    for (int p = 0; p < RSD_TF; ++p) {
+        idf[p] = df[p] == 0 ? 0.0 : std::log((double)N / df[p]) / l10;
+        nonneg = nonneg && std::isfinite(idf[p]) && !std::signbit(idf[p]);
+    }
+    return nonneg;
+}
+
+// the table to the device (idf_dev[0..225)) and the context's host copies
+static int idf_upload(rsd_ctx *c, const double *df, const double *idf, bool nonneg) {
+    RSD_OK_OR_RETURN(c->ensure_device());
+    RSD_OK_OR_RETURN(c->idf_dev.ensure(sizeof(double) * 2 * RSD_TF));
+    RSD_CUDA(cudaMemcpyAsync(c->idf_dev.p, idf, sizeof(double) * RSD_TF, cudaMemcpyHostToDevice, c->stream));
+    RSD_CUDA(cudaStreamSynchronize(c->stream));
+    memcpy(c->idf_df, df, sizeof c->idf_df); memcpy(c->idf_tab, idf, sizeof c->idf_tab);
+    c->idf_nonneg = nonneg;
+    return RSD_OK;
+}
+
+// the loaded database's table, built when the context does not hold it yet (timed on its own: rsd_set_timing)
+static int idf_ensure(rsd_ctx *c, const char *fn) {
+    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "%s: no database loaded (rsd_db_load)", fn);
+    if (c->db_base != 0)
+        return rsd_fail(RSD_EINVAL, "%s: the database was loaded with global_index_base %lld: a shard cannot know the collection's "
+                        "document frequencies (rsd_multi holds every shard)", fn, (long long)c->db_base);
+    if (c->idf_ready) return RSD_OK;
+    c->timed = false; c->last_ms_override = 0.0;
+    if (c->timing) RSD_CUDA(cudaEventRecord(c->ev0, c->stream));
+    double df[RSD_TF] = {}, idf[RSD_TF];
+    RSD_OK_OR_RETURN(idf_df_shard(c, df));
+    if (c->timing) { RSD_CUDA(cudaEventRecord(c->ev1, c->stream)); RSD_CUDA(cudaEventSynchronize(c->ev1)); c->timed = true; }
+    RSD_OK_OR_RETURN(idf_upload(c, df, idf, idf_from_df(df, c->db_n, idf)));
+    c->idf_ready = true;
+    return RSD_OK;
+}
+
+extern "C" int rsd_db_idf_table(rsd_ctx *c, double *df, double *idf) {
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    RSD_OK_OR_RETURN(c->ensure_device());
+    RSD_OK_OR_RETURN(idf_ensure(c, "rsd_db_idf_table"));
+    if (df) memcpy(df, c->idf_df, sizeof c->idf_df);
+    if (idf) memcpy(idf, c->idf_tab, sizeof c->idf_tab);
+    return RSD_OK;
+}
+
+// the host-side checks of a vector-type batch, in front of sim_batch_args
+static int vec_batch_args(const char *fn, int vector_type, int method) {
+    if (vector_type != RSD_VEC_IDF && vector_type != RSD_VEC_TFIDF) return rsd_fail(RSD_EINVAL, "%s: unknown vector type %d", fn, vector_type);
+    if (method < RSD_SIM_COSINE || method > RSD_SIM_DICE)
+        return rsd_fail(RSD_EINVAL, "%s: method %d is not a vector measure (RSD_SIM_COSINE..RSD_SIM_DICE)", fn, method);
+    return RSD_OK;
+}
+
+extern "C" int rsd_db_vector_similarity_batch(rsd_ctx *c, const uint8_t *q_codes, const int64_t *q_off, int64_t n_queries,
+                                              int vector_type, int method, int k, int64_t *top_idx, double *top_score, double *all_scores) {
+    const char *fn = "rsd_db_vector_similarity_batch";
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    RSD_OK_OR_RETURN(vec_batch_args(fn, vector_type, method));
+    RSD_OK_OR_RETURN(sim_batch_args(fn, q_codes, q_off, n_queries, method, k, top_idx, top_score));
+    RSD_OK_OR_RETURN(c->ensure_device());
+    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "%s: no database loaded (rsd_db_load)", fn);
+    if (n_queries == 0) return RSD_OK;
+    RSD_OK_OR_RETURN(idf_ensure(c, fn));
+    return sim_batch_host(c, vector_type, q_codes, q_off, n_queries, method, k, top_idx, top_score, all_scores);
 }
 
 // ------------------------------------------------------------------------------------------------

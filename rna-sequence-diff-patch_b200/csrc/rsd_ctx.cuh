@@ -132,6 +132,12 @@ struct rsd_ctx {
     DevBuf rng_keys, rng_dist, rng_n, rng_tmp;
     DevBuf sim_q, sim_scores, sim_aux, sim_codes, sim_work;
     DevBuf sim_off, sim_top;               // rsd_db_similarity_batch: query offsets, [2][Q][k] top-k lists
+    // idf / tf-idf vectors: idf_dev = idf[225] then the df partial sums [225]; idf_exp = IdfExp; idf_work = one chunk of
+    // presence sets, then the inverse of db_perm, while the table is built
+    DevBuf idf_dev, idf_exp, idf_work;
+    bool idf_ready = false;                // idf_df / idf_tab / idf_dev hold the loaded database's table
+    bool idf_nonneg = true;                // every idf entry is finite and >= +0
+    double idf_df[225], idf_tab[225];
 
     int ensure_device();
     int classify(uint32_t symmask, int64_t max_m, int64_t max_n, int bits, int force_mode, ModeInfo &mi) const;
@@ -164,7 +170,8 @@ struct rsd_ctx {
         for (PlanSlot &s : slots) s.release();
         DevBuf *all[] = {&out_f64, &mat_vals, &mat_mask, &mat_ab,
                          &long_pool, &long_jobs, &dirs, &s_op, &s_oi, &s_oj, &s_nops, &s_ok, &s_tmp, &p_out, &p_len, &p_err, &misc,
-                         &db_dist, &db_topi, &db_tops, &db_aux, &db_perm, &rng_keys, &rng_dist, &rng_n, &rng_tmp, &sim_q, &sim_scores, &sim_aux, &sim_codes, &sim_work, &sim_off, &sim_top};
+                         &db_dist, &db_topi, &db_tops, &db_aux, &db_perm, &rng_keys, &rng_dist, &rng_n, &rng_tmp, &sim_q, &sim_scores, &sim_aux, &sim_codes, &sim_work, &sim_off, &sim_top,
+                         &idf_dev, &idf_exp, &idf_work};
         for (DevBuf *b : all) b->release();
         d_stage.release(); for (int s = 0; s < 2; ++s) { raw_codes[s].release(); sym_start[s].release(); }
         if (h_stage) { cudaFreeHost(h_stage); h_stage = nullptr; h_stage_cap = 0; }

@@ -5,7 +5,11 @@ index (balanced by total symbols), the query batch is the same on every rank, ea
 its local top-k per query with key (score desc, global index asc), and ONE all_gather of
 Q x k x (fp64 score, int64 index) per rank brings the candidates together; the merge with the same
 key (rsd_topk_merge) reproduces the reference's stable descending sort over the whole collection
-because shards are index-contiguous.  torch is plumbing only (process group, device tensors)."""
+because shards are index-contiguous.  torch is plumbing only (process group, device tensors).
+
+There is no idf / tf-idf similarity here: a rank holds one shard and cannot know the collection's document
+frequencies.  Callers that need those vector types over several GPUs use MultiEngine (one process), which runs the
+document-frequency sums through its shards in order."""
 from __future__ import annotations
 
 import numpy as np

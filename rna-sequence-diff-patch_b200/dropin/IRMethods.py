@@ -10,9 +10,13 @@ fa_import.py:5.  What runs where:
     vectors (gui.py:455-500, timing.py): host objects by nature (Python sets, numpy arrays) —
     rna_sequence_diff_patch_b200/measures.py, same values as the reference.  A measure called on two
     SEQUENCES (str) scores that pair on the GPU instead.
-  * search_collection with vector_type 'idf' / 'tf-idf' (IR:458-465): host, like the reference; a document
-    that lacks the stored 'idf' / 'tf' vector gets it computed from its sequence (the reference would raise
-    KeyError there: its importer never stores 'idf', fa_import.py:30-36,49).
+  * search_collection with vector_type 'idf' / 'tf-idf' (IR:458-465) and a vector measure: ONE GPU pass too
+    when every document is laid out as the reference's importer writes it -- a stored 'tf' vector and no stored
+    'idf' (fa_import.py:30-36,49) -- the collection's document-frequency table is built on the device and the
+    vectors are rebuilt from the sequences.  Any other collection keeps the host branch, like the reference:
+    one with stored 'idf' vectors (only a caller's own update_idfs writes them, and they may be stale) is scored
+    from those, and a document that lacks the stored 'idf' / 'tf' vector gets it computed from its sequence (the
+    reference would raise KeyError there).
   * create_search_threads (IR:480-515): one GPU scan per method, no fork, no second WF pass, no pandas."""
 import math  # noqa: F401  (module-level names of the reference module, visible to `from IRMethods import *`)
 import os
@@ -100,6 +104,9 @@ def search_collection(query, vector_type, collection, method, return_dict=None, 
         scores = _ir.score_collection(query, [doc['sequence'] for doc in collection.find({})], _SED.default_costs)
     elif method in _SET_MULTI or (method in _VECTOR and vector_type == 'tf'):
         scores = _ir.similarity_collection(query, [doc['sequence'] for doc in collection.find({})], method.__name__)
+    elif method in _VECTOR and all('tf' in doc and 'idf' not in doc for doc in collection.find({})):
+        scores = _ir.similarity_collection(query, [doc['sequence'] for doc in collection.find({})], method.__name__,
+                                           vector_type='idf' if vector_type == 'idf' else 'tf-idf')
     elif method in _VECTOR:
         def idf_of(s):
             return convert_to_idf_vector(s, collection)

@@ -61,6 +61,32 @@ def _sim_queries(queries):
     return np.ascontiguousarray(codes, np.uint8), off
 
 
+VECTOR_TYPES = {"tf": 0, "idf": 1, "tf-idf": 2}          # search_collection's vector_type (IR:455-465); 1, 2 = RSD_VEC_*
+
+
+def _vector_type(vector_type) -> int:
+    if isinstance(vector_type, str):
+        if vector_type not in VECTOR_TYPES:
+            raise _lib.RsdError(_lib.RSD_EINVAL, f"unknown vector type {vector_type!r}")
+        return VECTOR_TYPES[vector_type]
+    return int(vector_type)
+
+
+def _sim_entry(tf_fn, vec_fn, vector_type):
+    """The entry point of a similarity batch: the 'tf' one, or the idf / tf-idf one with the vector type bound."""
+    vt = _vector_type(vector_type)
+    if vt == 0:
+        return tf_fn
+    return lambda h, codes, off, nq, method, k, idx, sc, alls: vec_fn(h, codes, off, nq, vt, method, k, idx, sc, alls)
+
+
+def _idf_table(fn, h):
+    """Calls rsd_db_idf_table / rsd_multi_db_idf_table -> (df [15, 15], idf [15, 15])."""
+    df = np.zeros((15, 15), np.float64); idf = np.zeros((15, 15), np.float64)
+    check(fn(h, ptr(df, _f64), ptr(idf, _f64)))
+    return df, idf
+
+
 def _similarity_batch(fn, h, db_n: int, queries, method, k: int, want_scores: bool):
     """Calls rsd_db_similarity_batch / rsd_multi_db_similarity -> (all_scores [q, n] | None, top_idx [q, k], top_score [q, k])."""
     codes, off = _sim_queries(queries)
@@ -284,9 +310,13 @@ class Engine:
                    "multi_intersection_similarity", "multi_jaccard_similarity", "multi_dice_similarity",
                    "cosine", "pearson", "euclidian_distance", "manhattan_distance", "tanimoto_distance", "dice_dist")
 
-    def db_similarity(self, query_codes: np.ndarray, method, k: int = 0, want_scores: bool = True):
-        """IR:443-477 for the measures of IR:49-389 against the loaded database.
+    def db_similarity(self, query_codes: np.ndarray, method, k: int = 0, want_scores: bool = True, vector_type="tf"):
+        """IR:443-477 for the measures of IR:49-389 against the loaded database; vector_type 'idf' / 'tf-idf' (vector
+        measures only) scores the idf / tf-idf vectors of IR:189-225 instead of the TF matrices (IR:458-465).
         -> (all_scores f64[n_db] | None, top_idx int64[k], top_score f64[k])."""
+        if _vector_type(vector_type) != 0:
+            alls, idx, sc = self.db_similarity_batch([np.asarray(query_codes, np.uint8)], method, k, want_scores, vector_type)
+            return (alls[0] if want_scores else None), idx[0], sc[0]
         mid = _sim_method(method)
         q = np.ascontiguousarray(query_codes, np.uint8)
         qq = q if q.shape[0] else np.zeros(1, np.uint8)
@@ -296,11 +326,17 @@ class Engine:
                                           ptr(alls, _f64) if want_scores and self._db_n else None))
         return alls, idx[:k], sc[:k]
 
-    def db_similarity_batch(self, queries, method, k: int = 0, want_scores: bool = True):
+    def db_similarity_batch(self, queries, method, k: int = 0, want_scores: bool = True, vector_type="tf"):
         """db_similarity for a batch of queries in one pass over the database per query batch: `queries` is a list of
         code arrays or a (codes, offsets) tuple, as pack takes it.  Row q equals db_similarity(queries[q], ...) bit for bit.
         -> (all_scores f64[q, n_db] | None, top_idx int64[q, k], top_score f64[q, k])."""
-        return _similarity_batch(self._lib.rsd_db_similarity_batch, self._ctx, getattr(self, "_db_n", 0), queries, method, k, want_scores)
+        fn = _sim_entry(self._lib.rsd_db_similarity_batch, self._lib.rsd_db_vector_similarity_batch, vector_type)
+        return _similarity_batch(fn, self._ctx, getattr(self, "_db_n", 0), queries, method, k, want_scores)
+
+    def db_idf_table(self):
+        """The document frequencies and idf values of the loaded database (IR:189-216), built on the device on first use
+        after db_load -> (df f64[15, 15], idf f64[15, 15]).  A database loaded with global_index_base != 0 is refused."""
+        return _idf_table(self._lib.rsd_db_idf_table, self._ctx)
 
     def topk_merge(self, idx: np.ndarray, score: np.ndarray):
         return topk_merge(idx, score)
@@ -367,7 +403,7 @@ class Engine:
 class MultiEngine:
     """Database search over several GPUs from one process (include/rsd.h, rsd_multi_*): contiguous shards, the
     query batch on every device, local top-k, one NCCL all-gather of the lists, merge.  Same search interface as
-    Engine (set_costs / db_load / db_search_topk / db_search_range / db_similarity[_batch] / db_free), so
+    Engine (set_costs / db_load / db_search_topk / db_search_range / db_similarity[_batch] / db_idf_table / db_free), so
     ir.score_collection and ir.similarity_collection run on either."""
 
     def __init__(self, devices=None):
@@ -436,14 +472,19 @@ class MultiEngine:
         self._range_total = int(res[0][-1])
         return res
 
-    def db_similarity(self, query_codes: np.ndarray, method, k: int = 0, want_scores: bool = True):
+    def db_similarity(self, query_codes: np.ndarray, method, k: int = 0, want_scores: bool = True, vector_type="tf"):
         """Engine.db_similarity over the whole sharded database."""
-        alls, idx, sc = self.db_similarity_batch([np.asarray(query_codes, np.uint8)], method, k, want_scores)
+        alls, idx, sc = self.db_similarity_batch([np.asarray(query_codes, np.uint8)], method, k, want_scores, vector_type)
         return (alls[0] if want_scores else None), idx[0], sc[0]
 
-    def db_similarity_batch(self, queries, method, k: int = 0, want_scores: bool = True):
+    def db_similarity_batch(self, queries, method, k: int = 0, want_scores: bool = True, vector_type="tf"):
         """Engine.db_similarity_batch over the whole sharded database."""
-        return _similarity_batch(self._lib.rsd_multi_db_similarity, self._h, self._db_n, queries, method, k, want_scores)
+        fn = _sim_entry(self._lib.rsd_multi_db_similarity, self._lib.rsd_multi_db_vector_similarity, vector_type)
+        return _similarity_batch(fn, self._h, self._db_n, queries, method, k, want_scores)
+
+    def db_idf_table(self):
+        """Engine.db_idf_table over the whole sharded database: the sums run through the shards in order."""
+        return _idf_table(self._lib.rsd_multi_db_idf_table, self._h)
 
     def launch_count(self) -> int:
         return int(self._lib.rsd_multi_launch_count(self._h))

@@ -111,14 +111,19 @@ SIM_METHODS = ("set_intersection_similarity", "set_jaccard_similarity", "set_dic
                "cosine", "pearson", "euclidian_distance", "manhattan_distance", "tanimoto_distance", "dice_dist")
 
 
-def similarity_collection(query: str, sequences, method: str, engine=None):
+def similarity_collection(query: str, sequences, method: str, engine=None, vector_type: str = "tf"):
     """[(sequence, method(query, sequence))] in collection order for one of SIM_METHODS — what
-    search_collection(query, 'tf', collection, <method>) returns (IR:449-477), one GPU pass.  The documents'
+    search_collection(query, vector_type, collection, <method>) returns (IR:449-477), one GPU pass.  The documents'
     stored 'tf' vectors are rebuilt from the sequences on the device (they are convert_to_tf_vector(sequence),
-    fa_import.py:49).  Unknown symbols raise KeyError (the reference: KeyError IR:106 / ValueError IR:155).  Sharded over
-    every visible GPU like score_collection."""
+    fa_import.py:49).  vector_type 'idf' / 'tf-idf' (the six vector measures only; IR:458-465) scores the idf / tf-idf
+    vectors of IR:189-225 over these sequences as the whole collection.  Unknown symbols raise KeyError (the reference:
+    KeyError IR:106 / ValueError IR:155).  Sharded over every visible GPU like score_collection."""
     if method not in SIM_METHODS:
         raise ValueError(f"unknown similarity method {method!r}")
+    if vector_type not in ("tf", "idf", "tf-idf"):
+        raise ValueError(f"unknown vector type {vector_type!r}")
+    if method not in SIM_METHODS[6:]:
+        vector_type = "tf"               # the set / multiset measures have no vector type (IR:449-454)
     sequences = list(sequences)
     if not sequences:
         return []
@@ -126,7 +131,7 @@ def similarity_collection(query: str, sequences, method: str, engine=None):
     eng = engine or get_search_engine()
     qc = encode(query)
     _Resident.load(eng, sequences, upper=False)
-    scores, _, _ = eng.db_similarity(qc, method)
+    scores, _, _ = eng.db_similarity(qc, method, vector_type=vector_type)
     return [(s, float(v)) for s, v in zip(sequences, scores)]
 
 
