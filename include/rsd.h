@@ -178,6 +178,23 @@ int rsd_script_patch_check_batch(rsd_ctx *ctx,
 int rsd_db_load(rsd_ctx *ctx, const uint32_t *words, const int64_t *start, const int32_t *len,
                 int64_t n_records, int64_t n_words, int bits, uint32_t symmask, int64_t global_index_base);
 int rsd_db_free(rsd_ctx *ctx);
+/* Append n_records records (packed like rsd_db_load, same `bits` as the loaded database) to the end of the loaded
+ * database: record j gets global index global_index_base + db_n + j.  The state afterwards is the one rsd_db_load
+ * gives for the concatenation (old records, then new ones, in order): the same stored order (records sorted by tier,
+ * length and collection index, the tiers re-derived from the symbol counts of the concatenation), tiers, maximum
+ * length and word count; the symbol mask is the OR of the old mask and `symmask`.  Every search then answers as after
+ * a fresh load.  The stored order is rebuilt on the device: the loaded records are not uploaded again.  A built idf
+ * table is continued over the new records, not rebuilt.  Refused with RSD_EINVAL, before any device work: no database
+ * loaded, `bits` other than the database's, a 2-bit database with `symmask` outside ACGU, a negative length, a record
+ * outside the word buffer, NULL buffers with n_records > 0.  n_records == 0 changes nothing.  An error before the new
+ * layout is complete leaves the loaded database and its idf table unchanged; if only the idf continuation fails, the
+ * appended database stands (RSD_OK) and its table is rebuilt on next use. */
+int rsd_db_append(rsd_ctx *ctx, const uint32_t *words, const int64_t *start, const int32_t *len,
+                  int64_t n_records, int64_t n_words, int bits, uint32_t symmask);
+/* Introspection (tests, tools): the stored order of the loaded database.  *n_records = db_n; perm[db_n] (may be NULL)
+ * = global index of stored record r; tier_end[16], tier_mask[16] (either may be NULL): stored records
+ * [0, tier_end[t]) use only the symbols tier_mask[t]. */
+int rsd_db_layout(rsd_ctx *ctx, int64_t *n_records, int64_t *perm, int64_t *tier_end, uint32_t *tier_mask);
 /* queries packed like a batch; for each query q: the k best records of this shard by
  * (score = 1/(1+D) descending, global index ascending): top_idx[q*k+r] (global index, -1 when the
  * shard has fewer than k records), top_score[q*k+r].  all_scores (optional, host) receives
@@ -231,7 +248,8 @@ int rsd_db_similarity_batch(rsd_ctx *ctx, const uint8_t *q_codes, const int64_t 
  * The idf vector of a sequence is idf[p] = log10(N / df[p]) (0 where df[p] == 0) at each distinct literal bigram p of
  * it, 0 elsewhere; tf-idf is the matrix product tf . idf.  df[p] is the sum over the collection, in collection order,
  * of compare_pair_to_seq(p, document) (IRMethods.py:225-252), N the number of records.  The table is built on the
- * device on first use after rsd_db_load and kept until the next rsd_db_load / rsd_db_free; idf is computed on the host
+ * device on first use after rsd_db_load, continued by rsd_db_append and kept until the next rsd_db_load / rsd_db_free;
+ * idf is computed on the host
  * from df exactly as Python's math.log(N / df, 10).  A database loaded with global_index_base != 0 is one shard of a
  * collection whose other records it does not know: these calls refuse it (RSD_EINVAL); use rsd_multi for shards. */
 enum { RSD_VEC_IDF = 1, RSD_VEC_TFIDF = 2 };
@@ -265,6 +283,10 @@ int rsd_multi_set_costs(rsd_multi *m, double ins, double del, const double *sub)
 int rsd_multi_db_load(rsd_multi *m, const uint32_t *words, const int64_t *start, const int32_t *len,
                       int64_t n_records, int64_t n_words, int bits, uint32_t symmask);
 int rsd_multi_db_free(rsd_multi *m);
+/* rsd_db_append over the whole database: the records go to the last shard (shards stay index-contiguous, they are not
+ * rebalanced: a reload does that); a built idf table is continued and the new table goes to every device */
+int rsd_multi_db_append(rsd_multi *m, const uint32_t *words, const int64_t *start, const int32_t *len,
+                        int64_t n_records, int64_t n_words, int bits, uint32_t symmask);
 /* like rsd_db_search_topk, over the whole database; all_scores (optional) is [n_queries][n_records] */
 int rsd_multi_db_search_topk(rsd_multi *m, const uint32_t *q_words, const int64_t *q_start, const int32_t *q_len,
                              int64_t n_queries, int64_t q_nwords, int bits, uint32_t q_symmask, int k, int force_mode,

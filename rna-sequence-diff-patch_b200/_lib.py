@@ -58,6 +58,8 @@ SIGNATURES = {
                                           u8p, i32p, i32p, i32p, f64p, u8p, intp]),
     "rsd_db_load": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, i64]),
     "rsd_db_free": (ci, [vp]),
+    "rsd_db_append": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32]),
+    "rsd_db_layout": (ci, [vp, i64p, i64p, i64p, u32p]),
     "rsd_db_search_topk": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, ci, ci, i64p, f64p, f64p, intp]),
     "rsd_db_search_topk_dev": (ci, [vp, vp, vp, vp, i64, i64, ci, u32, ci, ci, vp, vp, intp, vp]),
     "rsd_db_search_range": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, C.c_double, ci, i64, i64p, i64p, f64p, intp]),
@@ -72,6 +74,7 @@ SIGNATURES = {
     "rsd_multi_set_costs": (ci, [vp, C.c_double, C.c_double, f64p]),
     "rsd_multi_db_load": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32]),
     "rsd_multi_db_free": (ci, [vp]),
+    "rsd_multi_db_append": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32]),
     "rsd_multi_db_search_topk": (ci, [vp, u32p, i64p, i32p, i64, i64, ci, u32, ci, ci, i64p, f64p, f64p, intp]),
     "rsd_multi_db_similarity": (ci, [vp, u8p, i64p, i64, ci, ci, i64p, f64p, f64p]),
     "rsd_multi_db_idf_table": (ci, [vp, f64p, f64p]),

@@ -24,8 +24,10 @@
 #include "k_long.cuh"
 #include "k_long2.cuh"
 #include "k_ingest.cuh"
+#include "k_layout.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 // ------------------------------------------------------------------------------------------------
 // errors
@@ -1445,6 +1447,38 @@ extern "C" int rsd_patch_batch(rsd_ctx *c,
 // ------------------------------------------------------------------------------------------------
 // database search (BASELINE config 5)
 // ------------------------------------------------------------------------------------------------
+// The tier policy of the stored order, shared by rsd_db_load (host counts) and rsd_db_append (device counts).
+// holds[b] = the records that contain symbol b.  rank[b] = b's place when the symbols are ordered by holds, most held
+// first (stable: ties keep code order); a record's tier is the rank of its rarest symbol.
+static void tier_ranks(const int64_t holds[16], int rank[16]) {
+    int order[16];
+    for (int b = 0; b < 16; ++b) order[b] = b;
+    std::stable_sort(order, order + 16, [&](int x, int y) { return holds[x] > holds[y]; });
+    for (int r = 0; r < 16; ++r) rank[order[r]] = r;
+}
+
+// tcnt[t] = the records of unmerged tier t, n their total -> r0, the number of leading tiers merged into tier 0, and
+// per merged tier t: tier_end[t] (stored records [0, tier_end[t]) are of tiers <= t) and tier_mask[t] (their symbols).
+static int tier_cut(const int64_t holds[16], const int64_t tcnt[16], int64_t n, int64_t tier_end[16], uint32_t tier_mask[16]) {
+    int rank[16], order[16];
+    tier_ranks(holds, rank);
+    for (int b = 0; b < 16; ++b) order[rank[b]] = b;
+    uint32_t acc = 0, mask[16];
+    int64_t cum[16], s = 0;
+    for (int r = 0; r < 16; ++r) {
+        if (holds[order[r]] > 0) acc |= 1u << order[r];
+        mask[r] = acc; s += tcnt[r]; cum[r] = s;
+    }
+    // The first tiers are merged up to the one that brings the prefix to half of the records: the bulk of the database
+    // (for RNA: everything made of A, G, C, U, whether or not a record happens to lack one of them) is then ONE tier
+    // sorted by length, and the short chunk that seeds the top-k threshold holds typical records (seeding it from
+    // the handful of records that lack a common symbol gave a useless threshold: 8.7 ms in the next fold, ncu).
+    int r0 = 0;
+    while (r0 < 15 && cum[r0] * 2 < n) ++r0;
+    for (int t = 0; t < 16; ++t) { tier_end[t] = cum[std::min(15, t + r0)]; tier_mask[t] = mask[std::min(15, t + r0)]; }
+    return r0;
+}
+
 extern "C" int rsd_db_load(rsd_ctx *c, const uint32_t *words, const int64_t *start, const int32_t *len,
                            int64_t n_records, int64_t n_words, int bits, uint32_t symmask, int64_t global_index_base) {
     if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
@@ -1488,36 +1522,20 @@ extern "C" int rsd_db_load(rsd_ctx *c, const uint32_t *words, const int64_t *sta
         if (bad_rec.load()) return rsd_fail(RSD_EINVAL, "rsd_db_load: a record lies outside the word buffer");
         int64_t holds[16] = {0};
         for (int64_t i = 0; i < n_records; ++i) for (int b = 0; b < 16; ++b) holds[b] += (rmask[(size_t)i] >> b) & 1;
-        int order[16];
-        for (int b = 0; b < 16; ++b) order[b] = b;
-        std::stable_sort(order, order + 16, [&](int x, int y) { return holds[x] > holds[y]; });
         int rank[16];
-        for (int r = 0; r < 16; ++r) rank[order[r]] = r;
-        uint32_t acc_mask = 0;
-        for (int r = 0; r < 16; ++r) { if (holds[order[r]] > 0) acc_mask |= 1u << order[r]; c->db_tier_mask[r] = acc_mask; }
+        tier_ranks(holds, rank);
         std::vector<uint8_t> tier((size_t)std::max<int64_t>(n_records, 1), 0);
-        int64_t tcnt[17] = {0};
+        int64_t tcnt[16] = {0};
         for (int64_t i = 0; i < n_records; ++i) {
             int t = 0;
             for (int b = 0; b < 16; ++b) if ((rmask[(size_t)i] >> b) & 1) t = std::max(t, rank[b]);
-            tier[(size_t)i] = (uint8_t)t; ++tcnt[t + 1];
+            tier[(size_t)i] = (uint8_t)t; ++tcnt[t];
         }
-        for (int t = 1; t <= 16; ++t) tcnt[t] += tcnt[t - 1];
-        // The first tiers are merged up to the one that brings the prefix to half of the records: the bulk of the database
-        // (for RNA: everything made of A, G, C, U, whether or not a record happens to lack one of them) is then ONE tier
-        // sorted by length, and the short chunk that seeds the top-k threshold holds typical records (seeding it from
-        // the handful of records that lack a common symbol gave a useless threshold: 8.7 ms in the next fold, ncu).
-        int r0 = 0;
-        while (r0 < 15 && tcnt[r0 + 1] * 2 < n_records) ++r0;
-        if (r0 > 0) {
-            for (int64_t i = 0; i < n_records; ++i) tier[(size_t)i] = (uint8_t)std::max(0, (int)tier[(size_t)i] - r0);
-            for (int t = 0; t + r0 <= 16; ++t) tcnt[t] = t == 0 ? 0 : tcnt[t + r0];
-            for (int t = 16 - r0 + 1; t <= 16; ++t) tcnt[t] = n_records;
-            for (int t = 0; t < 16; ++t) c->db_tier_mask[t] = c->db_tier_mask[std::min(15, t + r0)];
-        }
-        for (int t = 0; t < 16; ++t) c->db_tier_end[t] = tcnt[t + 1];
+        const int r0 = tier_cut(holds, tcnt, n_records, c->db_tier_end, c->db_tier_mask);
+        int64_t pos[16];                                            // first stored record of each merged tier
+        for (int t = 0; t < 16; ++t) pos[t] = t == 0 ? 0 : c->db_tier_end[t - 1];
         std::vector<int64_t> perm2((size_t)std::max<int64_t>(n_records, 1));
-        for (int64_t r = 0; r < n_records; ++r) { const int64_t i = perm[(size_t)r]; perm2[(size_t)tcnt[tier[(size_t)i]]++] = i; }     // stable: lengths stay sorted inside a tier
+        for (int64_t r = 0; r < n_records; ++r) { const int64_t i = perm[(size_t)r]; perm2[(size_t)pos[std::max(0, tier[(size_t)i] - r0)]++] = i; }     // stable: lengths stay sorted inside a tier
         perm.swap(perm2);
     }
     std::vector<uint32_t> s_words((size_t)n_words + 8, 0u);
@@ -2301,25 +2319,26 @@ static const IdfExp &idf_expansions() {
     return X;
 }
 
-// Continues the 225 df sums (host df, in and out) over the records of the shard loaded in c, in collection order.
-static int idf_df_shard(rsd_ctx *c, double *df) {
+// Continues the 225 df sums (host df, in and out) over the records [first, db_n) of the shard loaded in c (shard-local
+// collection indices), in collection order.
+static int idf_df_shard(rsd_ctx *c, double *df, int64_t first = 0) {
     cudaStream_t st = c->stream;
     const int64_t n = c->db_n;
     RSD_OK_OR_RETURN(c->idf_dev.ensure(sizeof(double) * 2 * RSD_TF));
     double *d_df = (double *)c->idf_dev.p + RSD_TF;
     RSD_CUDA(cudaMemcpyAsync(d_df, df, sizeof(double) * RSD_TF, cudaMemcpyHostToDevice, st));
-    if (n > 0) {
+    if (n > first) {
         RSD_OK_OR_RETURN(c->idf_exp.ensure(sizeof(IdfExp)));
         RSD_CUDA(cudaMemcpyAsync(c->idf_exp.p, &idf_expansions(), sizeof(IdfExp), cudaMemcpyHostToDevice, st));
         // chunks of 2^20 records: the presence sets take 32 bytes per record of the chunk
-        const int64_t CH = std::min<int64_t>(n, (int64_t)1 << 20);
+        const int64_t CH = std::min<int64_t>(n - first, (int64_t)1 << 20);
         RSD_OK_OR_RETURN(c->idf_work.ensure(32 * (size_t)CH + sizeof(int64_t) * (size_t)n));
         uint32_t *pres = (uint32_t *)c->idf_work.p;            // first: the kernels access it as 16-byte uint4
         int64_t *inv = (int64_t *)(pres + 8 * CH);
         const uint32_t *dbw = (const uint32_t *)c->db.words.p; const int64_t *dbs = (const int64_t *)c->db.start.p; const int32_t *dbl = (const int32_t *)c->db.len.p;
         k_idf_inv<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const int64_t *)c->db_perm.p, c->db_base, n, inv);
         c->launches += 1;
-        for (int64_t i0 = 0; i0 < n; i0 += CH) {
+        for (int64_t i0 = first; i0 < n; i0 += CH) {
             const int64_t nn = std::min(CH, n - i0);
             k_idf_pres<<<(unsigned)((nn + 255) / 256), 256, 0, st>>>(dbw, dbs, dbl, c->db_bits, inv, i0, nn, pres);
             k_idf_chain<<<15, 32 + RSD_IDF_T, 0, st>>>(pres, nn, (const IdfExp *)c->idf_exp.p, d_df);
@@ -2402,6 +2421,137 @@ extern "C" int rsd_db_vector_similarity_batch(rsd_ctx *c, const uint8_t *q_codes
     if (n_queries == 0) return RSD_OK;
     RSD_OK_OR_RETURN(idf_ensure(c, fn));
     return sim_batch_host(c, vector_type, q_codes, q_off, n_queries, method, k, top_idx, top_score, all_scores);
+}
+
+// ------------------------------------------------------------------------------------------------
+// appending records to the loaded database
+// ------------------------------------------------------------------------------------------------
+// The buffers of one device rebuild: scratch, and the new store, which is swapped into the context when it is complete.
+// Whatever the context does not take (the scratch, or the new store after a failure) is freed on the way out.
+struct LayBufs {
+    DevBuf inv, mask, lenc, keys, vals, nw, tmp, cnt, perm;
+    SeqBufs db;
+    ~LayBufs() { DevBuf *all[] = {&inv, &mask, &lenc, &keys, &vals, &nw, &tmp, &cnt, &perm}; for (DevBuf *b : all) b->release(); db.release(); }
+};
+
+extern "C" int rsd_db_append(rsd_ctx *c, const uint32_t *words, const int64_t *start, const int32_t *len,
+                             int64_t n_records, int64_t n_words, int bits, uint32_t symmask) {
+    if (!c) return rsd_fail(RSD_EINVAL, "ctx is NULL");
+    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_append: no database loaded (rsd_db_load)");
+    if (n_records < 0 || n_words < 0 || (n_records > 0 && (!words || !start || !len))) return rsd_fail(RSD_EINVAL, "rsd_db_append: bad arguments");
+    if (bits != c->db_bits) return rsd_fail(RSD_EINVAL, "rsd_db_append: %d-bit records for a %d-bit database (reload it to change the packing)", bits, c->db_bits);
+    if (bits == 2 && (symmask & ~0xFu)) return rsd_fail(RSD_EINVAL, "rsd_db_append: 2-bit packing with symbols outside ACGU");
+    const int per = 32 / bits;
+    int32_t mx = 0;
+    int64_t add_w = 0;
+    for (int64_t i = 0; i < n_records; ++i) {
+        if (len[i] < 0) return rsd_fail(RSD_EINVAL, "rsd_db_append: negative length");
+        const int64_t nw = ((int64_t)len[i] + per - 1) / per;
+        if (start[i] < 0 || start[i] + nw > n_words) return rsd_fail(RSD_EINVAL, "rsd_db_append: record %lld lies outside the word buffer", (long long)i);
+        mx = std::max(mx, len[i]); add_w += nw;
+    }
+    if (n_records == 0) return RSD_OK;
+    RSD_OK_OR_RETURN(c->ensure_device());
+    cudaStream_t st = c->stream;
+    const int64_t n_old = c->db_n, N = n_old + n_records, W = c->db_nwords + add_w;
+    const int64_t maxlen = std::max<int64_t>(c->db_maxlen, mx);
+    LayBufs b;
+    RSD_OK_OR_RETURN(c->upload_seqs(c->bufA, words, start, len, n_records, n_words, st));         // the staging copy
+    RSD_OK_OR_RETURN(b.inv.ensure(sizeof(int64_t) * (size_t)std::max<int64_t>(n_old, 1)));
+    RSD_OK_OR_RETURN(b.mask.ensure(sizeof(uint16_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.lenc.ensure(sizeof(int32_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.keys.ensure(2 * sizeof(uint64_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.vals.ensure(2 * sizeof(int64_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.nw.ensure(sizeof(int64_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.cnt.ensure(sizeof(unsigned long long) * 32));
+    RSD_OK_OR_RETURN(b.perm.ensure(sizeof(int64_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.db.words.ensure(sizeof(uint32_t) * (size_t)(std::max<int64_t>(W, 1) + 8)));
+    RSD_OK_OR_RETURN(b.db.start.ensure(sizeof(int64_t) * (size_t)N));
+    RSD_OK_OR_RETURN(b.db.len.ensure(sizeof(int32_t) * (size_t)N));
+    const unsigned g1 = (unsigned)((N + 255) / 256);
+    if (n_old > 0) {
+        k_idf_inv<<<(unsigned)((n_old + 255) / 256), 256, 0, st>>>((const int64_t *)c->db_perm.p, c->db_base, n_old, (int64_t *)b.inv.p);
+        c->launches += 1;
+    }
+    const LaySrc src{(const uint32_t *)c->db.words.p, (const int64_t *)c->db.start.p, (const int32_t *)c->db.len.p, (const int64_t *)b.inv.p, n_old,
+                     (const uint32_t *)c->bufA.words.p, (const int64_t *)c->bufA.start.p, (const int32_t *)c->bufA.len.p};
+    unsigned long long *d_cnt = (unsigned long long *)b.cnt.p, h_cnt[32];
+    RSD_CUDA(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long) * 32, st));
+    k_lay_mask<<<g1, 256, 0, st>>>(src, N, bits, (uint16_t *)b.mask.p, (int32_t *)b.lenc.p, d_cnt);
+    c->launches += 1;
+    RSD_CUDA(cudaGetLastError());
+    RSD_CUDA(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 16, cudaMemcpyDeviceToHost, st));
+    RSD_CUDA(cudaStreamSynchronize(st));
+    int64_t holds[16], tcnt[16];
+    for (int s = 0; s < 16; ++s) holds[s] = (int64_t)h_cnt[s];
+    int rank[16];
+    tier_ranks(holds, rank);
+    uint64_t rk = 0;
+    for (int s = 0; s < 16; ++s) rk |= (uint64_t)rank[s] << (4 * s);
+    k_lay_tier<<<g1, 256, 0, st>>>((const uint16_t *)b.mask.p, N, rk, d_cnt + 16);
+    c->launches += 1;
+    RSD_CUDA(cudaGetLastError());
+    RSD_CUDA(cudaMemcpyAsync(h_cnt + 16, d_cnt + 16, sizeof(unsigned long long) * 16, cudaMemcpyDeviceToHost, st));
+    RSD_CUDA(cudaStreamSynchronize(st));
+    for (int t = 0; t < 16; ++t) tcnt[t] = (int64_t)h_cnt[16 + t];
+    int64_t tier_end[16];
+    uint32_t tier_mask[16];
+    const int r0 = tier_cut(holds, tcnt, N, tier_end, tier_mask);
+    // stable radix sort by (merged tier, length) over the records in collection order = rsd_db_load's (tier, length,
+    // collection index) order
+    const int lenbits = ceil_log2_i64(maxlen + 1);
+    uint64_t *keys = (uint64_t *)b.keys.p;
+    int64_t *vals = (int64_t *)b.vals.p;
+    k_lay_key<<<g1, 256, 0, st>>>((const uint16_t *)b.mask.p, (const int32_t *)b.lenc.p, N, rk, r0, lenbits, keys, vals);
+    c->launches += 1;
+    RSD_CUDA(cudaGetLastError());
+    cub::DoubleBuffer<uint64_t> kb(keys, keys + N);
+    cub::DoubleBuffer<int64_t> vb(vals, vals + N);
+    size_t tmp_sort = 0, tmp_scan = 0;
+    int64_t *d_nw = (int64_t *)b.nw.p, *d_start = (int64_t *)b.db.start.p;
+    RSD_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_sort, kb, vb, N, 0, 4 + lenbits, st));
+    RSD_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_scan, d_nw, d_start, N, st));
+    RSD_OK_OR_RETURN(b.tmp.ensure(std::max(tmp_sort, tmp_scan)));
+    RSD_CUDA(cub::DeviceRadixSort::SortPairs(b.tmp.p, tmp_sort, kb, vb, N, 0, 4 + lenbits, st));
+    const int64_t *idx = vb.Current();
+    k_lay_order<<<g1, 256, 0, st>>>(idx, (const int32_t *)b.lenc.p, N, bits, c->db_base, (int32_t *)b.db.len.p, d_nw, (int64_t *)b.perm.p);
+    c->launches += 1;
+    RSD_CUDA(cudaGetLastError());
+    RSD_CUDA(cub::DeviceScan::ExclusiveSum(b.tmp.p, tmp_scan, d_nw, d_start, N, st));
+    k_lay_copy<<<(unsigned)((N + 7) / 8), 256, 0, st>>>(src, idx, d_start, N, bits, (uint32_t *)b.db.words.p);
+    c->launches += 1;
+    RSD_CUDA(cudaGetLastError());
+    RSD_CUDA(cudaMemsetAsync((uint32_t *)b.db.words.p + W, 0, sizeof(uint32_t) * (size_t)(std::max<int64_t>(W, 1) - W + 8), st));
+    RSD_CUDA(cudaStreamSynchronize(st));
+    // the new layout is complete: swap it in (the old store goes with b)
+    std::swap(c->db, b.db);
+    std::swap(c->db_perm, b.perm);
+    c->db_n = N; c->db_nwords = W; c->db_maxlen = maxlen; c->db_symmask |= symmask;
+    memcpy(c->db_tier_end, tier_end, sizeof tier_end); memcpy(c->db_tier_mask, tier_mask, sizeof tier_mask);
+    // The df sums are chains in collection order: the appended records continue them.  A failure here leaves the
+    // appended database standing and the table to be rebuilt on next use.
+    if (c->idf_ready) {
+        double df[RSD_TF], idf[RSD_TF];
+        memcpy(df, c->idf_df, sizeof df);
+        int rc = idf_df_shard(c, df, n_old);
+        if (rc == RSD_OK) rc = idf_upload(c, df, idf, idf_from_df(df, N, idf));
+        if (rc != RSD_OK) c->idf_ready = false;
+    }
+    return RSD_OK;
+}
+
+extern "C" int rsd_db_layout(rsd_ctx *c, int64_t *n_records, int64_t *perm, int64_t *tier_end, uint32_t *tier_mask) {
+    if (!c || !n_records) return rsd_fail(RSD_EINVAL, "rsd_db_layout: bad arguments");
+    if (!c->db_loaded) return rsd_fail(RSD_EINVAL, "rsd_db_layout: no database loaded (rsd_db_load)");
+    *n_records = c->db_n;
+    if (tier_end) memcpy(tier_end, c->db_tier_end, sizeof c->db_tier_end);
+    if (tier_mask) memcpy(tier_mask, c->db_tier_mask, sizeof c->db_tier_mask);
+    if (perm && c->db_n > 0) {
+        RSD_OK_OR_RETURN(c->ensure_device());
+        RSD_CUDA(cudaMemcpyAsync(perm, c->db_perm.p, sizeof(int64_t) * (size_t)c->db_n, cudaMemcpyDeviceToHost, c->stream));
+        RSD_CUDA(cudaStreamSynchronize(c->stream));
+    }
+    return RSD_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -273,6 +273,23 @@ class Engine:
         check(self._lib.rsd_db_free(self._ctx))
         self._db_gen = getattr(self, "_db_gen", 0) + 1
 
+    def db_append(self, db: PackedSeqs):
+        """Append db's records (same packing as the loaded database) after the loaded ones: the database then answers
+        every search exactly as a db_load of the concatenation would, and a built idf table is continued, not rebuilt."""
+        check(self._lib.rsd_db_append(self._ctx, ptr(db.words, _u32), ptr(db.start, _i64), ptr(db.len, _i32),
+                                      db.n, db.words.shape[0], db.bits, db.symmask))
+        self._db_n += db.n
+        self._db_gen += 1
+
+    def db_layout(self):
+        """The stored order of the loaded database -> (perm int64[n_db]: global index of stored record r,
+        tier_end int64[16], tier_mask uint32[16])."""
+        n = C.c_int64()
+        check(self._lib.rsd_db_layout(self._ctx, C.byref(n), None, None, None))
+        perm = np.zeros(max(n.value, 1), np.int64); te = np.zeros(16, np.int64); tm = np.zeros(16, np.uint32)
+        check(self._lib.rsd_db_layout(self._ctx, C.byref(n), ptr(perm, _i64), ptr(te, _i64), ptr(tm, _u32)))
+        return perm[:n.value], te, tm
+
     def db_search_topk(self, Q: PackedSeqs, k: int, want_scores: bool = False, force_mode: int = 0):
         """-> (top_idx int64[q,k], top_score f64[q,k][, all_scores f64[q, n_db]])."""
         Q = _db_query(Q, self._db_bits)
@@ -449,6 +466,13 @@ class MultiEngine:
 
     def db_free(self):
         check(self._lib.rsd_multi_db_free(self._h))
+        self._db_gen += 1
+
+    def db_append(self, db: PackedSeqs):
+        """Engine.db_append over the whole database: the records go to the last shard (no rebalancing)."""
+        check(self._lib.rsd_multi_db_append(self._h, ptr(db.words, _u32), ptr(db.start, _i64), ptr(db.len, _i32), db.n,
+                                            db.words.shape[0], db.bits, db.symmask))
+        self._db_n += db.n
         self._db_gen += 1
 
     def db_search_topk(self, Q: PackedSeqs, k: int, want_scores: bool = False, force_mode: int = 0):

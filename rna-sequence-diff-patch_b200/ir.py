@@ -45,16 +45,24 @@ class _Resident:
     session that searches the same collection again (gui.py:532-600: every search re-reads collection.find({})) pays
     rsd_db_load once per engine.  The copy is keyed on its content (the documents after the case rule of the measure
     that loaded them), so wf_score (upper case) and the other measures (as stored) share it when the collection has no
-    lower-case letters."""
+    lower-case letters.  A collection that only grew (gui.py's imports, fa_import.py: records added at the end) has its
+    new documents appended to the held copy instead of being reloaded."""
     held = weakref.WeakKeyDictionary()      # engine -> (load generation, documents as given, upper, documents as loaded)
 
     @classmethod
     def load(cls, eng, sequences, upper: bool):
         h = cls.held.get(eng)
-        if h is not None and h[0] == getattr(eng, "_db_gen", 0):
-            if (h[2] == upper and h[1] == sequences) or h[3] == (_upper(sequences) if upper else sequences):
-                return
+        if h is not None and h[0] == getattr(eng, "_db_gen", 0) and h[2] == upper and h[1] == sequences:
+            return
         content = _upper(sequences) if upper else sequences
+        if h is not None and h[0] == getattr(eng, "_db_gen", 0):
+            if h[3] == content:
+                return
+            n = len(h[3])
+            if n < len(content) and content[:n] == h[3]:
+                eng.db_append(pack(content[n:], bits=4))
+                cls.held[eng] = (eng._db_gen, sequences, upper, content)
+                return
         cls.held.pop(eng, None)
         eng.db_load(pack(content, bits=4))
         cls.held[eng] = (eng._db_gen, sequences, upper, content)

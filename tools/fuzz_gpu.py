@@ -77,7 +77,7 @@ def main():
     ap.add_argument("--seed", type=int, default=1)
     args = ap.parse_args()
     rng = np.random.default_rng(args.seed)
-    eng = R.Engine(0)
+    eng, ref = R.Engine(0), None
     t_end = time.time() + args.seconds
     rounds = bad = 0
     cells = 0.0
@@ -86,7 +86,7 @@ def main():
         alpha = [SYM[:4], SYM[:4], SYM[:4] + "N", SYM, SYM[:2], "ACGUYR"][int(rng.integers(0, 6))]
         ckind = ["default", "user", "dyadic", "int", "decimal"][int(rng.integers(0, 5))]
         lkind = ["tiny", "short", "c2", "kb", "skew", "wide"][int(rng.integers(0, 6))]
-        what = ["dist", "dist", "script", "search", "long", "sim", "range", "simb"][int(rng.integers(0, 8))]
+        what = ["dist", "dist", "script", "search", "long", "sim", "range", "simb", "append"][int(rng.integers(0, 9))]
         costs = random_costs(rng, ckind)
         eng.set_costs(costs)
         force = int(rng.choice([0, 0, 0, 2, 3]))
@@ -256,6 +256,48 @@ def main():
                     ok = ok and np.array_equal(idx[off[q]:off[q + 1]], w) and np.array_equal(dist[off[q]:off[q + 1]], D[q, w])
                 cells += float(ql.sum()) * float(lens.sum())
                 desc = f"range n={n} q={nq} max_dist={bound!r} hits={int(off[-1])} mode={eng.last_mode}"
+            elif what == "append":
+                # a collection split at random into a load and 1-3 appends (some empty, some of other alphabets, so the
+                # tiers move); everything compared with a fresh load of the whole collection
+                n = int(rng.choice([1, 50, 3000, 40000]))
+                lens = rng.integers(0 if rng.random() < 0.3 else 20, int(rng.choice([32, 33, 60])), size=n)
+                cuts = np.sort(rng.integers(0, n + 1, size=int(rng.integers(1, 4))))
+                bounds = [0, *cuts.tolist(), n]
+                parts = [make(rng, lens[a:b], alpha if rng.random() < 0.7 else str(rng.choice([SYM, "ACGUYR", "YR", SYM[:4] + "N"])))
+                         for a, b in zip(bounds[:-1], bounds[1:])]
+                cd = np.concatenate([c for c, _ in parts]); od = np.zeros(n + 1, np.int64); np.cumsum(lens, out=od[1:])
+                nq = int(rng.integers(1, 5)); k = int(rng.choice([1, 6, 10, 128]))
+                ql = rng.integers(1, int(rng.choice([32, 65])), size=nq)
+                cq, oq = make(rng, ql, alpha)
+                Qp = R.pack((cq, oq), bits=4)
+                method = str(rng.choice(IO.METHODS))
+                ref = ref or R.Engine(0)                        # the fresh load
+                ref.set_costs(costs)
+                idf_first = rng.random() < 0.5
+                bound = float(rng.choice([1.0, 4.0, np.inf]))
+                got, want = [], []
+                for e, pieces in ((eng, parts), (ref, [(cd, od)])):
+                    e.db_load(R.pack(pieces[0], bits=4))
+                    try:
+                        if idf_first:
+                            e.db_idf_table()
+                        for p in pieces[1:]:
+                            e.db_append(R.pack(p, bits=4))
+                        out = [e.db_layout(), e.db_search_topk(Qp, k, want_scores=True), e.db_search_range(Qp, bound),
+                               e.db_similarity_batch([cq[oq[q]:oq[q + 1]] for q in range(nq)], method, k=10)]
+                        if method in IO.METHODS[6:]:
+                            out.append(e.db_similarity_batch([cq[oq[q]:oq[q + 1]] for q in range(nq)], method, k=10, vector_type="tf-idf"))
+                            out.append(e.db_idf_table())
+                    finally:
+                        e.db_free()
+                    (got if e is eng else want).append(out)
+                flat = lambda xs: [np.asarray(a) for x in xs for y in x for a in (y if isinstance(y, tuple) else (y,)) if a is not None]
+                fg, fw = flat(got[0]), flat(want[0])
+                diff = [i for i, (a, b) in enumerate(zip(fg, fw)) if a.shape != b.shape or a.tobytes() != b.tobytes()]
+                ok = len(fg) == len(fw) and not diff
+                cells += float(ql.sum()) * float(lens.sum())
+                desc = (f"append n={n} parts={[b - a for a, b in zip(bounds[:-1], bounds[1:])]} q={nq} k={k} {method} "
+                        f"idf_first={idf_first} max_dist={bound}" + (f" differing outputs {diff}" if diff else ""))
             else:
                 n = int(rng.choice([1, 50, 3000, 40000]))
                 lens = rng.integers(0 if rng.random() < 0.3 else 20, int(rng.choice([32, 33, 60])), size=n)
